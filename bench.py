@@ -2,6 +2,7 @@
 """Headline benchmark: EGConv forward+backward edges/s on synthetic graphs of the shapes BASELINE.json names.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload arxiv|mag|zinc|cifar|rmag] [--layers L] [--impl ours|reference]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
            bench.py --gpus N --steps K --warmup W
 
@@ -23,7 +24,8 @@ measured HBM peak (`traffic` = its DRAM bytes from the committed ncu capture of 
 `step_roofline` = the step's unique bytes / step time; `cpu_baseline` = the oracle port of the reference path timed on
 this box's host cores, whose results are also the checker of `parity_check` at N = 1 (GPU vs fp64 oracle, full graph);
 `gpu_launches` = kernels of libegc_b200 launched in the timed region.  `--impl reference` times the CPU path alone on
-the same workload.
+the same workload.  `--dump-outputs DIR` (one GPU, full-graph workloads) writes what the last timed step returned as
+DIR/<name>.npy (`dump_outputs`); the inputs are seeded (`--seed`), so two builds can be compared output for output.
 """
 import argparse
 import json
@@ -369,8 +371,9 @@ def device_graph_input(w, n, edge_index, dev):
     return egc_b200.SparseTensor(rowptr=rowptr.to(dev), col=col.to(dev), sparse_sizes=(n, n), is_sorted=True)
 
 
-def cuda_timed(fn, steps, warmup, barrier=None):
-    """CUDA-event time per call of `fn` after `warmup` untimed calls; (ms, kernels launched by libegc_b200)."""
+def cuda_timed(fn, steps, warmup, barrier=None, last=None):
+    """CUDA-event time per call of `fn` after `warmup` untimed calls; (ms, kernels launched by libegc_b200).
+    `last` (a list), when given, receives what the last timed call returned."""
     from egc_b200 import _lib
     for _ in range(warmup):
         fn()
@@ -380,13 +383,35 @@ def cuda_timed(fn, steps, warmup, barrier=None):
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     l0 = _lib.launch_count()
     ev0.record()
-    for _ in range(steps):
-        fn()
+    if last is None:
+        for _ in range(steps):
+            fn()
+    else:
+        for _ in range(steps):
+            last[:] = [fn()]
     ev1.record()
     torch.cuda.synchronize()
     if barrier:
         barrier()
     return ev0.elapsed_time(ev1) / steps, _lib.launch_count() - l0
+
+
+DUMP_ROWS = 16_384          # rows kept of each per-node array by --dump-outputs (8 MB for a 128-wide fp32 array)
+
+
+def dump_outputs(directory, named, n, seed=0):
+    """Write the arrays a step returned (`named`: name -> tensor) as `directory`/<name>.npy in float32.  Per-node arrays
+    (first dimension `n`: the output, d_x) keep the same DUMP_ROWS rows, drawn with a fixed seed and sorted, so that
+    the files of two builds compare row for row and stay far below 64 MB; parameter gradients are written whole."""
+    os.makedirs(directory, exist_ok=True)
+    rows = None
+    if n > DUMP_ROWS:
+        rows = torch.from_numpy(np.sort(np.random.default_rng(seed).choice(n, DUMP_ROWS, replace=False)))
+    for name, t in named.items():
+        t = t.detach()
+        if rows is not None and t.dim() > 0 and t.size(0) == n:
+            t = t[rows.to(t.device)]
+        np.save(os.path.join(directory, f"{name}.npy"), t.float().cpu().numpy())
 
 
 def traced_kernels(fn, steps):
@@ -513,12 +538,17 @@ def run_single_gpu(args, name, w):
     l0 = _lib.launch_count()
     job.step()
     launches_per_step = _lib.launch_count() - l0
+    last = [] if args.dump_outputs else None
     with ClockSampler(dev.index or 0) as clocks:
         if args.no_graph:
-            ms, _ = cuda_timed(job.step, args.steps, args.warmup)
+            ms, _ = cuda_timed(job.step, args.steps, args.warmup, last=last)
             ms_eager = ms
         else:
-            ms, _ = cuda_timed(job.replay, args.steps, args.warmup)
+            ms, _ = cuda_timed(job.replay, args.steps, args.warmup, last=last)
+        if args.dump_outputs:
+            out, grads = job.grads_named(last[0])
+            dump_outputs(args.dump_outputs, {"out": out, **{f"grad_{k}": g for k, g in grads.items()}}, n, args.seed)
+        if not args.no_graph:
             ms_eager, _ = cuda_timed(job.step, args.steps, args.warmup)
         ms_e2e, _ = cuda_timed(step_e2e, max(3, min(args.steps, 10)), 2)
     prof, kernels = traced_kernels(job.step, args.steps)
@@ -1041,7 +1071,7 @@ def run_minibatch(args, m):
         torch.cuda.synchronize()
         return ev0.elapsed_time(ev1) / steps, _lib.launch_count() - l0
 
-    steps = max(args.steps, n_batches)
+    steps = args.steps
     with ClockSampler(dev.index or 0) as clocks:
         ms_eager, launches = timed(step, steps, args.warmup)
         ms_eager_e2e, _ = timed(step_e2e, steps, 2)
@@ -1189,7 +1219,7 @@ def run_minibatch_dp(args, m):
     del ref_model, ref_grads
 
     nnz_local = sum(step()[1] for _ in range(n_batches)) / n_batches      # also the warm-up of every kernel shape
-    steps = max(args.steps, n_batches)
+    steps = args.steps
 
     # fixed-shape path: the whole local step replays from ONE CUDA graph, which also packs the (scaled) parameter
     # gradients into one flat buffer; then ONE NCCL all-reduce of that buffer.  Every rank pads to its own capacity.
@@ -1519,7 +1549,15 @@ def main():
     ap.add_argument("--bwd-flags", type=int, default=0, help="EGC_BWD_* tuning bits passed to egc_aggregate_bwd (A/B runs)")
     ap.add_argument("--locality", type=float, default=-1.0,
                     help="p_intra of the synthetic generator (default 0.8 with 8 id blocks, for every GPU count)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned (output, d_x, parameter "
+                         "gradients) as DIR/<name>.npy; single-GPU full-graph workloads")
     args = ap.parse_args()
+    if args.steps < 1:
+        sys.exit("--steps must be >= 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload not in WORKLOADS or args.gpus > 1
+                              or int(os.environ.get("WORLD_SIZE", 1)) > 1):
+        sys.exit("--dump-outputs is implemented for the single-GPU full-graph workloads (" + ", ".join(WORKLOADS) + ")")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", 0))
     if args.workload == "rmag":

@@ -2,25 +2,27 @@
 
 TEST INFRASTRUCTURE ONLY - nothing under `egc_b200/` may import this module.
 
-`/root/reference/experiments/optimized_layers.py` (EGConv) and
-`/root/reference/experiments/layers.py` (EfficientGraphConv) depend on
+The reference's `experiments/optimized_layers.py` (EGConv) and
+`experiments/layers.py` (EfficientGraphConv) depend on
 torch_geometric / torch_scatter / torch_sparse, none of which is installable
 offline.  `oracle/shims/` holds original pure-torch stand-ins for the leaf ops;
 with them on `sys.path` the reference's own `forward`, `aggregate` and
 `message_and_aggregate` run verbatim and autograd yields reference gradients.
 
-`/root/reference` exists only in the build container.  On the GPU box
-`available()` is False and parity rests on `oracle/restatement.py` (asserted
-equal to this loader in `tests/test_oracle.py`) and on `tests/golden/*.pt`
-(generated from this loader by `oracle/make_golden.py`).
+The reference sources are not part of this repository.  They are looked for
+in `oracle/_ref/` (a checkout of shyam196/egc, ignored by git) or in the
+directory `EGC_REFERENCE_ROOT` names.  Without them `available()` is False and
+parity rests on `oracle/restatement.py` and on `tests/golden/*.pt` (generated
+from this loader by `oracle/make_golden*.py`).
 """
 import importlib
 import os
 import sys
 from types import SimpleNamespace
 
-REFERENCE_ROOT = os.environ.get("EGC_REFERENCE_ROOT", "/root/reference")
-_SHIMS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "shims")
+_ORACLE_DIR = os.path.dirname(os.path.abspath(__file__))
+REFERENCE_ROOT = os.environ.get("EGC_REFERENCE_ROOT", os.path.join(_ORACLE_DIR, "_ref"))
+_SHIMS = os.path.join(_ORACLE_DIR, "shims")
 _cache = None
 
 
@@ -34,7 +36,7 @@ def _ensure_shims() -> None:
 
 
 def shims() -> SimpleNamespace:
-    """The shim modules themselves (usable without /root/reference)."""
+    """The shim modules themselves (usable without the reference sources)."""
     _ensure_shims()
     return SimpleNamespace(
         torch_scatter=importlib.import_module("torch_scatter"),

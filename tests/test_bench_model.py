@@ -4,6 +4,7 @@ import json
 import subprocess
 import sys
 
+import numpy as np
 import torch
 
 import bench
@@ -54,9 +55,30 @@ def test_reference_arm_prints_the_contract_line():
     out = subprocess.run([sys.executable, "bench.py", "--impl", "reference", "--workload", "zinc", "--steps", "1", "--warmup", "0"],
                          capture_output=True, text=True, cwd=bench.ROOT, timeout=600)
     line = json.loads(out.stdout.strip().splitlines()[-1])
-    assert line["impl"] == "reference" and line["unit"] == "edges/s" and line["value"] > 0
+    assert line["impl"] == "reference" and line["unit"] == "edges/s" and line["value"] > 0 and line["steps"] == 1
     assert line["cpu_baseline"]["kind"] == "port" and line["cpu_baseline"]["cores"] >= 1
     assert line["e2e"] == {"value": line["value"], "unit": "edges/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
+
+
+def test_dump_outputs_keeps_the_same_seeded_rows(tmp_path):
+    n = bench.DUMP_ROWS + 1000
+    out = torch.arange(n, dtype=torch.float64)[:, None].repeat(1, 3)          # row i holds i
+    grad_w = torch.randn(4, 5)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), {"out": out, "grad_w": grad_w}, n)
+    o = np.load(tmp_path / "a" / "out.npy")
+    assert o.dtype == np.float32 and o.shape == (bench.DUMP_ROWS, 3)
+    assert (np.diff(o[:, 0]) > 0).all() and o[-1, 0] < n and (o[:, 1] == o[:, 0]).all()
+    assert np.array_equal(np.load(tmp_path / "b" / "out.npy"), o)
+    assert np.array_equal(np.load(tmp_path / "a" / "grad_w.npy"), grad_w.numpy())
+
+
+def test_rejected_arguments_exit_before_any_work():
+    for extra, msg in ((["--steps", "0"], "--steps must be >= 1"),
+                       (["--workload", "zinc", "--dump-outputs", "unused"], "--dump-outputs is implemented for")):
+        out = subprocess.run([sys.executable, "bench.py"] + extra, capture_output=True, text=True, cwd=bench.ROOT,
+                             timeout=120)
+        assert out.returncode != 0 and not out.stdout.strip() and msg in out.stderr
 
 
 def test_local_roofline_of_partitioned_runs():

@@ -1,6 +1,6 @@
 """Heterogeneous layer REGConv (SURVEY.md section 8 f-2; ref experiments/rmag/models.py:75-148).
 CPU: the restatement (oracle/hetero.py) against the golden vectors generated from the UNMODIFIED reference class and,
-where /root/reference is mounted, against that class executed through the shims.  GPU: egc_b200.REGConv against the
+where the reference sources are present, against that class executed through the shims.  GPU: egc_b200.REGConv against the
 goldens and the fp64 restatement, through the C ABI."""
 import importlib
 
@@ -44,7 +44,7 @@ def test_restatement_matches_reference_golden(name):
             assert rel_err(g, rec[tag]["grad_p"][n]) < tol, n
 
 
-@pytest.mark.skipif(not rl.available(), reason="needs /root/reference")
+@pytest.mark.skipif(not rl.available(), reason="needs the reference sources (oracle/_ref or EGC_REFERENCE_ROOT)")
 def test_restatement_matches_reference_source():
     rl.load()
     ref = importlib.import_module("experiments.rmag.models")

@@ -1,6 +1,6 @@
 """Pins the CPU oracle (oracle/restatement.py): against the golden vectors generated from the
 UNMODIFIED reference source (tests/golden, made by oracle/make_golden.py) and, where
-/root/reference is present, against the reference itself executed through oracle/shims."""
+the reference sources are present (oracle/reference_loader.py), against the reference itself executed through oracle/shims."""
 import itertools
 
 import pytest
@@ -112,7 +112,7 @@ def test_hand_computed_tiny_graph():
     assert g3.rowptr.tolist() == [0, 4, 5, 6, 6]
 
 
-@pytest.mark.skipif(not rl.available(), reason="/root/reference not present (GPU box)")
+@pytest.mark.skipif(not rl.available(), reason="needs the reference sources (oracle/_ref or EGC_REFERENCE_ROOT)")
 def test_restatement_matches_reference_source():
     ref = rl.load()
     n = 150
@@ -142,7 +142,7 @@ def test_restatement_matches_reference_source():
     assert worst < 1e-12
 
 
-@pytest.mark.skipif(not rl.available(), reason="/root/reference not present (GPU box)")
+@pytest.mark.skipif(not rl.available(), reason="needs the reference sources (oracle/_ref or EGC_REFERENCE_ROOT)")
 def test_paper_layer_agrees_with_fused_layer():
     """Secondary pin (SURVEY.md App. B): EfficientGraphConv == EGConv under the weight permutation when
     add_self_loops=False (the only setting where their self-loop rules coincide)."""
@@ -192,7 +192,22 @@ def test_paper_to_egconv_permutation():
     assert perm.tolist() == expect and sorted(perm.tolist()) == list(range(h * b * a))
 
 
-@pytest.mark.skipif(not rl.available(), reason="needs /root/reference")
+ADJ_CASES = [n for n in golden_cases() + golden_cases("paper_") if load_golden(n)["kind"] != "edge_index"]
+
+
+@pytest.mark.parametrize("name", ADJ_CASES)
+def test_to_sparse_tensor_matches_the_golden_adjacency_bit_exact(name):
+    """egc_b200.to_sparse_tensor against the adj_t the golden generator built from the same edge list with the
+    reference's ordering (experiments/utils.py:93; duplicates, self-loops and isolated nodes kept): same rowptr, same
+    column order."""
+    import egc_b200
+    rec = load_golden(name)
+    rowptr, col, value = egc_b200.to_sparse_tensor(rec["edge_index"], rec["n"]).csr()
+    assert value is None
+    assert torch.equal(rowptr, rec["adj_rowptr"]) and torch.equal(col, rec["adj_col"])
+
+
+@pytest.mark.skipif(not rl.available(), reason="needs the reference sources (oracle/_ref or EGC_REFERENCE_ROOT)")
 def test_to_sparse_tensor_matches_the_reference_transform_bit_exact():
     """egc_b200.to_sparse_tensor == experiments/utils.py:82-118 ToSparseTensor (run through the shims) on an edge list
     with duplicates and self-loops: same rowptr, same column order."""
