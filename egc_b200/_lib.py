@@ -63,6 +63,7 @@ SIGNATURES = {
     "egc_plan_build": (c_int32, [_P, c_int32, c_int32, c_int32, _P, _P, _P, _P, _P, c_size_t, _P]),
     "egc_plan_build_workspace_bytes": (c_size_t, [c_int32]),
     "egc_project_fwd": (c_int32, [_P, _P, _P, _P, c_int32, c_int32, c_int32, c_int32, c_int32, _P, _P, c_int32, _P]),
+    "egc_project_fwd_bf16": (c_int32, [_P, _P, _P, _P, c_int32, c_int32, c_int32, c_int32, c_int32, _P, _P, c_int32, _P]),
     "egc_project_bwd_workspace_bytes": (c_size_t, [c_int32, c_int32, c_int32, c_int32]),
     "egc_project_bwd": (c_int32, [_P, _P, _P, _P, _P, c_int32, c_int32, c_int32, c_int32, _P, _P, _P, _P,
                                   c_int32, _P, c_size_t, _P]),
@@ -71,6 +72,11 @@ SIGNATURES = {
     "egc_aggregate_fwd_workspace_bytes": (c_size_t, [POINTER(LayerDesc), POINTER(RowPlan)]),
     "egc_aggregate_fwd": (c_int32, [POINTER(LayerDesc), _P, _P, _P, _P, POINTER(RowPlan), _P, _P, _P, POINTER(Epilogue), _P, c_int32,
                                     _P, _P, _P, _P, _P, _P, c_size_t, _P]),
+    "egc_aggregate_fwd_bf16": (c_int32, [POINTER(LayerDesc), _P, _P, _P, POINTER(RowPlan), _P, _P, _P, POINTER(Epilogue),
+                                         _P, _P, _P, _P, _P, _P, c_size_t, _P]),
+    "egc_aggregate_bwd_bf16_workspace_bytes": (c_size_t, [POINTER(LayerDesc), POINTER(RowPlan), c_int32]),
+    "egc_aggregate_bwd_bf16": (c_int32, [POINTER(LayerDesc), _P, _P, _P, _P, _P, _P, POINTER(RowPlan), _P, _P, _P, _P, _P, _P, _P,
+                                         _P, _P, _P, _P, c_int32, _P, c_size_t, _P]),
     "egc_aggregate_bwd_workspace_bytes": (c_size_t, [POINTER(LayerDesc), POINTER(RowPlan), c_int32]),
     "egc_aggregate_bwd": (c_int32, [POINTER(LayerDesc), _P, _P, _P, _P, _P, _P, _P, _P, POINTER(RowPlan), _P, _P, _P,
                                     _P, _P, _P, _P, _P, _P, _P, _P, _P, c_int32, c_int32, _P, c_size_t, _P]),

@@ -58,6 +58,9 @@ class EfficientGraphConv(torch.nn.Module):
                 raise ValueError(f'Unknown aggregator "{a}".')
         self.cache = cache
         self.gemm_algo = kwargs.pop("gemm_algo", _lib.GEMM_AUTO)
+        if kwargs.pop("storage_dtype", torch.float32) != torch.float32:
+            raise NotImplementedError("EfficientGraphConv: bf16 storage is not supported; use egc_b200.EGConv(..., "
+                                      "storage_dtype=torch.bfloat16)")
         self.comb_weights = Linear(in_channels, num_heads * num_bases * len(self.aggregators))
         self.bases_weight = ParameterList([Parameter(torch.empty(in_channels, out_channels // num_heads))
                                            for _ in range(num_bases)])

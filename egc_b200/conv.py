@@ -14,7 +14,7 @@ from torch import Tensor
 from torch.nn import Linear, Parameter
 
 from . import _lib
-from .functional import egconv
+from .functional import check_storage_dtype, egconv
 from .graph import GraphStructure, adjacency_to_csr
 
 _AGGREGATORS = {"sum", "mean", "symnorm", "min", "max", "var", "std"}
@@ -28,12 +28,16 @@ class EGConv(torch.nn.Module):
     sigmoid=False.  Extra keyword-only knobs of this implementation:
       gemm_algo: one of egc_b200.GEMM_* (projection kernels; default AUTO)
       deterministic: route min/max gradients without fp32 atomics
+      storage_dtype: torch.float32 (default) or torch.bfloat16 - bf16 storage (round to nearest even) of the two gathered
+        tensors, the basis rows and the backward's target-side streams; x, parameters, out, all accumulation and every
+        gradient stay fp32.  Covers num_bases * out_channels / num_heads of 40..128, a multiple of 8; other shapes raise
+        ValueError at the first forward.
     """
 
     def __init__(self, in_channels: int, out_channels: int, aggrs: Iterable[str] = ("symnorm",),
                  num_heads: int = 8, num_bases: int = 4, cached: bool = False, add_self_loops: bool = True,
                  bias: bool = True, sigmoid: bool = False, *, gemm_algo: int = _lib.GEMM_AUTO,
-                 deterministic: bool = False, **kwargs):
+                 deterministic: bool = False, storage_dtype: torch.dtype = torch.float32, **kwargs):
         super().__init__()
         if out_channels % num_heads != 0:
             raise ValueError("out_channels must be divisible by the number of heads")          # ref :89-90
@@ -52,6 +56,7 @@ class EGConv(torch.nn.Module):
         self.sigmoid = sigmoid
         self.gemm_algo = gemm_algo
         self.deterministic = deterministic
+        self.storage_dtype = check_storage_dtype(storage_dtype)
         self.node_dim = 0                                                                        # ref :87
 
         self.bases_weight = Parameter(torch.empty(in_channels, (out_channels // num_heads) * num_bases))
@@ -112,7 +117,7 @@ class EGConv(torch.nn.Module):
         flags = (_lib.BWD_DETERMINISTIC if self.deterministic else 0) | int(getattr(self, "bwd_flags", 0))
         return egconv(x, graph, self.bases_weight, self.comb_weight.weight, self.comb_weight.bias, self.bias,
                       self.num_heads, self.num_bases, self.aggregators, self.sigmoid, self.gemm_algo, flags, relu,
-                      scale, shift, residual)
+                      scale, shift, residual, self.storage_dtype)
 
     def __repr__(self):                                                                          # ref :280-286
         return "{}({}, {}, {})".format(self.__class__.__name__, self.in_channels, self.out_channels,

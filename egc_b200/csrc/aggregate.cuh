@@ -405,5 +405,9 @@ int launch_aggregate_rows_static(int cfg_index, const AggParams& p, bool arg, in
 int launch_aggregate_rows_g32(const AggParams& p, int mask, bool arg, int* task_counter, cudaStream_t st);
 int launch_aggregate_rows_g16(const AggParams& p, int mask, bool arg, int* task_counter, cudaStream_t st);
 int rows_kernel_smem_bytes(const AggParams& p);
+// the same kernel over bf16 basis rows (p.bases -> bf16, p.nvec = B*D / 8; aggregate_rows_bf16_*.cu)
+int launch_aggregate_rows_bf16_static(int cfg_index, const AggParams& p, bool arg, int* task_counter, cudaStream_t st);
+int launch_aggregate_rows_bf16_g8(const AggParams& p, int mask, bool arg, int* task_counter, cudaStream_t st);
+int launch_aggregate_rows_bf16_g16(const AggParams& p, int mask, bool arg, int* task_counter, cudaStream_t st);
 
 }  // namespace egc

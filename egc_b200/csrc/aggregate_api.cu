@@ -74,6 +74,8 @@ static int validate_plan(const egc_row_plan* plan, const char* who) {
 
 namespace egc {
 
+constexpr int kBf16RingDepth = 8;
+
 // which target-side streams does this aggregator list need?  bit0 sym, bit1 lin, bit2 sq
 static int stream_mask_of(const egc_layer_desc& d, bool& has_route) {
   int m = 0;
@@ -97,7 +99,8 @@ struct BwdLayout {
   bool has_route;
 };
 
-static BwdLayout bwd_layout(const egc_layer_desc& d, const egc_row_plan* csc_plan) {
+// ts_elem: bytes per stored target-side stream value (4, or 2 with bf16 storage)
+static BwdLayout bwd_layout(const egc_layer_desc& d, const egc_row_plan* csc_plan, size_t ts_elem = 4) {
   BwdLayout L{};
   L.tsmask = stream_mask_of(d, L.has_route);
   int s = 0;
@@ -106,7 +109,7 @@ static BwdLayout bwd_layout(const egc_layer_desc& d, const egc_row_plan* csc_pla
   L.ts_sq = (L.tsmask & 4) ? s++ : -1;
   L.n_ts = s;
   const size_t bd = static_cast<size_t>(d.bases) * d.dim;
-  L.ts_bytes = align_up(static_cast<size_t>(d.n_dst) * std::max(L.n_ts, 1) * bd * 4, 256);
+  L.ts_bytes = align_up(static_cast<size_t>(d.n_dst) * std::max(L.n_ts, 1) * bd * ts_elem, 256);
   L.csc_part_bytes = align_up(static_cast<size_t>(csc_plan ? csc_plan->n_chunks : 0) * std::max(L.n_ts, 1) * bd * 4, 256) +
                      align_up(static_cast<size_t>(csc_plan ? csc_plan->n_long : 0) * sizeof(int), 256) +
                      256;   // + the task counter of k_scatter_cols
@@ -126,7 +129,7 @@ static BwdLayout bwd_layout(const egc_layer_desc& d, const egc_row_plan* csc_pla
 static int run_pass2(const egc_layer_desc& desc, const BwdLayout& L, const int32_t* colptr, const int32_t* rowidx,
                      const float* csc_val_sym, const float* csc_val_lin, const egc_row_plan* csc_plan, const float* tstreams,
                      const float* bases, float* d_bases, int col_begin, int col_end, bool accumulate, float* csc_part, bool vec4,
-                     cudaStream_t st) {
+                     cudaStream_t st, bool bf16_store = false) {
   const int bd = desc.bases * desc.dim;
   AggParams geo{};
   fill_agg_params(geo, desc, vec4);
@@ -148,7 +151,9 @@ static int run_pass2(const egc_layer_desc& desc, const BwdLayout& L, const int32
   // column-block kernel: 128-bit pieces, unweighted entries, one pass, interleaved streams
   // (EGC_BWD_WARP_PER_COLUMN=1 keeps the warp-per-column kernel)
   static const bool legacy_cols = getenv("EGC_BWD_WARP_PER_COLUMN") != nullptr;
-  const bool col_blocks = vec4 && csc_val_lin == nullptr && geo.n_pass == 1 && (geo.G == 32 || geo.G == 16) && !legacy_cols;
+  const bool col_blocks = vec4 && csc_val_lin == nullptr && geo.n_pass == 1 && (geo.G == 32 || geo.G == 16) && (!legacy_cols || bf16_store);
+  EGC_REQUIRE(col_blocks || !bf16_store, "egc_aggregate_bwd_bf16: the column pass needs rows of 36..128 values, a multiple of 4, 16-byte "
+              "aligned, and no per-entry linear weights");
   const bool fuse_merge = geo.n_pass == 1 && s.n_long > 0;     // the last chunk warp of a long column merges its partials
   s.long_counter = (col_blocks || fuse_merge) ? long_counter : nullptr;
   s.tstreams = tstreams; s.bases = bases; s.d_bases = d_bases;
@@ -166,8 +171,9 @@ static int run_pass2(const egc_layer_desc& desc, const BwdLayout& L, const int32
   // EGC_BWD_NEAR_MB overrides the span for every layer (0 = no hints).
   static const int near_env = [] { const char* e = getenv("EGC_BWD_NEAR_MB"); return e ? std::max(0, atoi(e)) : -1; }();
   const int near_mb = near_env >= 0 ? near_env : (L.n_ts >= 2 ? 64 : 0);
+  const int64_t ts_elem = bf16_store ? 2 : 4;
   s.near_rows = static_cast<int>(std::min<int64_t>(int64_t{1} << 30, (static_cast<int64_t>(near_mb) << 20) /
-                                                       std::max<int64_t>(1, static_cast<int64_t>(std::max(L.n_ts, 1)) * bd * 4 * 2)));
+                                                       std::max<int64_t>(1, static_cast<int64_t>(std::max(L.n_ts, 1)) * bd * ts_elem * 2)));
   s.mode = 0;
   if (s.col_end <= s.col_begin) return EGC_OK;
   if (col_blocks) {
@@ -175,9 +181,18 @@ static int run_pass2(const egc_layer_desc& desc, const BwdLayout& L, const int32
     // ring variant (rows land in a per-warp shared-memory ring, R entries ahead across columns): 128-float rows, two or more
     // streams.  Measured on B200, arxiv-shaped EGC-M (profiles/r02r_ring.txt): 0.334 -> 0.282 ms (depth 4 = depth 7), uniform
     // graph 0.480 -> 0.439 ms.  EGC_BWD_RING = ring depth (4: three CTAs per SM, 7: two), 0 = the register-gather kernel.
-    static const int ring = [] { const char* e = getenv("EGC_BWD_RING"); return e ? atoi(e) : 4; }();
-    if (ring > 0 && geo.G == 32 && L.n_ts >= 2)
-      return ring >= 7 ? launch_scatter_ring<7>(s, L.tsmask, task_counter, st) : launch_scatter_ring<4>(s, L.tsmask, task_counter, st);
+    static const int ring = [] { const char* e = getenv("EGC_BWD_RING"); return e ? atoi(e) : -1; }();
+    if (bf16_store) {
+      // bf16 streams: a slot holds half the bytes, so depth 8 keeps the fp32 ring's shared memory (and bytes in flight) per
+      // warp at three CTAs per SM.  EGC_BWD_RING=4 selects the shallower ring, 0 the register-gather kernel.
+      const int r = ring < 0 ? kBf16RingDepth : ring;
+      if (r > 0 && geo.G == 32 && L.n_ts >= 2)
+        return r >= 8 ? launch_scatter_ring<8, bf16>(s, L.tsmask, task_counter, st) : launch_scatter_ring<4, bf16>(s, L.tsmask, task_counter, st);
+      return geo.G == 32 ? launch_scatter_cols<32, bf16>(s, L.tsmask, task_counter, st) : launch_scatter_cols<16, bf16>(s, L.tsmask, task_counter, st);
+    }
+    const int r = ring < 0 ? 4 : ring;
+    if (r > 0 && geo.G == 32 && L.n_ts >= 2)
+      return r >= 7 ? launch_scatter_ring<7>(s, L.tsmask, task_counter, st) : launch_scatter_ring<4>(s, L.tsmask, task_counter, st);
     return geo.G == 32 ? launch_scatter_cols<32>(s, L.tsmask, task_counter, st) : launch_scatter_cols<16>(s, L.tsmask, task_counter, st);
   }
   if (fuse_merge) EGC_CUDA(cudaMemsetAsync(long_counter, 0, counters_bytes, st));
@@ -291,26 +306,95 @@ int egc_aggregate_fwd(const egc_layer_desc* desc, const int32_t* rowptr, const i
   return EGC_OK;
 }
 
+int egc_aggregate_fwd_bf16(const egc_layer_desc* desc, const int32_t* rowptr, const int32_t* col, const float* val_sym,
+                           const egc_row_plan* plan, const uint16_t* bases, const float* weightings, const float* bias,
+                           const egc_epilogue* epilogue, float* out, float* agg_out, int32_t* arg_out, float* saved,
+                           int32_t* saved_arg, void* workspace, size_t workspace_bytes, void* stream) {
+  if (int rc = validate_desc(desc, "egc_aggregate_fwd_bf16")) return rc;
+  if (int rc = validate_plan(plan, "egc_aggregate_fwd_bf16")) return rc;
+  EGC_REQUIRE(rowptr && col && bases, "egc_aggregate_fwd_bf16: null graph / bases pointer");
+  EGC_REQUIRE(out == nullptr || weightings != nullptr, "egc_aggregate_fwd_bf16: weightings required to produce out");
+  EGC_REQUIRE(out || agg_out || arg_out || saved, "egc_aggregate_fwd_bf16: no output requested");
+  const int mask = prim_mask_of(*desc);
+  EGC_REQUIRE(!(mask & P_SYM) || val_sym != nullptr, "egc_aggregate_fwd_bf16: symnorm requested without val_sym");
+  EGC_REQUIRE(workspace_bytes >= egc_aggregate_fwd_workspace_bytes(desc, plan) && workspace != nullptr,
+              "egc_aggregate_fwd_bf16: workspace too small");
+  const int n_arg = n_arg_slots(*desc);
+  EGC_REQUIRE(saved == nullptr || n_arg == 0 || saved_arg != nullptr, "egc_aggregate_fwd_bf16: saved_arg required with saved for min/max");
+  const int bd = desc->bases * desc->dim, hd = desc->heads * desc->dim;
+  EGC_REQUIRE(bd % 8 == 0 && bd >= 40 && bd <= 128,
+              "egc_aggregate_fwd_bf16: bf16 storage covers basis rows of 40..128 values, a multiple of 8 (B*D = %d)", bd);
+  EGC_REQUIRE(aligned16(bases) && aligned16(out) && aligned16(agg_out) && aligned16(workspace) && aligned16(arg_out) &&
+              aligned16(saved) && aligned16(saved_arg), "egc_aggregate_fwd_bf16: tensors must be 16-byte aligned");
+  EGC_REQUIRE(hd <= ((desc->dim % 4 == 0) ? 512 : 128), "egc_aggregate_fwd_bf16: H*D = %d outputs per row exceed one pass", hd);
+  EGC_REQUIRE(static_cast<int64_t>(desc->n_src) * bd < (int64_t{1} << 32), "egc_aggregate_fwd_bf16: bases exceed 2^32 values");
+  AggParams p{};
+  fill_agg_params(p, *desc, true);
+  p.nvec = bd / 8;                                     // 16-byte pieces of 8 bf16 values
+  p.G = p.nvec > 8 ? 16 : 8;
+  p.n_pass = 1;
+  EGC_REQUIRE(rows_kernel_smem_bytes(p) <= 72 * 1024, "egc_aggregate_fwd_bf16: layer too wide for the row-block staging (%d bytes)",
+              rows_kernel_smem_bytes(p));
+  p.rowptr = rowptr; p.col = col; p.val_sym = val_sym; p.val_lin = nullptr; p.n_rows = desc->n_dst;
+  p.row_map = nullptr;
+  p.n_row_tasks = desc->n_dst;
+  set_plan(p, plan);
+  p.partials = static_cast<float*>(workspace);
+  p.n_slots = n_slots_of_mask(mask);
+  p.long_counter = reinterpret_cast<int*>(static_cast<char*>(workspace) +
+                                          align_up(static_cast<size_t>(p.n_chunks) * p.n_slots * bd * 4, 256));
+  p.bases = reinterpret_cast<const float*>(bases);     // bf16 rows (k_aggregate_rows<.., bf16> reads them as such)
+  p.weightings = weightings; p.bias = bias;
+  if (epilogue != nullptr) {
+    EGC_REQUIRE((epilogue->scale == nullptr) == (epilogue->shift == nullptr), "egc_aggregate_fwd_bf16: epilogue scale and shift come together");
+    EGC_REQUIRE(out != nullptr || (!epilogue->scale && !epilogue->add), "egc_aggregate_fwd_bf16: an epilogue needs the `out` output");
+    EGC_REQUIRE(epilogue->agg_init == nullptr, "egc_aggregate_fwd_bf16: agg_init is not supported");
+    p.epi_scale = epilogue->scale; p.epi_shift = epilogue->shift; p.epi_add = epilogue->add;
+  }
+  EGC_REQUIRE(desc->dim % 4 != 0 || (aligned16(bias) && aligned16(p.epi_scale) && aligned16(p.epi_shift) && aligned16(p.epi_add)),
+              "egc_aggregate_fwd_bf16: bias / epilogue tensors must be 16-byte aligned");
+  p.out = out; p.agg_out = agg_out; p.arg_out = arg_out; p.saved = saved; p.saved_arg = saved_arg;
+  cudaStream_t st = as_stream(stream);
+  const bool want_arg = (arg_out != nullptr || saved_arg != nullptr) && n_arg > 0;
+  if (arg_out != nullptr && !want_arg)                 // no min/max slot: every arg is "none"
+    EGC_CUDA(cudaMemsetAsync(arg_out, 0xff, static_cast<size_t>(desc->n_dst) * desc->n_aggr * bd * sizeof(int32_t), st));
+  p.mode = 0;
+  const size_t counter_off = align_up(static_cast<size_t>(p.n_long) * sizeof(int), 256);
+  int* task_counter = reinterpret_cast<int*>(reinterpret_cast<char*>(p.long_counter) + counter_off);
+  EGC_CUDA(cudaMemsetAsync(p.long_counter, 0, counter_off + sizeof(int), st));
+  const int static_idx = static_cfg_index(*desc);
+  if (static_idx >= 0) return launch_aggregate_rows_bf16_static(static_idx, p, want_arg, task_counter, st);
+  return (p.G == 16 ? launch_aggregate_rows_bf16_g16 : launch_aggregate_rows_bf16_g8)(p, mask, want_arg, task_counter, st);
+}
+
 size_t egc_aggregate_bwd_workspace_bytes(const egc_layer_desc* desc, const egc_row_plan* csc_plan, int32_t flags) {
   (void)flags;
   if (desc == nullptr || prim_mask_of(*desc) <= 0) return 0;
   return bwd_layout(*desc, csc_plan).total;
 }
 
-int egc_aggregate_bwd(const egc_layer_desc* desc, const int32_t* rowptr, const int32_t* col, const float* val_lin,
-                      const int32_t* colptr, const int32_t* rowidx, const int32_t* csr2csc, const float* csc_val_sym,
-                      const float* csc_val_lin, const egc_row_plan* csc_plan, const float* bases,
-                      const float* weightings, const float* saved, const int32_t* saved_arg, const float* grad_out,
-                      const float* out_act, const float* epi_scale, float* d_weightings, float* d_bases, float* d_bias,
-                      float* d_lin_colsum, float* tstreams_out, int32_t flags, int32_t col_split, void* workspace,
-                      size_t workspace_bytes, void* stream) {
+}  // extern "C"
+
+// egc_aggregate_bwd / egc_aggregate_bwd_bf16.  bf16: `bases` points at bf16 rows and the target-side streams are stored as
+// bf16 in the workspace (bwd_layout with 2-byte elements); every other tensor and all arithmetic stay fp32.
+static int aggregate_bwd_impl(const egc_layer_desc* desc, const int32_t* rowptr, const int32_t* col, const float* val_lin,
+                              const int32_t* colptr, const int32_t* rowidx, const int32_t* csr2csc, const float* csc_val_sym,
+                              const float* csc_val_lin, const egc_row_plan* csc_plan, const float* bases,
+                              const float* weightings, const float* saved, const int32_t* saved_arg, const float* grad_out,
+                              const float* out_act, const float* epi_scale, float* d_weightings, float* d_bases, float* d_bias,
+                              float* d_lin_colsum, float* tstreams_out, int32_t flags, int32_t col_split, void* workspace,
+                              size_t workspace_bytes, void* stream, bool bf16_store) {
   if (int rc = validate_desc(desc, "egc_aggregate_bwd")) return rc;
   if (int rc = validate_plan(csc_plan, "egc_aggregate_bwd")) return rc;
   const bool pass1_only = (flags & EGC_BWD_PASS1_ONLY) != 0;
+  EGC_REQUIRE(!bf16_store || (!pass1_only && tstreams_out == nullptr && !(flags & (EGC_BWD_COLS_HEAD | EGC_BWD_COLS_TAIL)) &&
+                              val_lin == nullptr && csc_val_lin == nullptr),
+              "egc_aggregate_bwd_bf16: no column phases, no EGC_BWD_PASS1_ONLY / tstreams_out and no per-entry linear weights");
   EGC_REQUIRE(rowptr && col && bases && weightings && saved && grad_out && d_weightings && workspace &&
               (pass1_only || (colptr && rowidx && d_bases)), "egc_aggregate_bwd: null pointer");
   EGC_REQUIRE((desc->relu != 0) == (out_act != nullptr), "egc_aggregate_bwd: out_act must be given exactly when desc->relu is set");
-  const BwdLayout L = bwd_layout(*desc, csc_plan);
+  const size_t ts_elem = bf16_store ? 2 : 4;
+  const BwdLayout L = bwd_layout(*desc, csc_plan, ts_elem);
   const bool det_route = (flags & EGC_BWD_DETERMINISTIC) != 0 && L.has_route;
   EGC_REQUIRE(!det_route || csr2csc != nullptr, "egc_aggregate_bwd: EGC_BWD_DETERMINISTIC needs csr2csc");
   const int mask = prim_mask_of(*desc);
@@ -320,7 +404,7 @@ int egc_aggregate_bwd(const egc_layer_desc* desc, const int32_t* rowptr, const i
   EGC_REQUIRE((val_lin == nullptr) == (csc_val_lin == nullptr), "egc_aggregate_bwd: val_lin and csc_val_lin must come together");
   EGC_REQUIRE(!((mask & P_SYM) && val_lin), "egc_aggregate_bwd: val_lin cannot be combined with symnorm");
   EGC_REQUIRE(workspace_bytes >= L.total, "egc_aggregate_bwd: workspace too small (%zu < %zu)", workspace_bytes, L.total);
-  EGC_REQUIRE(L.ts_bytes / 4 < (size_t{1} << 32), "egc_aggregate_bwd: target-side streams exceed 2^32 floats");
+  EGC_REQUIRE(L.ts_bytes / ts_elem < (size_t{1} << 32), "egc_aggregate_bwd: target-side streams exceed 2^32 values");
   // Column phases (row-partitioned callers): HEAD = pass 1, routing and pass 2 of the source columns >= col_split (the
   // halo columns, whose partial sums travel to their owners while ...) TAIL = pass 2 of the columns < col_split runs.
   const bool head = (flags & EGC_BWD_COLS_HEAD) != 0, tail = (flags & EGC_BWD_COLS_TAIL) != 0;
@@ -390,9 +474,9 @@ int egc_aggregate_bwd(const egc_layer_desc* desc, const int32_t* rowptr, const i
     c.colsum_part = fuse_colsum ? static_cast<float*>(colsum_ws) : nullptr;
     c.skip_route = skip_route ? 1 : 0;
     c.t_route = t_route;
-#define EGC_LAUNCH_COMBINE_CFG(CFG, EV, LW)                                                                    \
+#define EGC_LAUNCH_COMBINE_CFG(CFG, EV, LW, TS)                                                                \
     {                                                                                                          \
-      auto kern = k_combine_bwd<CFG, EV, LW>;                                                                    \
+      auto kern = k_combine_bwd<CFG, EV, LW, TS>;                                                                \
       if (smem > 48 * 1024) EGC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); \
       LaunchScope egc_ls_("k_combine_bwd", st);                                                                \
       kern<<<grid, kAggThreads, smem, st>>>(c);                                                                \
@@ -406,16 +490,19 @@ int egc_aggregate_bwd(const egc_layer_desc* desc, const int32_t* rowptr, const i
       EGC_REQUIRE(SC::bsm_per_warp == c.sm_per_warp && SC::bsm_saved == c.sm_saved && SC::bsm_arg == c.sm_arg && \
                   SC::ts_sym == c.ts_sym && SC::ts_lin == c.ts_lin && SC::ts_sq == c.ts_sq,                    \
                   "egc_aggregate_bwd: static configuration %d disagrees with the host layout", I);             \
-      EGC_LAUNCH_COMBINE_CFG(SC, 4, false)                                                                     \
+      if (bf16_store) EGC_LAUNCH_COMBINE_CFG(SC, 4, false, bf16)                                               \
+      else EGC_LAUNCH_COMBINE_CFG(SC, 4, false, float)                                                                \
       launched = true;                                                                                         \
     }
     EGC_STATIC_CFGS(X)
 #undef X
     if (launched) {
-    } else if (ev4 && !linw) EGC_LAUNCH_COMBINE_CFG(Dyn, 4, false)
-    else if (ev4 && linw) EGC_LAUNCH_COMBINE_CFG(Dyn, 4, true)
-    else if (!linw) EGC_LAUNCH_COMBINE_CFG(Dyn, 1, false)
-    else EGC_LAUNCH_COMBINE_CFG(Dyn, 1, true)
+    } else if (bf16_store && ev4) EGC_LAUNCH_COMBINE_CFG(Dyn, 4, false, bf16)
+    else if (bf16_store) EGC_LAUNCH_COMBINE_CFG(Dyn, 1, false, bf16)
+    else if (ev4 && !linw) EGC_LAUNCH_COMBINE_CFG(Dyn, 4, false, float)
+    else if (ev4 && linw) EGC_LAUNCH_COMBINE_CFG(Dyn, 4, true, float)
+    else if (!linw) EGC_LAUNCH_COMBINE_CFG(Dyn, 1, false, float)
+    else EGC_LAUNCH_COMBINE_CFG(Dyn, 1, true, float)
 #undef EGC_LAUNCH_COMBINE_CFG
     EGC_LAUNCH_CHECK("k_combine_bwd");
     if (fuse_colsum) {
@@ -471,7 +558,7 @@ int egc_aggregate_bwd(const egc_layer_desc* desc, const int32_t* rowptr, const i
   // ---- pass 2: per source column (CSC), atomic-free
   if (L.tsmask != 0 && !pass1_only) {
     if (int rc = run_pass2(*desc, L, colptr, rowidx, csc_val_sym, csc_val_lin, csc_plan, tstreams, bases, d_bases,
-                           head ? col_split : 0, tail ? col_split : desc->n_src, pass2_accumulates, csc_part, vec4, st))
+                           head ? col_split : 0, tail ? col_split : desc->n_src, pass2_accumulates, csc_part, vec4, st, bf16_store))
       return rc;
   }
 
@@ -490,6 +577,38 @@ int egc_aggregate_bwd(const egc_layer_desc* desc, const int32_t* rowptr, const i
     }
   }
   return EGC_OK;
+}
+
+extern "C" {
+
+int egc_aggregate_bwd(const egc_layer_desc* desc, const int32_t* rowptr, const int32_t* col, const float* val_lin,
+                      const int32_t* colptr, const int32_t* rowidx, const int32_t* csr2csc, const float* csc_val_sym,
+                      const float* csc_val_lin, const egc_row_plan* csc_plan, const float* bases,
+                      const float* weightings, const float* saved, const int32_t* saved_arg, const float* grad_out,
+                      const float* out_act, const float* epi_scale, float* d_weightings, float* d_bases, float* d_bias,
+                      float* d_lin_colsum, float* tstreams_out, int32_t flags, int32_t col_split, void* workspace,
+                      size_t workspace_bytes, void* stream) {
+  return aggregate_bwd_impl(desc, rowptr, col, val_lin, colptr, rowidx, csr2csc, csc_val_sym, csc_val_lin, csc_plan, bases,
+                            weightings, saved, saved_arg, grad_out, out_act, epi_scale, d_weightings, d_bases, d_bias,
+                            d_lin_colsum, tstreams_out, flags, col_split, workspace, workspace_bytes, stream, false);
+}
+
+size_t egc_aggregate_bwd_bf16_workspace_bytes(const egc_layer_desc* desc, const egc_row_plan* csc_plan, int32_t flags) {
+  (void)flags;
+  if (desc == nullptr || prim_mask_of(*desc) <= 0) return 0;
+  return bwd_layout(*desc, csc_plan, 2).total;
+}
+
+int egc_aggregate_bwd_bf16(const egc_layer_desc* desc, const int32_t* rowptr, const int32_t* col, const int32_t* colptr,
+                           const int32_t* rowidx, const int32_t* csr2csc, const float* csc_val_sym, const egc_row_plan* csc_plan,
+                           const uint16_t* bases, const float* weightings, const float* saved, const int32_t* saved_arg,
+                           const float* grad_out, const float* out_act, const float* epi_scale, float* d_weightings,
+                           float* d_bases, float* d_bias, float* d_lin_colsum, int32_t flags, void* workspace,
+                           size_t workspace_bytes, void* stream) {
+  return aggregate_bwd_impl(desc, rowptr, col, nullptr, colptr, rowidx, csr2csc, csc_val_sym, nullptr, csc_plan,
+                            reinterpret_cast<const float*>(bases), weightings, saved, saved_arg, grad_out, out_act, epi_scale,
+                            d_weightings, d_bases, d_bias, d_lin_colsum, nullptr, flags, 0, workspace, workspace_bytes, stream,
+                            true);
 }
 
 size_t egc_aggregate_bwd_cols_workspace_bytes(const egc_layer_desc* desc, const egc_row_plan* csc_plan) {

@@ -15,6 +15,7 @@
 #pragma once
 
 #include "aggregate_fast.cuh"
+#include "bf16.cuh"
 
 namespace egc {
 
@@ -41,13 +42,63 @@ struct RowsSmem {                          // per-warp layout in floats, from A 
   }
 };
 
-template <class Cfg, bool ARG>
+// One 16-byte gather per lane and neighbour: 4 fp32 or 8 bf16 basis values (ST = the storage type of `bases`; p.bases
+// then points at bf16 rows and p.nvec counts 8-wide pieces).  Values are widened to fp32 before any arithmetic.
+template <class ST>
+struct RowPiece {
+  using T = float4;
+  static constexpr int V = 4;
+  static __device__ __forceinline__ T load(const ST* p, uint64_t pol) { return ldg_f4_hint(p, pol); }
+};
+template <>
+struct RowPiece<bf16> {
+  using T = uint4;
+  static constexpr int V = 8;
+  static __device__ __forceinline__ T load(const bf16* p, uint64_t pol) {
+    uint4 v;
+    asm volatile("ld.global.nc.L2::cache_hint.v4.u32 {%0, %1, %2, %3}, [%4], %5;"
+                 : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p), "l"(pol));
+    return v;
+  }
+};
+
+template <int MASK, bool ARG>
+__device__ __forceinline__ void add_edge(Acc<MASK, 8, false, ARG>& acc, const uint4& xv, float vs, int e) {
+  const float x[8] = {bf16_lo(xv.x), bf16_hi(xv.x), bf16_lo(xv.y), bf16_hi(xv.y),
+                      bf16_lo(xv.z), bf16_hi(xv.z), bf16_lo(xv.w), bf16_hi(xv.w)};
+#pragma unroll
+  for (int k = 0; k < 8; ++k) {          // the operations of add_edge<4> (aggregate_fast.cuh), per feature
+    if constexpr (MASK & P_SUM) acc.sum[k] = __fadd_rn(acc.sum[k], x[k]);
+    if constexpr (MASK & P_SQ) acc.sq[k] = fmaf(x[k], x[k], acc.sq[k]);
+    if constexpr (MASK & P_SYM) acc.sym[k] = __fadd_rn(acc.sym[k], __fmul_rn(x[k], vs));
+    if constexpr (MASK & P_MAX) {
+      if constexpr (ARG) { if (x[k] > acc.mx[k]) { acc.mx[k] = x[k]; acc.amx[k] = e; } }
+      else acc.mx[k] = fmaxf(acc.mx[k], x[k]);
+    }
+    if constexpr (MASK & P_MIN) {
+      if constexpr (ARG) { if (x[k] < acc.mn[k]) { acc.mn[k] = x[k]; acc.amn[k] = e; } }
+      else acc.mn[k] = fminf(acc.mn[k], x[k]);
+    }
+  }
+}
+
+// bf16 geometry of a layer configuration: 8-wide pieces, G = lanes per basis row (8 or 16 for rows of 40..128 values)
+template <class Cfg>
+struct Bf16Cfg : Cfg {
+  static constexpr int nvec = Cfg::BD / 8;
+  static constexpr int G = nvec > 8 ? 16 : 8;
+  static_assert(Cfg::BD % 8 == 0 && nvec <= 16, "Bf16Cfg: basis rows of at most 128 values, a multiple of 8");
+};
+
+template <class Cfg, bool ARG, class ST = float>
 __global__ void __launch_bounds__(kAggThreads, EGC_ROWS_CTAS) k_aggregate_rows(const __grid_constant__ AggParams p, int* __restrict__ task_counter) {
   extern __shared__ __align__(16) float smem_all[];
   constexpr int MASK = Cfg::MASK, G = Cfg::G;
   using GC = Get<Cfg>;
   constexpr int NG = 32 / G;
   constexpr int U = EGC_ROWS_UNROLL;
+  using PC = RowPiece<ST>;
+  constexpr int V = PC::V;                                      // features per lane
   constexpr int STEP = U * NG;                                  // nnz consumed by one batch of the warp
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const RowsSmem lay(GC::A(p) * GC::BD(p), GC::HAB(p));
@@ -58,11 +109,11 @@ __global__ void __launch_bounds__(kAggThreads, EGC_ROWS_CTAS) k_aggregate_rows(c
   float* s_val = sm + lay.val;
   const int g = lane / G, li = lane & (G - 1);
   const bool writer = li < GC::nvec(p) && lane < G;                  // lanes of group 0 that own a real piece
-  const int foff = min(li, GC::nvec(p) - 1) * 4;                     // idle lanes shadow the last piece, never write
-  const float* __restrict__ src = p.bases + foff;
+  const int foff = min(li, GC::nvec(p) - 1) * V;                     // idle lanes shadow the last piece, never write
+  const ST* __restrict__ src = reinterpret_cast<const ST*>(p.bases) + foff;
   const uint32_t BD = static_cast<uint32_t>(GC::BD(p));
   const uint64_t pol_keep = l2_policy_keep(), pol_stream = l2_policy_stream();
-  using AccT = Acc<MASK, 4, false, ARG>;
+  using AccT = Acc<MASK, V, false, ARG>;
   const bool stage_w = p.out != nullptr;
 
   // epilogue geometry of this lane: outputs o = lane * EV + 32 * EV * it  ->  (weight row, offset in the head)
@@ -83,68 +134,81 @@ __global__ void __launch_bounds__(kAggThreads, EGC_ROWS_CTAS) k_aggregate_rows(c
       const bool nonempty = end > begin;
       const float cntf = static_cast<float>(max(end - begin, 1));   // mean divides by the nnz count, min 1
       const float inv = __frcp_rn(cntf);
-      float mean[4] = {0.f, 0.f, 0.f, 0.f}, var[4] = {0.f, 0.f, 0.f, 0.f};
+      float mean[V], var[V];
+#pragma unroll
+      for (int k = 0; k < V; ++k) { mean[k] = 0.f; var[k] = 0.f; }
       if constexpr ((MASK & P_SUM) != 0) {
 #pragma unroll
-        for (int k = 0; k < 4; ++k) mean[k] = div_by(acc.sum[k], cntf, inv);
+        for (int k = 0; k < V; ++k) mean[k] = div_by(acc.sum[k], cntf, inv);
       }
       if constexpr ((MASK & P_SQ) != 0) {
 #pragma unroll
-        for (int k = 0; k < 4; ++k)      // mean_sq - mean * mean, ref :242 / :271
+        for (int k = 0; k < V; ++k)      // mean_sq - mean * mean, ref :242 / :271
           var[k] = __fsub_rn(div_by(acc.sq[k], cntf, inv), __fmul_rn(mean[k], mean[k]));
       }
       const size_t row_s = static_cast<size_t>(row);
 #pragma unroll
       for (int a = 0; a < GC::A(p); ++a) {
         const int code = GC::aggr(p, a);
-        float v[4] = {0.f, 0.f, 0.f, 0.f}, sv[4];
-        int arg[4] = {-1, -1, -1, -1};
+        float v[V], sv[V];
+        int arg[V];
+#pragma unroll
+        for (int k = 0; k < V; ++k) { v[k] = 0.f; arg[k] = -1; }
         bool gate_sign = false;
         switch (code) {
           case EGC_AGGR_SUM:
-            if constexpr ((MASK & P_SUM) != 0) { for (int k = 0; k < 4; ++k) v[k] = acc.sum[k]; }
+            if constexpr ((MASK & P_SUM) != 0) { for (int k = 0; k < V; ++k) v[k] = acc.sum[k]; }
             break;
           case EGC_AGGR_MEAN:
-            if constexpr ((MASK & P_SUM) != 0) { for (int k = 0; k < 4; ++k) v[k] = mean[k]; }
+            if constexpr ((MASK & P_SUM) != 0) { for (int k = 0; k < V; ++k) v[k] = mean[k]; }
             break;
           case EGC_AGGR_SYMNORM:
-            if constexpr ((MASK & P_SYM) != 0) { for (int k = 0; k < 4; ++k) v[k] = acc.sym[k]; }
+            if constexpr ((MASK & P_SYM) != 0) { for (int k = 0; k < V; ++k) v[k] = acc.sym[k]; }
             break;
           case EGC_AGGR_MAX:
             if constexpr ((MASK & P_MAX) != 0) {
-              for (int k = 0; k < 4; ++k) { v[k] = nonempty ? acc.mx[k] : 0.f; if constexpr (ARG) arg[k] = acc.amx[k]; }
+              for (int k = 0; k < V; ++k) { v[k] = nonempty ? acc.mx[k] : 0.f; if constexpr (ARG) arg[k] = acc.amx[k]; }
             }
             break;
           case EGC_AGGR_MIN:
             if constexpr ((MASK & P_MIN) != 0) {
-              for (int k = 0; k < 4; ++k) { v[k] = nonempty ? acc.mn[k] : 0.f; if constexpr (ARG) arg[k] = acc.amn[k]; }
+              for (int k = 0; k < V; ++k) { v[k] = nonempty ? acc.mn[k] : 0.f; if constexpr (ARG) arg[k] = acc.amn[k]; }
             }
             break;
           case EGC_AGGR_VAR:
-            if constexpr ((MASK & P_SQ) != 0) { for (int k = 0; k < 4; ++k) v[k] = var[k]; }
+            if constexpr ((MASK & P_SQ) != 0) { for (int k = 0; k < V; ++k) v[k] = var[k]; }
             break;
           case EGC_AGGR_STD:
             if constexpr ((MASK & P_SQ) != 0) {       // sqrt(relu(var) + 1e-5), ref :244 / :273
-              for (int k = 0; k < 4; ++k) v[k] = sqrtf(__fadd_rn(fmaxf(var[k], 0.f), kStdEps));
+              for (int k = 0; k < V; ++k) v[k] = sqrtf(__fadd_rn(fmaxf(var[k], 0.f), kStdEps));
               gate_sign = true;
             }
             break;
         }
 #pragma unroll
-        for (int k = 0; k < 4; ++k) sv[k] = (gate_sign && !(var[k] > 0.f)) ? -v[k] : v[k];   // sign bit = relu gate closed
-        if (p.out != nullptr) st_row<4>(s_agg + a * BD + foff, v);
-        if (p.agg_out != nullptr) stg_f4_hint(p.agg_out + (row_s * GC::A(p) + a) * BD + foff, v, pol_stream);
-        if (p.saved != nullptr) stg_f4_hint(p.saved + (row_s * GC::n_saved(p) + a) * BD + foff, sv, pol_stream);
-        if constexpr (ARG) {
-          const float t[4] = {__int_as_float(arg[0]), __int_as_float(arg[1]), __int_as_float(arg[2]), __int_as_float(arg[3])};
-          if (p.arg_out != nullptr)
-            stg_f4_hint(reinterpret_cast<float*>(p.arg_out) + (row_s * GC::A(p) + a) * BD + foff, t, pol_stream);
-          if (p.saved_arg != nullptr && GC::arg_slot(p, a) >= 0)
-            stg_f4_hint(reinterpret_cast<float*>(p.saved_arg) + (row_s * GC::n_arg(p) + GC::arg_slot(p, a)) * BD + foff, t, pol_stream);
+        for (int k = 0; k < V; ++k) sv[k] = (gate_sign && !(var[k] > 0.f)) ? -v[k] : v[k];   // sign bit = relu gate closed
+#pragma unroll
+        for (int h = 0; h < V; h += 4) {                     // 4 features per 128-bit store
+          const float(&v4)[4] = *reinterpret_cast<const float(*)[4]>(v + h);
+          const float(&sv4)[4] = *reinterpret_cast<const float(*)[4]>(sv + h);
+          if (p.out != nullptr) st_row<4>(s_agg + a * BD + foff + h, v4);
+          if (p.agg_out != nullptr) stg_f4_hint(p.agg_out + (row_s * GC::A(p) + a) * BD + foff + h, v4, pol_stream);
+          if (p.saved != nullptr) stg_f4_hint(p.saved + (row_s * GC::n_saved(p) + a) * BD + foff + h, sv4, pol_stream);
+          if constexpr (ARG) {
+            const float t[4] = {__int_as_float(arg[h]), __int_as_float(arg[h + 1]), __int_as_float(arg[h + 2]), __int_as_float(arg[h + 3])};
+            if (p.arg_out != nullptr)
+              stg_f4_hint(reinterpret_cast<float*>(p.arg_out) + (row_s * GC::A(p) + a) * BD + foff + h, t, pol_stream);
+            if (p.saved_arg != nullptr && GC::arg_slot(p, a) >= 0)
+              stg_f4_hint(reinterpret_cast<float*>(p.saved_arg) + (row_s * GC::n_arg(p) + GC::arg_slot(p, a)) * BD + foff + h, t, pol_stream);
+          }
         }
       }
       if constexpr ((MASK & P_SQ) != 0) {
-        if (p.saved != nullptr && GC::n_saved(p) > GC::A(p)) stg_f4_hint(p.saved + (row_s * GC::n_saved(p) + GC::A(p)) * BD + foff, mean, pol_stream);
+#pragma unroll
+        for (int h = 0; h < V; h += 4) {
+          const float(&m4)[4] = *reinterpret_cast<const float(*)[4]>(mean + h);
+          if (p.saved != nullptr && GC::n_saved(p) > GC::A(p)) stg_f4_hint(p.saved + (row_s * GC::n_saved(p) + GC::A(p)) * BD + foff + h, m4, pol_stream);
+        }
       }
     }
     if (p.out == nullptr) return;
@@ -215,7 +279,7 @@ __global__ void __launch_bounds__(kAggThreads, EGC_ROWS_CTAS) k_aggregate_rows(c
           if constexpr (MASK & P_SYM) my_vs = __ldg(p.val_sym + e0 + lane);
         }
         for (int u0 = 0; u0 < cnt; u0 += STEP) {
-          float4 x[U];
+          typename PC::T x[U];
           float vs[U];
 #pragma unroll
           for (int t = 0; t < U; ++t) {
@@ -223,7 +287,7 @@ __global__ void __launch_bounds__(kAggThreads, EGC_ROWS_CTAS) k_aggregate_rows(c
             const uint32_t j = static_cast<uint32_t>(__shfl_sync(kFull, my_col, u));
             vs[t] = 0.f;
             if constexpr (MASK & P_SYM) vs[t] = __shfl_sync(kFull, my_vs, u);
-            x[t] = ldg_f4_hint(src + static_cast<size_t>(j * BD), pol_keep);
+            x[t] = PC::load(src + static_cast<size_t>(j * BD), pol_keep);
           }
 #pragma unroll
           for (int t = 0; t < U; ++t) {
@@ -337,13 +401,13 @@ __global__ void __launch_bounds__(kAggThreads, EGC_ROWS_CTAS) k_aggregate_rows(c
       __syncwarp();
 
       // gathers of one batch: positions b + t * NG + g clamped to the row's last nnz; wofs maps nnz position -> window
-      float4 x[U];
+      typename PC::T x[U];
       auto issue = [&](int b, int e, int wofs) {
 #pragma unroll
         for (int t = 0; t < U; ++t) {
           const int pos = min(b + t * NG + g, e - 1);
           const uint32_t j = static_cast<uint32_t>(s_col[pos + wofs]);
-          x[t] = ldg_f4_hint(src + static_cast<size_t>(j * BD), pol_keep);
+          x[t] = PC::load(src + static_cast<size_t>(j * BD), pol_keep);
         }
       };
       int b = __shfl_sync(kFull, rp, ri), e = __shfl_sync(kFull, rpn, ri);
@@ -414,11 +478,11 @@ inline int pick_rows_per_task(int n_row_tasks) {
   return rpt;
 }
 
-template <class Cfg, bool ARG>
+template <class Cfg, bool ARG, class ST = float>
 int launch_rows_one(const AggParams& p_in, int* task_counter, cudaStream_t st) {
   AggParams p = p_in;
   p.rows_per_task = pick_rows_per_task(p.n_row_tasks);
-  auto kern = k_aggregate_rows<Cfg, ARG>;
+  auto kern = k_aggregate_rows<Cfg, ARG, ST>;
   const int smem_bytes = rows_smem_bytes(p);
   if (smem_bytes > 48 * 1024) {
     EGC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
@@ -434,18 +498,18 @@ int launch_rows_one(const AggParams& p_in, int* task_counter, cudaStream_t st) {
   return EGC_OK;
 }
 
-template <class Cfg>
+template <class Cfg, class ST = float>
 int launch_rows_arg(const AggParams& p, bool arg, int* task_counter, cudaStream_t st) {
   if constexpr ((Cfg::MASK & (P_MAX | P_MIN)) != 0) {
-    if (arg) return launch_rows_one<Cfg, true>(p, task_counter, st);
+    if (arg) return launch_rows_one<Cfg, true, ST>(p, task_counter, st);
   }
-  return launch_rows_one<Cfg, false>(p, task_counter, st);
+  return launch_rows_one<Cfg, false, ST>(p, task_counter, st);
 }
 
-template <int G>
+template <int G, class ST = float>
 int launch_rows_family(const AggParams& p, int mask, bool arg, int* task_counter, cudaStream_t st) {
   switch (mask) {
-#define X(M) case M: return launch_rows_arg<DynCfg<M, G>>(p, arg, task_counter, st);
+#define X(M) case M: return launch_rows_arg<DynCfg<M, G>, ST>(p, arg, task_counter, st);
     EGC_FAST_MASK_CASES(X)
 #undef X
   }

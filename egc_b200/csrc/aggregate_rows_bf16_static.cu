@@ -1,0 +1,17 @@
+// Instantiates the row-block forward aggregation kernel (aggregate_rows.cuh) with bf16 basis rows for the specialised
+// layer shapes.
+#include <algorithm>
+
+#include "aggregate_rows.cuh"
+
+namespace egc {
+int launch_aggregate_rows_bf16_static(int cfg_index, const AggParams& p, bool arg, int* task_counter, cudaStream_t st) {
+  switch (cfg_index) {
+#define X(I, ...) case I: return launch_rows_arg<Bf16Cfg<StaticCfg<__VA_ARGS__>>, bf16>(p, arg, task_counter, st);
+    EGC_STATIC_CFGS(X)
+#undef X
+  }
+  set_error("aggregate: unknown static configuration %d", cfg_index);
+  return EGC_ERR_UNSUPPORTED;
+}
+}  // namespace egc

@@ -3,6 +3,7 @@
 #pragma once
 
 #include "aggregate_fast.cuh"
+#include "bf16.cuh"
 #include "colsum.cuh"
 
 namespace egc {
@@ -62,7 +63,8 @@ __device__ __forceinline__ void stg_stream_f4(float* p, const float (&v)[4]) {
 // once per CTA into shared-memory tables.  The column sums of grad_out (d_bias) and of d_weightings (the
 // gradient of the comb-weight bias) ride along in registers and leave as one partial row per CTA
 // (deterministic: reduced in CTA order by k_colsum_partials).
-template <class Cfg, int EV, bool LINW>
+// TS = storage type of the target-side streams (p.tstreams then points at bf16 rows, rounded to nearest even).
+template <class Cfg, int EV, bool LINW, class TS = float>
 __global__ void __launch_bounds__(kAggThreads, 4) k_combine_bwd(const __grid_constant__ CombineBwdParams p) {
   using GB = GetB<Cfg, CombineBwdParams>;
   extern __shared__ __align__(16) float smem_all[];
@@ -190,7 +192,7 @@ __global__ void __launch_bounds__(kAggThreads, 4) k_combine_bwd(const __grid_con
     }
 
     // (2) gradient w.r.t. the aggregates -> target-side streams and min/max routing
-    float* ts = p.tstreams + static_cast<int64_t>(row) * p.ts_row_stride;
+    TS* ts = reinterpret_cast<TS*>(p.tstreams) + static_cast<int64_t>(row) * p.ts_row_stride;
     for (int p0 = lane * EV; p0 < BD; p0 += 32 * EV) {
       const int b = p0 / D, d = p0 - b * D;
       float t_sym[EV], t_lin[EV], t_sq[EV];
@@ -239,10 +241,19 @@ __global__ void __launch_bounds__(kAggThreads, 4) k_combine_bwd(const __grid_con
         }
       }
       // plain (L2 write-back) stores: pass 2 gathers these rows next, whatever part of them survives in the L2 is a hit
-      float* tsp = ts + p0;
-      if (GB::ts_sym(p) >= 0) st_row<EV>(tsp + static_cast<int64_t>(GB::ts_sym(p)) * p.ts_stream_stride, t_sym);
-      if (GB::ts_lin(p) >= 0) st_row<EV>(tsp + static_cast<int64_t>(GB::ts_lin(p)) * p.ts_stream_stride, t_lin);
-      if (GB::ts_sq(p) >= 0) st_row<EV>(tsp + static_cast<int64_t>(GB::ts_sq(p)) * p.ts_stream_stride, t_sq);
+      TS* tsp = ts + p0;
+      if constexpr (kBf16<TS>) {
+        auto st_ts = [&](TS* q, const float (&v)[EV]) {
+          if constexpr (EV == 4) st4<TS>(q, v); else st1<TS>(q, v[0]);
+        };
+        if (GB::ts_sym(p) >= 0) st_ts(tsp + static_cast<int64_t>(GB::ts_sym(p)) * p.ts_stream_stride, t_sym);
+        if (GB::ts_lin(p) >= 0) st_ts(tsp + static_cast<int64_t>(GB::ts_lin(p)) * p.ts_stream_stride, t_lin);
+        if (GB::ts_sq(p) >= 0) st_ts(tsp + static_cast<int64_t>(GB::ts_sq(p)) * p.ts_stream_stride, t_sq);
+      } else {
+        if (GB::ts_sym(p) >= 0) st_row<EV>(tsp + static_cast<int64_t>(GB::ts_sym(p)) * p.ts_stream_stride, t_sym);
+        if (GB::ts_lin(p) >= 0) st_row<EV>(tsp + static_cast<int64_t>(GB::ts_lin(p)) * p.ts_stream_stride, t_lin);
+        if (GB::ts_sq(p) >= 0) st_row<EV>(tsp + static_cast<int64_t>(GB::ts_sq(p)) * p.ts_stream_stride, t_sq);
+      }
     }
     __syncwarp();     // the next row overwrites this warp's staging area
   }

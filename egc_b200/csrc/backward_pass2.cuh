@@ -3,6 +3,7 @@
 #pragma once
 
 #include "aggregate_fast.cuh"
+#include "bf16.cuh"
 
 namespace egc {
 
@@ -254,7 +255,21 @@ constexpr int kColsPerTask = 8;
 constexpr int kColWindow = 384;
 static_assert(kColWindow >= EGC_CHUNK_EDGES, "a normal column must fit the staging window");
 
-template <int TSMASK, int G, bool HINT = false>
+// four stored stream values -> fp32, with an L2 eviction hint
+template <class ST>
+__device__ __forceinline__ float4 ldg4_hint(const ST* p, uint64_t pol) {
+  if constexpr (kBf16<ST>) {
+    uint2 v;
+    asm volatile("ld.global.nc.L2::cache_hint.v2.u32 {%0, %1}, [%2], %3;" : "=r"(v.x), "=r"(v.y) : "l"(p), "l"(pol));
+    return widen_bf16x4(v);
+  } else {
+    return ldg_f4_hint(p, pol);
+  }
+}
+
+// ST = storage type of the target-side streams and of `bases` (bf16: p.tstreams / p.bases point at bf16 rows; a lane still
+// owns 4 features and sums them in fp32 in the same order)
+template <int TSMASK, int G, bool HINT = false, class ST = float>
 __global__ void __launch_bounds__(kAggThreads, (TSMASK & (TSMASK - 1)) == 0 ? 4 : 3) k_scatter_cols(const __grid_constant__ ScatterParams p, int* __restrict__ task_counter) {
   __shared__ int s_idx_all[kAggWarps][kColWindow];
   __shared__ float s_val_all[kAggWarps][(TSMASK & 1) ? kColWindow : 1];
@@ -268,9 +283,9 @@ __global__ void __launch_bounds__(kAggThreads, (TSMASK & (TSMASK - 1)) == 0 ? 4 
   const int foff = min(piece, p.nvec - 1) * 4;
   const uint32_t row_stride = static_cast<uint32_t>(p.ts_row_stride);   // n_dst * row_stride < 2^32 (checked by the host)
   const int64_t part_stride = static_cast<int64_t>(p.n_ts) * p.BD;
-  const float* __restrict__ src_sym = p.tstreams + p.off_sym + foff;
-  const float* __restrict__ src_lin = p.tstreams + p.off_lin + foff;
-  const float* __restrict__ src_sq = p.tstreams + p.off_sq + foff;
+  const ST* __restrict__ src_sym = reinterpret_cast<const ST*>(p.tstreams) + p.off_sym + foff;
+  const ST* __restrict__ src_lin = reinterpret_cast<const ST*>(p.tstreams) + p.off_lin + foff;
+  const ST* __restrict__ src_sq = reinterpret_cast<const ST*>(p.tstreams) + p.off_sq + foff;
   float a_sym[4], a_lin[4], a_sq[4];
 
   auto stage = [&](int wb, int we) {                           // entries [wb, we) -> shared memory (we - wb <= kColWindow)
@@ -298,9 +313,9 @@ __global__ void __launch_bounds__(kAggThreads, (TSMASK & (TSMASK - 1)) == 0 ? 4 
           const uint64_t pol = abs(ti - colj) <= p.near_rows ? pol_near : pol_far;
           m[u] = q < e ? 1.f : 0.f;
           vs[u] = 0.f;
-          if constexpr ((TSMASK & 1) != 0) { vs[u] = q < e ? s_val[qc - wb] : 0.f; xs[u] = ldg_f4_hint(src_sym + r, pol); }
-          if constexpr ((TSMASK & 2) != 0) xl[u] = ldg_f4_hint(src_lin + r, pol);
-          if constexpr ((TSMASK & 4) != 0) xq[u] = ldg_f4_hint(src_sq + r, pol);
+          if constexpr ((TSMASK & 1) != 0) { vs[u] = q < e ? s_val[qc - wb] : 0.f; xs[u] = ldg4_hint<ST>(src_sym + r, pol); }
+          if constexpr ((TSMASK & 2) != 0) xl[u] = ldg4_hint<ST>(src_lin + r, pol);
+          if constexpr ((TSMASK & 4) != 0) xq[u] = ldg4_hint<ST>(src_sq + r, pol);
         }
       } else {
 #pragma unroll
@@ -309,9 +324,9 @@ __global__ void __launch_bounds__(kAggThreads, (TSMASK & (TSMASK - 1)) == 0 ? 4 
         const size_t r = static_cast<size_t>(static_cast<uint32_t>(s_idx[qc - wb]) * row_stride);
         m[u] = q < e ? 1.f : 0.f;
         vs[u] = 0.f;
-        if constexpr ((TSMASK & 1) != 0) { vs[u] = q < e ? s_val[qc - wb] : 0.f; xs[u] = __ldg(reinterpret_cast<const float4*>(src_sym + r)); }
-        if constexpr ((TSMASK & 2) != 0) xl[u] = __ldg(reinterpret_cast<const float4*>(src_lin + r));
-        if constexpr ((TSMASK & 4) != 0) xq[u] = __ldg(reinterpret_cast<const float4*>(src_sq + r));
+        if constexpr ((TSMASK & 1) != 0) { vs[u] = q < e ? s_val[qc - wb] : 0.f; xs[u] = ldg4<ST>(src_sym + r); }
+        if constexpr ((TSMASK & 2) != 0) xl[u] = ldg4<ST>(src_lin + r);
+        if constexpr ((TSMASK & 4) != 0) xq[u] = ldg4<ST>(src_sq + r);
       }
       }
 #pragma unroll
@@ -347,7 +362,7 @@ __global__ void __launch_bounds__(kAggThreads, (TSMASK & (TSMASK - 1)) == 0 ? 4 
     if (p.routed) ld_plain<4>(r, dst);
     if constexpr ((TSMASK & 4) != 0) {
       float xj[4];
-      ld_row<4>(xj, p.bases + static_cast<int64_t>(colj) * p.BD + foff);
+      ldg4<ST>(xj, reinterpret_cast<const ST*>(p.bases) + static_cast<int64_t>(colj) * p.BD + foff);
 #pragma unroll
       for (int k = 0; k < 4; ++k) r[k] += 2.f * xj[k] * a_sq[k];
     }
@@ -451,7 +466,7 @@ __global__ void __launch_bounds__(kAggThreads, (TSMASK & (TSMASK - 1)) == 0 ? 4 
   }
 }
 
-template <int G>
+template <int G, class ST = float>
 static int launch_scatter_cols(const ScatterParams& p_in, int tsmask, int* task_counter, cudaStream_t st) {
   ScatterParams p = p_in;
   const int resident = (tsmask & (tsmask - 1)) == 0 ? 4 : 3;     // CTAs per SM, as the launch bounds
@@ -467,8 +482,8 @@ static int launch_scatter_cols(const ScatterParams& p_in, int tsmask, int* task_
     LaunchScope egc_ls_("k_scatter_bwd", st);
 #define EGC_SCATTER_COLS_CASE(M)                                                                           \
       case M:                                                                                              \
-        if (p.near_rows > 0) k_scatter_cols<M, G, true><<<grid, kAggThreads, 0, st>>>(p, task_counter);    \
-        else k_scatter_cols<M, G, false><<<grid, kAggThreads, 0, st>>>(p, task_counter);                   \
+        if (p.near_rows > 0) k_scatter_cols<M, G, true, ST><<<grid, kAggThreads, 0, st>>>(p, task_counter); \
+        else k_scatter_cols<M, G, false, ST><<<grid, kAggThreads, 0, st>>>(p, task_counter);                \
         break;
     switch (tsmask) {
       EGC_SCATTER_COLS_CASE(1) EGC_SCATTER_COLS_CASE(2) EGC_SCATTER_COLS_CASE(3) EGC_SCATTER_COLS_CASE(4)

@@ -12,6 +12,8 @@
 //     in the same order as k_scatter_cols, then the freed slot takes entry q + R;
 //   * a lane only ever reads what it wrote itself: no barrier, no bank conflict (lane l owns bytes [16 l, 16 l + 16)).
 // Task model, chunk partials of long columns, the ordered merge and the epilogue are those of k_scatter_cols.
+// bf16 streams (ST = bf16): a lane's piece is 8 bytes (4 features, still one lane per 4 features), a stream row 256 bytes,
+// so a slot holds half the bytes and the same shared memory holds twice the ring depth.
 #pragma once
 
 #include "backward_pass2.cuh"
@@ -22,6 +24,9 @@ namespace egc {
 __device__ __forceinline__ void cp_async_16_hint(uint32_t smem_dst, const void* gmem_src, uint64_t pol) {
   asm volatile("cp.async.cg.shared.global.L2::cache_hint [%0], [%1], 16, %2;\n" ::"r"(smem_dst), "l"(gmem_src), "l"(pol) : "memory");
 }
+__device__ __forceinline__ void cp_async_8_hint(uint32_t smem_dst, const void* gmem_src, uint64_t pol) {
+  asm volatile("cp.async.ca.shared.global.L2::cache_hint [%0], [%1], 8, %2;\n" ::"r"(smem_dst), "l"(gmem_src), "l"(pol) : "memory");
+}
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;\n" ::: "memory"); }
 template <int N>
 __device__ __forceinline__ void cp_async_wait_group() { asm volatile("cp.async.wait_group %0;\n" ::"n"(N) : "memory"); }
@@ -31,32 +36,35 @@ __device__ __forceinline__ uint64_t l2_policy_normal() {
   return pol;
 }
 
-template <int TSMASK, int R>
+template <int TSMASK, int R, class ST = float>
 struct RingLayout {
   static constexpr int NS = (TSMASK & 1) + ((TSMASK >> 1) & 1) + ((TSMASK >> 2) & 1);
-  static constexpr int kSlotBytes = NS * 512;
+  static constexpr int kPieceBytes = 4 * static_cast<int>(sizeof(ST));   // one lane's 4 features of one stream
+  static constexpr int kRowBytes = 32 * kPieceBytes;
+  static constexpr int kSlotBytes = NS * kRowBytes;
   static constexpr int kIdxBytes = kColWindow * 4;
   static constexpr int kValBytes = (TSMASK & 1) ? kColWindow * 4 : 0;
   static constexpr int kWarpBytes = kIdxBytes + kValBytes + R * kSlotBytes;
   static constexpr int kCtaBytes = kAggWarps * kWarpBytes;
 };
 
-template <int TSMASK, int R>
+template <int TSMASK, int R, class ST = float>
 __global__ void __launch_bounds__(kAggThreads, 3) k_scatter_ring(const __grid_constant__ ScatterParams p, int* __restrict__ task_counter) {
   extern __shared__ __align__(16) unsigned char ring_smem[];
-  using L = RingLayout<TSMASK, R>;
+  using L = RingLayout<TSMASK, R, ST>;
+  constexpr uint32_t RB = L::kRowBytes;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   unsigned char* base = ring_smem + warp * L::kWarpBytes;
   int* s_idx = reinterpret_cast<int*>(base);
   float* s_val = reinterpret_cast<float*>(base + L::kIdxBytes);
-  const uint32_t ring_lane = smem_u32(base + L::kIdxBytes + L::kValBytes) + static_cast<uint32_t>(lane) * 16u;
+  const uint32_t ring_lane = smem_u32(base + L::kIdxBytes + L::kValBytes) + static_cast<uint32_t>(lane) * L::kPieceBytes;
   const bool writer = lane < p.nvec;
   const int foff = min(lane, p.nvec - 1) * 4;                    // idle lanes shadow the last piece, never write
   const uint32_t row_stride = static_cast<uint32_t>(p.ts_row_stride);
   const int64_t part_stride = static_cast<int64_t>(p.n_ts) * p.BD;
-  const float* __restrict__ src_sym = p.tstreams + p.off_sym + foff;
-  const float* __restrict__ src_lin = p.tstreams + p.off_lin + foff;
-  const float* __restrict__ src_sq = p.tstreams + p.off_sq + foff;
+  const ST* __restrict__ src_sym = reinterpret_cast<const ST*>(p.tstreams) + p.off_sym + foff;
+  const ST* __restrict__ src_lin = reinterpret_cast<const ST*>(p.tstreams) + p.off_lin + foff;
+  const ST* __restrict__ src_sq = reinterpret_cast<const ST*>(p.tstreams) + p.off_sq + foff;
   const bool hinted = p.near_rows > 0;
   const uint64_t pol_near = hinted ? l2_policy_keep() : l2_policy_normal();
   const uint64_t pol_far = hinted ? l2_policy_stream() : pol_near;
@@ -77,9 +85,12 @@ __global__ void __launch_bounds__(kAggThreads, 3) k_scatter_ring(const __grid_co
       const size_t r = static_cast<size_t>(static_cast<uint32_t>(ti) * row_stride);
       const uint64_t pol = abs(ti - col_ref) <= p.near_rows ? pol_near : pol_far;
       uint32_t dst = ring_lane + static_cast<uint32_t>(slot_w) * L::kSlotBytes;
-      if constexpr ((TSMASK & 1) != 0) { cp_async_16_hint(dst, src_sym + r, pol); dst += 512u; }
-      if constexpr ((TSMASK & 2) != 0) { cp_async_16_hint(dst, src_lin + r, pol); dst += 512u; }
-      if constexpr ((TSMASK & 4) != 0) { cp_async_16_hint(dst, src_sq + r, pol); }
+      auto cp = [&](uint32_t d, const ST* s) {
+        if constexpr (kBf16<ST>) cp_async_8_hint(d, s, pol); else cp_async_16_hint(d, s, pol);
+      };
+      if constexpr ((TSMASK & 1) != 0) { cp(dst, src_sym + r); dst += RB; }
+      if constexpr ((TSMASK & 2) != 0) { cp(dst, src_lin + r); dst += RB; }
+      if constexpr ((TSMASK & 4) != 0) { cp(dst, src_sq + r); }
       slot_w = slot_w + 1 == R ? 0 : slot_w + 1;
     }
     cp_async_commit();
@@ -88,17 +99,26 @@ __global__ void __launch_bounds__(kAggThreads, 3) k_scatter_ring(const __grid_co
   auto consume = [&](float vs) {
     cp_async_wait_group<R - 1>();
     uint32_t src = ring_lane + static_cast<uint32_t>(slot_r) * L::kSlotBytes;
+    auto lds = [](uint32_t a) -> float4 {
+      if constexpr (kBf16<ST>) {
+        uint2 w;
+        asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(w.x), "=r"(w.y) : "r"(a));
+        return widen_bf16x4(w);
+      } else {
+        return lds128(a);
+      }
+    };
     if constexpr ((TSMASK & 1) != 0) {
-      const float4 x = lds128(src); src += 512u;
+      const float4 x = lds(src); src += RB;
       a_sym[0] = __fadd_rn(a_sym[0], __fmul_rn(x.x, vs)); a_sym[1] = __fadd_rn(a_sym[1], __fmul_rn(x.y, vs));
       a_sym[2] = __fadd_rn(a_sym[2], __fmul_rn(x.z, vs)); a_sym[3] = __fadd_rn(a_sym[3], __fmul_rn(x.w, vs));
     }
     if constexpr ((TSMASK & 2) != 0) {
-      const float4 x = lds128(src); src += 512u;
+      const float4 x = lds(src); src += RB;
       a_lin[0] += x.x; a_lin[1] += x.y; a_lin[2] += x.z; a_lin[3] += x.w;
     }
     if constexpr ((TSMASK & 4) != 0) {
-      const float4 x = lds128(src);
+      const float4 x = lds(src);
       a_sq[0] += x.x; a_sq[1] += x.y; a_sq[2] += x.z; a_sq[3] += x.w;
     }
     slot_r = slot_r + 1 == R ? 0 : slot_r + 1;
@@ -114,7 +134,7 @@ __global__ void __launch_bounds__(kAggThreads, 3) k_scatter_ring(const __grid_co
     if (p.routed) ld_plain<4>(r, dst);
     if constexpr ((TSMASK & 4) != 0) {
       float xj[4];
-      ld_row<4>(xj, p.bases + static_cast<int64_t>(colj) * p.BD + foff);
+      ldg4<ST>(xj, reinterpret_cast<const ST*>(p.bases) + static_cast<int64_t>(colj) * p.BD + foff);
 #pragma unroll
       for (int k = 0; k < 4; ++k) r[k] += 2.f * xj[k] * a_sq[k];
     }
@@ -243,13 +263,13 @@ __global__ void __launch_bounds__(kAggThreads, 3) k_scatter_ring(const __grid_co
   }
 }
 
-// ring depth picked by the host: 4 (three CTAs per SM) or 7 (two CTAs per SM) for a three-stream layer
-template <int R>
+// ring depth picked by the host: 4 (three CTAs per SM) or 7 (two CTAs per SM) for a three-stream fp32 layer
+template <int R, class ST = float>
 static int launch_scatter_ring(const ScatterParams& p_in, int tsmask, int* task_counter, cudaStream_t st) {
   ScatterParams p = p_in;
 #define EGC_RING_CASE(M)                                                                                         \
   case M: {                                                                                                      \
-    using L = RingLayout<M, R>;                                                                                  \
+    using L = RingLayout<M, R, ST>;                                                                              \
     const int resident = std::max(1, std::min(3, (227 * 1024) / (L::kCtaBytes + 1024)));                         \
     const int64_t warps = static_cast<int64_t>(sm_count()) * resident * kAggWarps;                               \
     int cpt = kColsPerTask;                                                                                      \
@@ -257,7 +277,7 @@ static int launch_scatter_ring(const ScatterParams& p_in, int tsmask, int* task_
     p.cols_per_task = cpt;                                                                                       \
     const int n_blocks = ceil_div(p.col_end - p.col_begin, p.cols_per_task);                                     \
     const int grid = std::max(1, std::min(ceil_div(std::max(n_blocks, p.n_chunks), kAggWarps), sm_count() * resident)); \
-    auto kern = k_scatter_ring<M, R>;                                                                            \
+    auto kern = k_scatter_ring<M, R, ST>;                                                                        \
     EGC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, L::kCtaBytes));             \
     LaunchScope egc_ls_("k_scatter_bwd", st);                                                                    \
     kern<<<grid, kAggThreads, L::kCtaBytes, st>>>(p, task_counter);                                              \

@@ -4,6 +4,7 @@
 // the tcgen05 tensor-core path lives in project_tc.cu and is selected by `algo`.
 #include <algorithm>
 
+#include "bf16.cuh"
 #include "colsum.cuh"
 #include "common.cuh"
 #include "project.cuh"
@@ -17,10 +18,11 @@ constexpr int kBM = 128, kBK = 16, kGemmThreads = 256;
 //   B_op(k,n) = B_NCONTIG ? b[k*ldb + n] : b[n*ldb + k]
 // grid = (ceil(N/BN), ceil(M/BM), splits); with splits > 1 each z-slice reduces its own K range
 // into c + z * M * ldc (split-K partials, summed by k_reduce_splits).
-template <int BN, bool A_KCONTIG, bool B_NCONTIG>
+// CT = element type of C: float, or bf16 (each result rounded to nearest even; `accumulate` is ignored)
+template <int BN, bool A_KCONTIG, bool B_NCONTIG, class CT = float>
 __global__ void __launch_bounds__(kGemmThreads) k_gemm_f32(const float* __restrict__ a, int lda,
                                                            const float* __restrict__ b, int ldb,
-                                                           float* __restrict__ c, int ldc, int M, int N, int K,
+                                                           CT* __restrict__ c, int ldc, int M, int N, int K,
                                                            int k_per_split, const float* __restrict__ bias,
                                                            int sigmoid, int accumulate) {
   constexpr int TM = 8, TN = BN / 16;
@@ -91,7 +93,7 @@ __global__ void __launch_bounds__(kGemmThreads) k_gemm_f32(const float* __restri
     __syncthreads();
   }
 
-  float* cz = c + static_cast<int64_t>(blockIdx.z) * M * ldc;
+  CT* cz = c + static_cast<int64_t>(blockIdx.z) * M * ldc;
 #pragma unroll
   for (int i = 0; i < TM; ++i) {
     const int m = m0 + ty * TM + i;
@@ -101,11 +103,14 @@ __global__ void __launch_bounds__(kGemmThreads) k_gemm_f32(const float* __restri
       const int n = n0 + tx * TN + j;
       if (n >= N) continue;
       float v = acc[i][j];
-      float* dst = cz + static_cast<int64_t>(m) * ldc + n;
-      if (accumulate) v += *dst;
+      CT* dst = cz + static_cast<int64_t>(m) * ldc + n;
+      if constexpr (!kBf16<CT>) {
+        if (accumulate) v += *dst;
+      }
       if (bias != nullptr) v += __ldg(bias + n);
       if (sigmoid) v = 1.f / (1.f + expf(-v));
-      *dst = v;
+      if constexpr (kBf16<CT>) *dst = __float2bfloat16_rn(v);
+      else *dst = v;
     }
   }
 }
@@ -125,18 +130,18 @@ __global__ void k_reduce_splits(const float* __restrict__ partial, int splits, i
   out[i] = (t0 + t1) + (t2 + t3);
 }
 
-template <bool A_KCONTIG, bool B_NCONTIG>
-static int gemm_f32(const float* a, int lda, const float* b, int ldb, float* c, int ldc, int M, int N, int K,
+template <bool A_KCONTIG, bool B_NCONTIG, class CT = float>
+static int gemm_f32(const float* a, int lda, const float* b, int ldb, CT* c, int ldc, int M, int N, int K,
                     int splits, const float* bias, int sigmoid, int accumulate, cudaStream_t st) {
   const int k_per_split = ceil_div(ceil_div(K, splits), kBK) * kBK;
   LaunchScope ls("k_gemm_f32", st);
   if (N > 64) {
     dim3 grid(ceil_div(N, 128), ceil_div(M, kBM), splits);
-    k_gemm_f32<128, A_KCONTIG, B_NCONTIG><<<grid, kGemmThreads, 0, st>>>(a, lda, b, ldb, c, ldc, M, N, K, k_per_split,
+    k_gemm_f32<128, A_KCONTIG, B_NCONTIG, CT><<<grid, kGemmThreads, 0, st>>>(a, lda, b, ldb, c, ldc, M, N, K, k_per_split,
                                                                        bias, sigmoid, accumulate);
   } else {
     dim3 grid(ceil_div(N, 64), ceil_div(M, kBM), splits);
-    k_gemm_f32<64, A_KCONTIG, B_NCONTIG><<<grid, kGemmThreads, 0, st>>>(a, lda, b, ldb, c, ldc, M, N, K, k_per_split,
+    k_gemm_f32<64, A_KCONTIG, B_NCONTIG, CT><<<grid, kGemmThreads, 0, st>>>(a, lda, b, ldb, c, ldc, M, N, K, k_per_split,
                                                                       bias, sigmoid, accumulate);
   }
   EGC_LAUNCH_CHECK("k_gemm_f32");
@@ -150,6 +155,13 @@ int project_fwd_simt(const float* x, const float* w_bases, const float* w_comb, 
   // bases[n,bd] = x[n,f_in] . W_b[f_in,bd]
   if (int rc = gemm_f32<true, true>(x, f_in, w_bases, bd, bases, bd, n, bd, f_in, 1, nullptr, 0, 0, st)) return rc;
   // weightings[n,hab] = act(x . W_c[hab,f_in]^T + b_c)
+  return gemm_f32<true, false>(x, f_in, w_comb, f_in, weightings, hab, n, hab, f_in, 1, b_comb, sigmoid, 0, st);
+}
+
+int project_fwd_simt_bf16(const float* x, const float* w_bases, const float* w_comb, const float* b_comb, int n, int f_in,
+                          int bd, int hab, int sigmoid, uint16_t* bases, float* weightings, cudaStream_t st) {
+  if (int rc = gemm_f32<true, true, bf16>(x, f_in, w_bases, bd, reinterpret_cast<bf16*>(bases), bd, n, bd, f_in, 1, nullptr, 0, 0, st))
+    return rc;
   return gemm_f32<true, false>(x, f_in, w_comb, f_in, weightings, hab, n, hab, f_in, 1, b_comb, sigmoid, 0, st);
 }
 
@@ -220,6 +232,24 @@ int egc_project_fwd(const float* x, const float* w_bases, const float* w_comb, c
     return EGC_ERR_UNSUPPORTED;
   }
   return project_fwd_simt(x, w_bases, w_comb, b_comb, n, f_in, bd, hab, sigmoid, bases, weightings, st);
+}
+
+int egc_project_fwd_bf16(const float* x, const float* w_bases, const float* w_comb, const float* b_comb, int32_t n,
+                         int32_t f_in, int32_t bd, int32_t hab, int32_t sigmoid, uint16_t* bases, float* weightings,
+                         int32_t algo, void* stream) {
+  EGC_REQUIRE(n > 0 && f_in > 0 && bd > 0 && hab > 0, "egc_project_fwd_bf16: n=%d f_in=%d bd=%d hab=%d", n, f_in, bd, hab);
+  EGC_REQUIRE(x && w_bases && w_comb && bases && weightings, "egc_project_fwd_bf16: null pointer");
+  EGC_REQUIRE(algo >= EGC_GEMM_AUTO && algo <= EGC_GEMM_TF32, "egc_project_fwd_bf16: unknown algo %d", algo);
+  cudaStream_t st = as_stream(stream);
+  if (algo != EGC_GEMM_FP32_SIMT && project_tc_supported(n, f_in, bd, hab)) {
+    return project_fwd_tc_bf16(x, w_bases, w_comb, b_comb, n, f_in, bd, hab, sigmoid, bases, weightings,
+                               algo == EGC_GEMM_TF32 ? 1 : 3, st);
+  }
+  if (algo == EGC_GEMM_3XTF32 || algo == EGC_GEMM_TF32) {
+    set_error("egc_project_fwd_bf16: tensor-core path does not support n=%d f_in=%d bd=%d hab=%d", n, f_in, bd, hab);
+    return EGC_ERR_UNSUPPORTED;
+  }
+  return project_fwd_simt_bf16(x, w_bases, w_comb, b_comb, n, f_in, bd, hab, sigmoid, bases, weightings, st);
 }
 
 size_t egc_project_bwd_workspace_bytes(int32_t n, int32_t f_in, int32_t bd, int32_t hab) {

@@ -18,6 +18,11 @@ int project_bwd_simt(const float* x, const float* w_bases, const float* w_comb, 
 bool project_tc_supported(int n, int f_in, int bd, int hab);
 int project_fwd_tc(const float* x, const float* w_bases, const float* w_comb, const float* b_comb, int n, int f_in,
                    int bd, int hab, int sigmoid, float* bases, float* weightings, int n_terms, cudaStream_t st);
+// the same with the basis rows stored as bf16 (round to nearest even); the weightings stay fp32
+int project_fwd_tc_bf16(const float* x, const float* w_bases, const float* w_comb, const float* b_comb, int n, int f_in,
+                        int bd, int hab, int sigmoid, uint16_t* bases, float* weightings, int n_terms, cudaStream_t st);
+int project_fwd_simt_bf16(const float* x, const float* w_bases, const float* w_comb, const float* b_comb, int n, int f_in,
+                          int bd, int hab, int sigmoid, uint16_t* bases, float* weightings, cudaStream_t st);
 size_t project_bwd_tc_workspace(int n, int f_in, int bd, int hab);
 int project_bwd_tc(const float* x, const float* w_bases, const float* w_comb, const float* d_bases, const float* d_lin,
                    int n, int f_in, int bd, int hab, float* d_x, float* d_w_bases, float* d_w_comb, float* d_b_comb,

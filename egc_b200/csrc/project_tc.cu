@@ -29,6 +29,7 @@
 
 #include <algorithm>
 
+#include "bf16.cuh"
 #include "project.cuh"
 #include "tc_common.cuh"
 
@@ -75,6 +76,9 @@ struct TcParams {
 // ---------------------------------------------------------------------------------------------
 // kernel
 // ---------------------------------------------------------------------------------------------
+// BF16_C1: the columns of c1 (the basis rows of the forward) are rounded to bf16 (nearest even) in the epilogue and stored
+// packed - c1 then points at bf16 rows; c2 (the weightings) stays fp32.  The TMA-store epilogue is not used with it.
+template <bool BF16_C1>
 __global__ void __launch_bounds__(kTcThreads, 1) k_project_tc(const __grid_constant__ TcParams p, const __grid_constant__ CUtensorMap tm_a1,
                                                                const __grid_constant__ CUtensorMap tm_a2, const __grid_constant__ CUtensorMap tm_c1,
                                                                const __grid_constant__ CUtensorMap tm_c2) {
@@ -341,7 +345,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) k_project_tc(const __grid_const
           if (width > 16) tmem_ld16(taddr + 16u, rb);
           tmem_ld_wait();
         }
-        if (p.use_tma_store) {
+        if (!BF16_C1 && p.use_tma_store) {
           // ---- TMA store: bias / sigmoid in registers, row `lane` into a 128B-swizzled [32 rows x 128 B] tile
           // (16-byte piece q of row r sits at piece q ^ (r & 7): conflict-free quarter-warp stores), one tensor store
           const int colg = n_begin + col0;                     // first output column of the block (multiple of 32)
@@ -396,7 +400,12 @@ __global__ void __launch_bounds__(kTcThreads, 1) k_project_tc(const __grid_const
             float4 v = lds128(stage_addr + rl * kEpiRowBytes + piece * 16);
             if (row < p.M) {
               if (to_c1) {
-                __stcs(reinterpret_cast<float4*>(p.c1 + row * p.ldc1 + col), v);
+                if constexpr (BF16_C1) {
+                  __stcs(reinterpret_cast<uint2*>(reinterpret_cast<bf16*>(p.c1) + row * p.ldc1 + col),
+                         make_uint2(pack_bf16x2(v.x, v.y), pack_bf16x2(v.z, v.w)));
+                } else {
+                  __stcs(reinterpret_cast<float4*>(p.c1 + row * p.ldc1 + col), v);
+                }
               } else {
                 v.x += bb.x; v.y += bb.y; v.z += bb.z; v.w += bb.w;
                 if (p.sigmoid2) {
@@ -503,6 +512,7 @@ static bool make_a_map_sw64(CUtensorMap* m, const float* base, int k, int64_t ld
             CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
+template <bool BF16_C1 = false>
 static int launch_tc(TcParams& p, cudaStream_t st) {
   const int K = p.k1 + p.k2, N = p.n1 + p.n2;
   TcPlan plan;
@@ -515,7 +525,7 @@ static int launch_tc(TcParams& p, cudaStream_t st) {
   if (const char* ab = getenv("EGC_TC_ABLATE")) p.ablate = atoi(ab);
   static bool attr_set = false;
   if (!attr_set) {
-    EGC_CUDA(cudaFuncSetAttribute(k_project_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxSmem));
+    EGC_CUDA(cudaFuncSetAttribute(k_project_tc<BF16_C1>, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxSmem));
     attr_set = true;
   }
   // TMA feed of the A operand (default; EGC_TC_NO_TMA=1 keeps the cp.async producers): needs the driver's tensor-map
@@ -540,14 +550,14 @@ static int launch_tc(TcParams& p, cudaStream_t st) {
   memset(&tc2, 0, sizeof(tc2));
   static const bool want_tma_store = getenv("EGC_TC_TMA_STORE") != nullptr;
   p.use_tma_store = 0;
-  if (want_tma_store && p.n1 % 32 == 0 && p.cols_per_group % 32 == 0 && p.ldc1 % 4 == 0 && (p.n2 == 0 || (p.ldc2 % 4 == 0 && p.n2 % 4 == 0)) &&
+  if (!BF16_C1 && want_tma_store && p.n1 % 32 == 0 && p.cols_per_group % 32 == 0 && p.ldc1 % 4 == 0 && (p.n2 == 0 || (p.ldc2 % 4 == 0 && p.n2 % 4 == 0)) &&
       make_c_map(&tc1, p.c1, p.n1, p.ldc1, p.M) && (p.n2 == 0 || make_c_map(&tc2, p.c2, p.n2, p.ldc2, p.M)))
     p.use_tma_store = 1;
   const int per_group = std::max(1, std::min(p.num_tiles, sm_count() / p.n_split));
   const int grid = per_group * p.n_split;
   {
     LaunchScope ls("k_project_tc", st);
-    k_project_tc<<<grid, kTcThreads, plan.smem, st>>>(p, tm1, tm2, tc1, tc2);
+    k_project_tc<BF16_C1><<<grid, kTcThreads, plan.smem, st>>>(p, tm1, tm2, tc1, tc2);
   }
   EGC_LAUNCH_CHECK("k_project_tc");
   return EGC_OK;
@@ -565,6 +575,20 @@ int project_fwd_tc(const float* x, const float* w_bases, const float* w_comb, co
   p.c1 = bases; p.ldc1 = bd; p.c2 = weightings; p.ldc2 = hab; p.bias2 = b_comb; p.sigmoid2 = sigmoid;
   p.n_terms = n_terms;
   return launch_tc(p, st);
+}
+
+int project_fwd_tc_bf16(const float* x, const float* w_bases, const float* w_comb, const float* b_comb, int n, int f_in,
+                        int bd, int hab, int sigmoid, uint16_t* bases, float* weightings, int n_terms, cudaStream_t st) {
+  EGC_REQUIRE(aligned16(x) && aligned16(bases) && aligned16(weightings) && (b_comb == nullptr || aligned16(b_comb)),
+              "tensor-core projection needs 16-byte aligned tensors");
+  TcParams p{};
+  p.a1 = x; p.lda1 = f_in; p.k1 = f_in; p.a2 = nullptr; p.lda2 = 0; p.k2 = 0; p.M = n;
+  p.b[0][0] = w_bases; p.b_sn[0][0] = 1; p.b_sk[0][0] = bd;
+  p.b[1][0] = w_comb; p.b_sn[1][0] = f_in; p.b_sk[1][0] = 1;
+  p.n1 = bd; p.n2 = hab;
+  p.c1 = reinterpret_cast<float*>(bases); p.ldc1 = bd; p.c2 = weightings; p.ldc2 = hab; p.bias2 = b_comb; p.sigmoid2 = sigmoid;
+  p.n_terms = n_terms;
+  return launch_tc<true>(p, st);
 }
 
 size_t project_bwd_tc_workspace(int n, int f_in, int bd, int hab) {

@@ -551,6 +551,9 @@ def partitioned_egconv(x_local: Tensor, pg: PartitionedGraph, conv, relu: bool =
     """Run `conv` (an `egc_b200.EGConv` with replicated parameters) on this rank's rows of a partitioned graph.
     Output rows / input gradients are local; parameter gradients are summed over the ranks (= single-GPU values).
     With the peer transport every layer keeps its own exchange buffers (keyed by the module), one step in flight."""
+    if getattr(conv, "storage_dtype", torch.float32) != torch.float32:
+        raise NotImplementedError("partitioned_egconv / PartitionedGraph: bf16 storage is not supported (the halo and peer "
+                                  "buffers are fp32); use storage_dtype=torch.float32")
     return _PartitionedEGConvFunction.apply(x_local, conv.bases_weight, conv.comb_weight.weight, conv.comb_weight.bias,
                                             conv.bias, pg, conv.num_heads, conv.num_bases, tuple(conv.aggregators),
                                             bool(conv.sigmoid), int(conv.gemm_algo), id(conv), torch.is_grad_enabled(),

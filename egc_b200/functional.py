@@ -43,18 +43,46 @@ def _require_cuda_f32(name: str, t: Optional[Tensor]) -> Optional[Tensor]:
     return t.contiguous()
 
 
+STORAGE_DTYPES = (torch.float32, torch.bfloat16)
+
+
+def check_storage_dtype(storage_dtype) -> torch.dtype:
+    if storage_dtype not in STORAGE_DTYPES:
+        raise ValueError(f"storage_dtype must be torch.float32 or torch.bfloat16 (got {storage_dtype})")
+    return storage_dtype
+
+
+def check_bf16_layer(desc: LayerDesc, graph: GraphStructure) -> None:
+    """Raises ValueError for the layers the bf16-storage kernels do not cover (include/egc_b200.h, the *_bf16 entry points)."""
+    bd, hd = desc.bases * desc.dim, desc.heads * desc.dim
+    hab = desc.heads * desc.n_aggr * desc.bases
+    if bd % 8 != 0 or not 40 <= bd <= 128:
+        raise ValueError(f"storage_dtype=torch.bfloat16 needs num_bases * out_channels / num_heads between 40 and 128 and a "
+                         f"multiple of 8 (got {bd})")
+    if hd > (512 if desc.dim % 4 == 0 else 128):
+        raise ValueError(f"storage_dtype=torch.bfloat16: out_channels={hd} is too wide for one pass of the bf16 kernels")
+    # per-warp staging of the row-block kernel: aggregates, 8 rows of weights, column ids and weights of 384 nnz (floats)
+    if (desc.n_aggr * bd + 3) // 4 * 4 + (8 * hab + 3) // 4 * 4 + 768 > 72 * 1024 // 32:
+        raise ValueError(f"storage_dtype=torch.bfloat16: {desc.n_aggr} aggregators x {bd} basis values and {hab} weights per "
+                         "row are too wide for one pass of the bf16 kernels")
+    if graph.val_lin is not None:
+        raise ValueError("storage_dtype=torch.bfloat16 does not support an adjacency with edge values (without symnorm)")
+
+
 def project(x: Tensor, bases_weight: Tensor, comb_weight: Tensor, comb_bias: Optional[Tensor], sigmoid: bool,
-            algo: int = _lib.GEMM_AUTO, bases_out: Optional[Tensor] = None):
+            algo: int = _lib.GEMM_AUTO, bases_out: Optional[Tensor] = None, storage_dtype: torch.dtype = torch.float32):
     """bases = x @ W_b ; weightings = act(x @ W_c^T + b_c)   (ref :180-184).  `bases_out` lets a caller
-    provide the (row-prefix of a larger) buffer the basis rows are written to."""
+    provide the (row-prefix of a larger) buffer the basis rows are written to.  storage_dtype=torch.bfloat16: `bases` is
+    stored as bf16 (round to nearest even from the fp32 product); the weightings stay fp32."""
     lib = _lib.load()
     n, f_in = x.shape
     bd, hab = bases_weight.shape[1], comb_weight.shape[0]
-    bases = bases_out if bases_out is not None else torch.empty((n, bd), dtype=torch.float32, device=x.device)
+    bases = bases_out if bases_out is not None else torch.empty((n, bd), dtype=storage_dtype, device=x.device)
     weightings = torch.empty((n, hab), dtype=torch.float32, device=x.device)
+    fn = lib.egc_project_fwd_bf16 if bases.dtype == torch.bfloat16 else lib.egc_project_fwd
     if n > 0:
-        check(lib.egc_project_fwd(ptr(x), ptr(bases_weight), ptr(comb_weight), ptr(comb_bias), n, f_in, bd, hab,
-                                  int(sigmoid), ptr(bases), ptr(weightings), algo, _stream()), "egc_project_fwd")
+        check(fn(ptr(x), ptr(bases_weight), ptr(comb_weight), ptr(comb_bias), n, f_in, bd, hab,
+                 int(sigmoid), ptr(bases), ptr(weightings), algo, _stream()), fn.__name__)
     return bases, weightings
 
 
@@ -83,6 +111,11 @@ def aggregate_combine(desc: LayerDesc, graph: GraphStructure, bases: Tensor, wei
     +add; agg_init [n_dst, A, B*D] = partial aggregates of an earlier call over another entry subset (sum / symnorm only)."""
     lib = _lib.load()
     dev = bases.device
+    bf16 = bases.dtype == torch.bfloat16
+    if bf16:
+        check_bf16_layer(desc, graph)
+        if row_subset is not None or not use_plan or (epilogue is not None and len(epilogue) > 3 and epilogue[3] is not None):
+            raise NotImplementedError("bf16 basis rows: row subsets, plan-less calls and agg_init are not supported")
     if outputs is None:
         outputs = alloc_aggregate_outputs(desc, dev, want_out, want_agg, want_arg, want_saved)
     out, agg, arg, saved, saved_arg = outputs
@@ -93,6 +126,14 @@ def aggregate_combine(desc: LayerDesc, graph: GraphStructure, bases: Tensor, wei
     plan = graph.plan.struct if use_plan else None
     nbytes = lib.egc_aggregate_fwd_workspace_bytes(desc, plan)
     ws = _ws(nbytes, dev)
+    if bf16:
+        epi = None
+        if epilogue is not None and any(t is not None for t in epilogue):
+            epi = _lib.Epilogue(*(t.data_ptr() if t is not None else None for t in tuple(epilogue)[:3]), None)
+        check(lib.egc_aggregate_fwd_bf16(desc, ptr(graph.rowptr), ptr(graph.col), ptr(graph.val_sym), plan, ptr(bases),
+                                         ptr(weightings), ptr(bias), epi, ptr(out), ptr(agg), ptr(arg), ptr(saved),
+                                         ptr(saved_arg), ptr(ws), nbytes, _stream()), "egc_aggregate_fwd_bf16")
+        return outputs
     n_subset = int(row_subset.numel()) if row_subset is not None else 0
     if row_subset is not None and n_subset == 0 and not (use_plan and graph.plan.n_long):
         return outputs
@@ -137,6 +178,9 @@ def aggregate_backward(desc: LayerDesc, graph: GraphStructure, bases: Tensor, we
             return d_w, d_bases, d_bias, (out_lin_colsum.zero_() if out_lin_colsum is not None else
                                           torch.zeros(hab, dtype=torch.float32, device=dev))
         return d_w, d_bases, d_bias
+    bf16 = bases.dtype == torch.bfloat16
+    if bf16 and (pass1_only or col_split is not None):
+        raise NotImplementedError("bf16 basis rows: column phases and the pass-1-only backward are not supported")
     if not pass1_only:
         graph.ensure_csc()
     d_w = torch.empty((desc.n_dst, hab), dtype=torch.float32, device=dev)
@@ -146,6 +190,17 @@ def aggregate_backward(desc: LayerDesc, graph: GraphStructure, bases: Tensor, we
     d_lin_sum = (out_lin_colsum if out_lin_colsum is not None else
                  torch.empty(hab, dtype=torch.float32, device=dev)) if want_lin_colsum else None
     csc_plan = graph.csc_plan.struct if not pass1_only else None
+    if bf16:
+        nbytes = lib.egc_aggregate_bwd_bf16_workspace_bytes(desc, csc_plan, flags)
+        ws = _ws(nbytes, dev)
+        check(lib.egc_aggregate_bwd_bf16(desc, ptr(graph.rowptr), ptr(graph.col), ptr(graph.colptr), ptr(graph.rowidx),
+                                         ptr(graph.csr2csc), ptr(graph.csc_val_sym), csc_plan, ptr(bases), ptr(weightings),
+                                         ptr(saved), ptr(saved_arg), ptr(grad_out), ptr(out_act), ptr(epi_scale), ptr(d_w),
+                                         ptr(d_bases), ptr(d_bias), ptr(d_lin_sum), flags, ptr(ws), nbytes, _stream()),
+              "egc_aggregate_bwd_bf16")
+        if want_lin_colsum:
+            return d_w, d_bases, d_bias, d_lin_sum
+        return d_w, d_bases, d_bias
     nbytes = lib.egc_aggregate_bwd_workspace_bytes(desc, csc_plan, flags)
     ws = _ws(nbytes, dev)
     def call(phase_flags):
@@ -219,7 +274,8 @@ def project_backward(x: Tensor, bases_weight: Tensor, comb_weight: Tensor, d_bas
 class _EGConvFunction(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, bases_weight, comb_weight, comb_bias, bias, graph, heads, num_bases, aggrs, sigmoid, algo,
-                bwd_flags, grad_mode=True, relu=False, epi_scale=None, epi_shift=None, epi_add=None):
+                bwd_flags, grad_mode=True, relu=False, epi_scale=None, epi_shift=None, epi_add=None,
+                storage_dtype=torch.float32):
         x = _require_cuda_f32("x", x)
         epi_scale, epi_shift = _require_cuda_f32("scale", epi_scale), _require_cuda_f32("shift", epi_shift)
         epi_add = _require_cuda_f32("residual", epi_add)
@@ -235,10 +291,12 @@ class _EGConvFunction(torch.autograd.Function):
             raise ValueError(f"x must be [num_nodes, in_channels] with num_nodes == {graph.n_src}")
         dim = bases_weight.size(1) // num_bases
         desc = make_desc(graph, heads, num_bases, dim, aggrs, sigmoid, relu)
+        if storage_dtype == torch.bfloat16:
+            check_bf16_layer(desc, graph)
         # needs_input_grad ignores torch.no_grad(); the caller samples the grad mode before apply()
         needs_grad = grad_mode and any(ctx.needs_input_grad[:5])
         with torch.cuda.device(x.device):
-            bases, weightings = project(x, bases_weight, comb_weight, comb_bias, sigmoid, algo)
+            bases, weightings = project(x, bases_weight, comb_weight, comb_bias, sigmoid, algo, storage_dtype=storage_dtype)
             hd = heads * dim
             for name, t, shape in (("scale", epi_scale, (hd,)), ("shift", epi_shift, (hd,)), ("residual", epi_add, (graph.n_dst, hd))):
                 if t is not None and tuple(t.shape) != shape:
@@ -263,7 +321,7 @@ class _EGConvFunction(torch.autograd.Function):
         need_x, need_wb, need_wc, need_bc, need_b = ctx.needs_input_grad[:5]
         d_add = grad_out if ctx.needs_input_grad[16] else None      # the residual is added after the activation
         if saved is None:                                           # only the residual needed a gradient
-            return (None,) * 16 + (d_add,)
+            return (None,) * 16 + (d_add, None)
         with torch.cuda.device(x.device):
             want_bc = bool(need_bc and ctx.has_comb_bias)
             d_w, d_bases, d_bias, d_bc = aggregate_backward(ctx.desc, ctx.graph, bases, weightings, saved, saved_arg,
@@ -273,21 +331,24 @@ class _EGConvFunction(torch.autograd.Function):
                                                   need_wc, False, ctx.algo)
             if not want_bc:
                 d_bc = None
-        return (d_x, d_wb, d_wc, d_bc, d_bias) + (None,) * 11 + (d_add,)
+        return (d_x, d_wb, d_wc, d_bc, d_bias) + (None,) * 11 + (d_add, None)
 
 
 def egconv(x: Tensor, graph: GraphStructure, bases_weight: Tensor, comb_weight: Tensor, comb_bias: Optional[Tensor],
            bias: Optional[Tensor], num_heads: int, num_bases: int, aggrs: Sequence[str], sigmoid: bool = False,
            algo: int = _lib.GEMM_AUTO, bwd_flags: int = 0, relu: bool = False, scale: Optional[Tensor] = None,
-           shift: Optional[Tensor] = None, residual: Optional[Tensor] = None) -> Tensor:
-    """Differentiable EGConv layer body on a prepared graph.  Fused epilogue of the stack around the layer (SURVEY 8 f-1):
+           shift: Optional[Tensor] = None, residual: Optional[Tensor] = None,
+           storage_dtype: torch.dtype = torch.float32) -> Tensor:
+    """Differentiable EGConv layer body on a prepared graph.  storage_dtype=torch.bfloat16 stores the basis rows and the
+    backward's target-side streams as bf16 (half the gathered bytes); x, parameters, weightings, out, the saved aggregates,
+    all accumulation and every gradient stay fp32.  Fused epilogue of the stack around the layer (SURVEY 8 f-1):
     `scale` / `shift` [F_out] = an eval-mode BatchNorm folded to an affine map (constants), `relu=True` the ReLU that
     follows (mag/models.py:63, arxiv/norm_models.py:35-36), `residual` [N, F_out] added after the activation (:38-39):
     out = relu(layer(x) * scale + shift) + residual, all inside the aggregation kernel's epilogue; the backward masks and
     scales grad_out while its first pass stages the row."""
     return _EGConvFunction.apply(x, bases_weight, comb_weight, comb_bias, bias, graph, num_heads, num_bases,
                                  tuple(aggrs), bool(sigmoid), int(algo), int(bwd_flags), torch.is_grad_enabled(), bool(relu),
-                                 scale, shift, residual)
+                                 scale, shift, residual, check_storage_dtype(storage_dtype))
 
 
 class _ProjectFunction(torch.autograd.Function):
@@ -324,6 +385,9 @@ class _AggregateCombineFunction(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, bases, weightings, bias, graph, heads, num_bases, aggrs, bwd_flags, grad_mode=True, add=None):
+        if bases is not None and bases.dtype == torch.bfloat16:
+            raise NotImplementedError("aggregate_combine_autograd: bf16 `bases` are not supported (use EGConv(..., "
+                                      "storage_dtype=torch.bfloat16))")
         bases = _require_cuda_f32("bases", bases)
         add = _require_cuda_f32("add", add)
         weightings = _require_cuda_f32("weightings", weightings)

@@ -39,8 +39,10 @@ EdgeType = Tuple[str, str, str]
 class REGConv(torch.nn.Module):
     def __init__(self, in_channels: int, out_channels: int, num_heads: int, num_bases: int,
                  node_types: Sequence[str] = NODE_TYPES, edge_types: Sequence[EdgeType] = EDGE_TYPES,
-                 cached: bool = True, gemm_algo: int = _lib.GEMM_AUTO):
+                 cached: bool = True, gemm_algo: int = _lib.GEMM_AUTO, *, storage_dtype: torch.dtype = torch.float32):
         super().__init__()
+        if storage_dtype != torch.float32:
+            raise NotImplementedError("REGConv: bf16 storage is not supported; use storage_dtype=torch.float32")
         if out_channels % num_heads != 0:
             raise ValueError("out_channels must be divisible by the number of heads")
         self.in_channels, self.out_channels = in_channels, out_channels

@@ -13,7 +13,7 @@
  *   - all work is enqueued on `stream` (a cudaStream_t passed as void*); nothing here
  *     allocates or frees caller-visible memory or synchronises the device; scratch space is
  *     a caller-owned workspace whose size comes from the matching *_workspace_bytes();
- *   - features are fp32, row-major, contiguous; graph indices are int32 on the device
+ *   - features are fp32 (the *_bf16 entry points: bf16 basis rows, see there), row-major, contiguous; graph indices are int32 on the device
  *     (the reference's int64 edge_index / rowptr / col are narrowed by the build functions);
  *   - target-major CSR: row i lists the sources j of the messages node i receives
  *     (= the reference's `adj_t`, ref experiments/utils.py:107-109).
@@ -189,6 +189,13 @@ int egc_project_fwd(const float* x, const float* w_bases, const float* w_comb, c
                     int32_t n, int32_t f_in, int32_t bd, int32_t hab, int32_t sigmoid,
                     float* bases, float* weightings, int32_t algo, void* stream);
 
+/* Opt-in bf16 storage of the basis rows (round to nearest even, packed [n, bd] bf16 = uint16_t bit patterns; bd % 4 == 0 on
+ * the tensor-core path): the same products as egc_project_fwd, accumulated in fp32, rounded once when stored.  weightings
+ * stay fp32.  The consumers of such `bases` are egc_aggregate_fwd_bf16 / egc_aggregate_bwd_bf16. */
+int egc_project_fwd_bf16(const float* x, const float* w_bases, const float* w_comb, const float* b_comb,
+                         int32_t n, int32_t f_in, int32_t bd, int32_t hab, int32_t sigmoid,
+                         uint16_t* bases, float* weightings, int32_t algo, void* stream);
+
 /* Autograd of the two projections (ref: implicit backward of :180-182).  d_lin is the gradient
  * w.r.t. the pre-activation of comb_weight (sigmoid' already applied by egc_aggregate_bwd).
  *   d_x[n,f_in]       = d_bases . w_bases^T + d_lin . w_comb        (d_x may be NULL)
@@ -233,6 +240,16 @@ int egc_aggregate_fwd(const egc_layer_desc* desc, const int32_t* rowptr, const i
                       float* out, float* agg_out, int32_t* arg_out, float* saved, int32_t* saved_arg,
                       void* workspace, size_t workspace_bytes, void* stream);
 
+/* egc_aggregate_fwd over bf16 basis rows (from egc_project_fwd_bf16): every value is widened to fp32 before any arithmetic,
+ * so sums, means, variances and the min/max winners (first nnz wins ties) are those of egc_aggregate_fwd on the widened rows;
+ * every output stays fp32 / int32.  Covers B*D in 40..128 with B*D % 8 == 0 and H*D <= 512 (128 when D % 4 != 0), no per-nnz
+ * linear weights (val_lin), no row subset and no epilogue agg_init; 16-byte aligned tensors.  Other shapes return
+ * EGC_ERR_INVALID_ARGUMENT.  Workspace: egc_aggregate_fwd_workspace_bytes() (never NULL). */
+int egc_aggregate_fwd_bf16(const egc_layer_desc* desc, const int32_t* rowptr, const int32_t* col, const float* val_sym,
+                           const egc_row_plan* plan, const uint16_t* bases, const float* weightings, const float* bias,
+                           const egc_epilogue* epilogue, float* out, float* agg_out, int32_t* arg_out, float* saved,
+                           int32_t* saved_arg, void* workspace, size_t workspace_bytes, void* stream);
+
 /* Backward of the above (ref: autograd of :191-208; torch_sparse spmm backward over the cached CSC).
  * Pass 1 (per target, streaming over `saved`): d_weightings (times sigmoid' when desc->sigmoid; = gradient
  * w.r.t. the Linear output) and the target-side streams t_sym / t_lin / t_sq; min/max gradients are routed
@@ -270,6 +287,20 @@ int egc_aggregate_bwd(const egc_layer_desc* desc, const int32_t* rowptr, const i
                       const float* grad_out, const float* out_act, const float* epi_scale, float* d_weightings,
                       float* d_bases, float* d_bias, float* d_lin_colsum, float* tstreams_out,
                       int32_t flags, int32_t col_split, void* workspace, size_t workspace_bytes, void* stream);
+
+/* egc_aggregate_bwd for a layer whose forward ran on bf16 basis rows (egc_aggregate_fwd_bf16): `bases` is bf16 (read by the
+ * var / std term 2 bases[j] t_sq[i]) and pass 1 stores the target-side streams t_sym / t_lin / t_sq as bf16 (round to
+ * nearest even) in the workspace, which pass 2 widens and sums in fp32.  saved, the routed min/max gradients, d_weightings,
+ * d_bases, d_bias and d_lin_colsum are fp32 as in egc_aggregate_bwd.  No per-entry linear weights (val_lin), no column
+ * phases and no EGC_BWD_PASS1_ONLY; EGC_BWD_DETERMINISTIC and the tuning flags are honoured.  The basis rows must be
+ * 36..128 values wide, a multiple of 4, 16-byte aligned.  Workspace: egc_aggregate_bwd_bf16_workspace_bytes(). */
+size_t egc_aggregate_bwd_bf16_workspace_bytes(const egc_layer_desc* desc, const egc_row_plan* csc_plan, int32_t flags);
+int egc_aggregate_bwd_bf16(const egc_layer_desc* desc, const int32_t* rowptr, const int32_t* col, const int32_t* colptr,
+                           const int32_t* rowidx, const int32_t* csr2csc, const float* csc_val_sym, const egc_row_plan* csc_plan,
+                           const uint16_t* bases, const float* weightings, const float* saved, const int32_t* saved_arg,
+                           const float* grad_out, const float* out_act, const float* epi_scale, float* d_weightings,
+                           float* d_bases, float* d_bias, float* d_lin_colsum, int32_t flags, void* workspace,
+                           size_t workspace_bytes, void* stream);
 
 /* Pass 2 alone, for row-partitioned callers that exchange the TARGET-SIDE STREAMS instead of partial sums (layers without
  * min / max; no reference counterpart, DESIGN.md "multi-GPU"): pass 1 runs through egc_aggregate_bwd with
