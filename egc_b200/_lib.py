@@ -77,11 +77,15 @@ SIGNATURES = {
     "egc_aggregate_bwd_bf16_workspace_bytes": (c_size_t, [POINTER(LayerDesc), POINTER(RowPlan), c_int32]),
     "egc_aggregate_bwd_bf16": (c_int32, [POINTER(LayerDesc), _P, _P, _P, _P, _P, _P, POINTER(RowPlan), _P, _P, _P, _P, _P, _P, _P,
                                          _P, _P, _P, _P, c_int32, _P, c_size_t, _P]),
+    "egc_aggregate_bwd_bf16_partitioned": (c_int32, [POINTER(LayerDesc), _P, _P, _P, _P, _P, _P, POINTER(RowPlan), _P, _P, _P, _P,
+                                                     _P, _P, _P, _P, _P, _P, _P, _P, c_int32, c_int32, _P, c_size_t, _P]),
     "egc_aggregate_bwd_workspace_bytes": (c_size_t, [POINTER(LayerDesc), POINTER(RowPlan), c_int32]),
     "egc_aggregate_bwd": (c_int32, [POINTER(LayerDesc), _P, _P, _P, _P, _P, _P, _P, _P, POINTER(RowPlan), _P, _P, _P,
                                     _P, _P, _P, _P, _P, _P, _P, _P, _P, c_int32, c_int32, _P, c_size_t, _P]),
     "egc_aggregate_bwd_cols_workspace_bytes": (c_size_t, [POINTER(LayerDesc), POINTER(RowPlan)]),
     "egc_aggregate_bwd_cols": (c_int32, [POINTER(LayerDesc), _P, _P, _P, _P, POINTER(RowPlan), _P, _P, _P, c_int32, _P, c_size_t, _P]),
+    "egc_aggregate_bwd_cols_bf16": (c_int32, [POINTER(LayerDesc), _P, _P, _P, POINTER(RowPlan), _P, _P, _P, c_int32, _P,
+                                              c_size_t, _P]),
     "egc_gather_rows": (c_int32, [_P, _P, c_int32, c_int32, _P, _P]),
     "egc_peer_alloc": (c_int32, [c_size_t, POINTER(c_void_p), _P]),
     "egc_peer_free": (c_int32, [_P]),

@@ -387,9 +387,8 @@ static int aggregate_bwd_impl(const egc_layer_desc* desc, const int32_t* rowptr,
   if (int rc = validate_desc(desc, "egc_aggregate_bwd")) return rc;
   if (int rc = validate_plan(csc_plan, "egc_aggregate_bwd")) return rc;
   const bool pass1_only = (flags & EGC_BWD_PASS1_ONLY) != 0;
-  EGC_REQUIRE(!bf16_store || (!pass1_only && tstreams_out == nullptr && !(flags & (EGC_BWD_COLS_HEAD | EGC_BWD_COLS_TAIL)) &&
-                              val_lin == nullptr && csc_val_lin == nullptr),
-              "egc_aggregate_bwd_bf16: no column phases, no EGC_BWD_PASS1_ONLY / tstreams_out and no per-entry linear weights");
+  EGC_REQUIRE(!bf16_store || (val_lin == nullptr && csc_val_lin == nullptr),
+              "egc_aggregate_bwd_bf16: no per-entry linear weights");
   EGC_REQUIRE(rowptr && col && bases && weightings && saved && grad_out && d_weightings && workspace &&
               (pass1_only || (colptr && rowidx && d_bases)), "egc_aggregate_bwd: null pointer");
   EGC_REQUIRE((desc->relu != 0) == (out_act != nullptr), "egc_aggregate_bwd: out_act must be given exactly when desc->relu is set");
@@ -605,10 +604,22 @@ int egc_aggregate_bwd_bf16(const egc_layer_desc* desc, const int32_t* rowptr, co
                            const float* grad_out, const float* out_act, const float* epi_scale, float* d_weightings,
                            float* d_bases, float* d_bias, float* d_lin_colsum, int32_t flags, void* workspace,
                            size_t workspace_bytes, void* stream) {
+  return egc_aggregate_bwd_bf16_partitioned(desc, rowptr, col, colptr, rowidx, csr2csc, csc_val_sym, csc_plan, bases, weightings,
+                                            saved, saved_arg, grad_out, out_act, epi_scale, d_weightings, d_bases, d_bias,
+                                            d_lin_colsum, nullptr, flags, 0, workspace, workspace_bytes, stream);
+}
+
+int egc_aggregate_bwd_bf16_partitioned(const egc_layer_desc* desc, const int32_t* rowptr, const int32_t* col,
+                                       const int32_t* colptr, const int32_t* rowidx, const int32_t* csr2csc,
+                                       const float* csc_val_sym, const egc_row_plan* csc_plan, const uint16_t* bases,
+                                       const float* weightings, const float* saved, const int32_t* saved_arg,
+                                       const float* grad_out, const float* out_act, const float* epi_scale, float* d_weightings,
+                                       float* d_bases, float* d_bias, float* d_lin_colsum, uint16_t* tstreams_out,
+                                       int32_t flags, int32_t col_split, void* workspace, size_t workspace_bytes, void* stream) {
   return aggregate_bwd_impl(desc, rowptr, col, nullptr, colptr, rowidx, csr2csc, csc_val_sym, nullptr, csc_plan,
                             reinterpret_cast<const float*>(bases), weightings, saved, saved_arg, grad_out, out_act, epi_scale,
-                            d_weightings, d_bases, d_bias, d_lin_colsum, nullptr, flags, 0, workspace, workspace_bytes, stream,
-                            true);
+                            d_weightings, d_bases, d_bias, d_lin_colsum, reinterpret_cast<float*>(tstreams_out), flags,
+                            col_split, workspace, workspace_bytes, stream, true);
 }
 
 size_t egc_aggregate_bwd_cols_workspace_bytes(const egc_layer_desc* desc, const egc_row_plan* csc_plan) {
@@ -616,13 +627,19 @@ size_t egc_aggregate_bwd_cols_workspace_bytes(const egc_layer_desc* desc, const 
   return bwd_layout(*desc, csc_plan).csc_part_bytes + 256;
 }
 
-int egc_aggregate_bwd_cols(const egc_layer_desc* desc, const int32_t* colptr, const int32_t* rowidx, const float* csc_val_sym,
-                           const float* csc_val_lin, const egc_row_plan* csc_plan, const float* tstreams, const float* bases,
-                           float* d_bases, int32_t flags, void* workspace, size_t workspace_bytes, void* stream) {
+}  // extern "C"
+
+// egc_aggregate_bwd_cols / egc_aggregate_bwd_cols_bf16.  bf16: `tstreams` and `bases` point at bf16 rows; d_bases and the
+// chunk partials in the workspace stay fp32, so both share egc_aggregate_bwd_cols_workspace_bytes().
+static int aggregate_bwd_cols_impl(const egc_layer_desc* desc, const int32_t* colptr, const int32_t* rowidx,
+                                   const float* csc_val_sym, const float* csc_val_lin, const egc_row_plan* csc_plan,
+                                   const float* tstreams, const float* bases, float* d_bases, int32_t flags, void* workspace,
+                                   size_t workspace_bytes, void* stream, bool bf16_store) {
   if (int rc = validate_desc(desc, "egc_aggregate_bwd_cols")) return rc;
   if (int rc = validate_plan(csc_plan, "egc_aggregate_bwd_cols")) return rc;
   EGC_REQUIRE(colptr && rowidx && tstreams && d_bases && workspace, "egc_aggregate_bwd_cols: null pointer");
-  const BwdLayout L = bwd_layout(*desc, csc_plan);
+  const size_t ts_elem = bf16_store ? 2 : 4;
+  const BwdLayout L = bwd_layout(*desc, csc_plan, ts_elem);
   EGC_REQUIRE(!L.has_route, "egc_aggregate_bwd_cols: min / max gradients are routed by egc_aggregate_bwd, not by the column pass");
   EGC_REQUIRE(L.tsmask != 0, "egc_aggregate_bwd_cols: the layer has no linear stream");
   const int mask = prim_mask_of(*desc);
@@ -630,11 +647,28 @@ int egc_aggregate_bwd_cols(const egc_layer_desc* desc, const int32_t* colptr, co
   EGC_REQUIRE(!((mask & P_SYM) && csc_val_lin), "egc_aggregate_bwd_cols: val_lin cannot be combined with symnorm");
   EGC_REQUIRE(L.ts_sq < 0 || bases != nullptr, "egc_aggregate_bwd_cols: var / std need the basis rows of the columns");
   EGC_REQUIRE(workspace_bytes >= L.csc_part_bytes, "egc_aggregate_bwd_cols: workspace too small (%zu < %zu)", workspace_bytes, L.csc_part_bytes);
-  EGC_REQUIRE(L.ts_bytes / 4 < (size_t{1} << 32), "egc_aggregate_bwd_cols: target-side streams exceed 2^32 floats");
+  EGC_REQUIRE(L.ts_bytes / ts_elem < (size_t{1} << 32), "egc_aggregate_bwd_cols: target-side streams exceed 2^32 values");
   const int bd = desc->bases * desc->dim;
   const bool vec4 = (bd % 4 == 0) && (bases == nullptr || aligned16(bases)) && aligned16(d_bases) && aligned16(tstreams) && aligned16(workspace);
   return run_pass2(*desc, L, colptr, rowidx, csc_val_sym, csc_val_lin, csc_plan, tstreams, bases, d_bases, 0, desc->n_src,
-                   (flags & EGC_BWD_ACCUMULATE) != 0, static_cast<float*>(workspace), vec4, as_stream(stream));
+                   (flags & EGC_BWD_ACCUMULATE) != 0, static_cast<float*>(workspace), vec4, as_stream(stream), bf16_store);
+}
+
+extern "C" {
+
+int egc_aggregate_bwd_cols(const egc_layer_desc* desc, const int32_t* colptr, const int32_t* rowidx, const float* csc_val_sym,
+                           const float* csc_val_lin, const egc_row_plan* csc_plan, const float* tstreams, const float* bases,
+                           float* d_bases, int32_t flags, void* workspace, size_t workspace_bytes, void* stream) {
+  return aggregate_bwd_cols_impl(desc, colptr, rowidx, csc_val_sym, csc_val_lin, csc_plan, tstreams, bases, d_bases, flags,
+                                 workspace, workspace_bytes, stream, false);
+}
+
+int egc_aggregate_bwd_cols_bf16(const egc_layer_desc* desc, const int32_t* colptr, const int32_t* rowidx,
+                                const float* csc_val_sym, const egc_row_plan* csc_plan, const uint16_t* tstreams,
+                                const uint16_t* bases, float* d_bases, int32_t flags, void* workspace, size_t workspace_bytes,
+                                void* stream) {
+  return aggregate_bwd_cols_impl(desc, colptr, rowidx, csc_val_sym, nullptr, csc_plan, reinterpret_cast<const float*>(tstreams),
+                                 reinterpret_cast<const float*>(bases), d_bases, flags, workspace, workspace_bytes, stream, true);
 }
 
 }  // extern "C"

@@ -237,7 +237,8 @@ class CudaHaloExchange(HaloExchange):
         q = next(i for i, t in enumerate(self.send_rows) if t is index)
         idx = self.send_rows32[q]
         out = torch.empty((idx.numel(), rows.size(1)), dtype=rows.dtype, device=rows.device)
-        _lib.check(_lib.load().egc_gather_rows(_lib.ptr(rows), _lib.ptr(idx), idx.numel(), rows.size(1), _lib.ptr(out),
+        words = rows.size(1) * rows.element_size() // 4                # the kernel moves 4-byte words (bf16: B*D % 8 == 0)
+        _lib.check(_lib.load().egc_gather_rows(_lib.ptr(rows), _lib.ptr(idx), idx.numel(), words, _lib.ptr(out),
                                                _stream()), "egc_gather_rows")
         return out
 
@@ -251,13 +252,21 @@ class PartitionedGraph:
 
     transport = "peer" (default): our own kernels over NVLink peer memory (`egc_b200.peer`, csrc/peer.cu) - posted
     stores into the consumer's memory ordered by epoch flags, graph-capturable, no NCCL on the data path;
-    transport = "nccl": point-to-point `batch_isend_irecv` + all-reduce (kept as the library baseline)."""
+    transport = "nccl": point-to-point `batch_isend_irecv` + all-reduce (kept as the library baseline).
+
+    storage_dtype=torch.bfloat16 declares that the exchanges of this graph may carry bf16 rows: layers built with
+    `EGConv(..., storage_dtype=torch.bfloat16)` then run on it, their halo basis rows and T-exchange stream rows travel as
+    bf16 (the halo partial sums stay fp32).  fp32 layers run on either kind of graph."""
 
     def __init__(self, part: LocalPartition, device, group=None, transport: str = "peer",
-                 tpart: Optional[LocalPartition] = None):
+                 tpart: Optional[LocalPartition] = None, storage_dtype: torch.dtype = torch.float32):
+        from .functional import check_storage_dtype
         from .graph import GraphStructure
         if transport not in ("peer", "nccl"):
             raise ValueError(f"unknown transport {transport!r}")
+        self.storage_dtype = check_storage_dtype(storage_dtype)
+        if storage_dtype == torch.bfloat16 and part.val_lin is not None:      # same on every rank; nothing collective yet
+            raise ValueError("storage_dtype=torch.bfloat16 does not support an adjacency with edge values (without symnorm)")
         self.part = part
         self.tpart = tpart                         # local block of the TRANSPOSED adjacency (T exchange), or None
         self._graph_t = None
@@ -296,10 +305,11 @@ class PartitionedGraph:
 
     @staticmethod
     def from_global(graph, rank: int, world_size: int, device, group=None, transport: str = "peer",
-                    t_exchange: Optional[bool] = None) -> "PartitionedGraph":
+                    t_exchange: Optional[bool] = None, storage_dtype: torch.dtype = torch.float32) -> "PartitionedGraph":
         """Partition a prepared single-device `GraphStructure` (every rank builds the same plan).  `t_exchange`: also
         partition the transposed adjacency (needed by the T-exchange backward; default: yes for square graphs on more
-        than one rank unless EGC_DIST_T_EXCHANGE=0)."""
+        than one rank unless EGC_DIST_T_EXCHANGE=0).  `storage_dtype`: see the class docstring; bf16 raises ValueError
+        for a graph with edge values, on every rank alike and before anything collective."""
         import os
         plan = PartitionPlan(graph.rowptr.cpu(), graph.col.cpu(), world_size,
                              val_sym=graph.val_sym.cpu() if graph.val_sym is not None else None,
@@ -307,7 +317,7 @@ class PartitionedGraph:
         if t_exchange is None:
             t_exchange = world_size > 1 and graph.n_dst == graph.n_src and os.environ.get("EGC_DIST_T_EXCHANGE", "auto") != "0"
         tpart = plan.transposed().local(rank) if t_exchange else None
-        return PartitionedGraph(plan.local(rank), device, group, transport, tpart)
+        return PartitionedGraph(plan.local(rank), device, group, transport, tpart, storage_dtype)
 
     @property
     def graph_t(self):
@@ -330,11 +340,12 @@ class PartitionedGraph:
                 for rp, col, vs, vl in part.split_by_column())
         return self._split[transposed]
 
-    def uses_overlap(self, aggrs) -> bool:
+    def uses_overlap(self, aggrs, storage_dtype: torch.dtype = torch.float32) -> bool:
         """Split launches around a copy-engine exchange: layers whose aggregators are all sum / symnorm (continuable sums
-        that do not depend on the row's entry count), peer transport, T-exchange backward."""
-        return (self.transport == "peer" and self.overlap != "0" and self.part.n_halo > 0 and
-                all(a in ("sum", "symnorm") for a in aggrs) and self.uses_t_exchange(aggrs))
+        that do not depend on the row's entry count), peer transport, T-exchange backward.  Never for bf16 layers: the
+        second forward launch continues the sums with `agg_init`, which the bf16 forward does not take."""
+        return (storage_dtype == torch.float32 and self.transport == "peer" and self.overlap != "0" and
+                self.part.n_halo > 0 and all(a in ("sum", "symnorm") for a in aggrs) and self.uses_t_exchange(aggrs))
 
     def uses_t_exchange(self, aggrs) -> bool:
         if self.tpart is None or self.t_exchange == "0" or any(a in ("max", "min") for a in aggrs):
@@ -343,14 +354,14 @@ class PartitionedGraph:
             return False
         return self.t_exchange == "1" or n_target_streams(aggrs) == 1
 
-    def peer_context(self, key, bd: int, n_flat: int, t_width: int = 0):
+    def peer_context(self, key, bd: int, n_flat: int, t_width: int = 0, storage_dtype: torch.dtype = torch.float32):
         """Exchange state of one layer (collective on first use: every rank must reach it in the same order)."""
-        k = (key, int(bd), int(n_flat), int(t_width))
+        k = (key, int(bd), int(n_flat), int(t_width), storage_dtype)
         ctx = self._peer_ctx.get(k)
         if ctx is None:
             from .peer import PeerLayerContext
             ctx = PeerLayerContext(self.part, bd, n_flat, self.device, self.group,
-                                   tpart=self.tpart if t_width else None, t_width=t_width)
+                                   tpart=self.tpart if t_width else None, t_width=t_width, storage_dtype=storage_dtype)
             self._peer_ctx[k] = ctx
         return ctx
 
@@ -374,33 +385,39 @@ def n_target_streams(aggrs) -> int:
 class _PartitionedEGConvFunction(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, bases_weight, comb_weight, comb_bias, bias, pg, heads, num_bases, aggrs, sigmoid, algo, key,
-                grad_mode=True, bwd_flags=0, relu=False):
+                grad_mode=True, bwd_flags=0, relu=False, storage_dtype=torch.float32):
         from . import functional as F
         from . import peer as P
         part, g = pg.part, pg.graph
         x = F._require_cuda_f32("x", x)
         bd = bases_weight.size(1)
         desc = F.make_desc(g, heads, num_bases, bd // num_bases, aggrs, sigmoid, relu)
+        bf16 = storage_dtype == torch.bfloat16
+        if bf16:
+            F.check_bf16_layer(desc, g)
+        # the bf16 forward has no row subset: bf16 layers wait for the halo rows and run one contiguous launch
+        rows_split = pg.overlap_interior and not bf16
         needs_grad = grad_mode and any(ctx.needs_input_grad[:5])       # needs_input_grad ignores torch.no_grad()
         peer = None
         with torch.cuda.device(x.device):
             if pg.transport == "peer":
                 n_flat = bases_weight.numel() + comb_weight.numel() + comb_weight.size(0) + heads * (bd // num_bases)
-                peer = pg.peer_context(key, bd, n_flat, n_target_streams(aggrs) * bd if pg.uses_t_exchange(aggrs) else 0)
+                peer = pg.peer_context(key, bd, n_flat, n_target_streams(aggrs) * bd if pg.uses_t_exchange(aggrs) else 0,
+                                       storage_dtype)
                 # new epoch; every peer is done with the halo rows of my previous step
                 ctx.step_id = peer.begin_step(needs_grad)
                 bases_ext = peer.bases_ext
             else:
-                bases_ext = torch.empty((part.n_local + part.n_halo, bd), dtype=torch.float32, device=x.device)
+                bases_ext = torch.empty((part.n_local + part.n_halo, bd), dtype=storage_dtype, device=x.device)
             _, weightings = F.project(x, bases_weight.contiguous(), comb_weight.contiguous(), comb_bias, sigmoid, algo,
                                       bases_out=bases_ext[:part.n_local])
             outs = F.alloc_aggregate_outputs(desc, x.device, want_out=True, want_saved=needs_grad)
             def interior():
-                if pg.overlap_interior:
+                if rows_split:
                     F.aggregate_combine(desc, g, bases_ext, weightings, bias, row_subset=pg.interior, use_plan=False,
                                         outputs=outs)
 
-            overlap = peer is not None and pg.uses_overlap(aggrs)
+            overlap = peer is not None and pg.uses_overlap(aggrs, storage_dtype)
             if overlap:
                 # copy-engine push on the side stream while the entries with own columns are aggregated here; the halo
                 # entries then continue those sums (agg_init) and the same launch combines and writes out / saved
@@ -426,7 +443,7 @@ class _PartitionedEGConvFunction(torch.autograd.Function):
                 bases_ext[part.n_local:].copy_(halo)
             if overlap:
                 pass
-            elif pg.overlap_interior:
+            elif rows_split:
                 F.aggregate_combine(desc, g, bases_ext, weightings, bias, row_subset=pg.boundary, use_plan=True,
                                     outputs=outs)
             else:                                          # one contiguous launch over every local row
@@ -437,6 +454,7 @@ class _PartitionedEGConvFunction(torch.autograd.Function):
         if needs_grad:
             ctx.save_for_backward(x, bases_weight, comb_weight, bases_ext, weightings, saved, saved_arg, out if relu else None)
         ctx.pg, ctx.desc, ctx.algo, ctx.peer, ctx.bwd_flags, ctx.aggrs = pg, desc, algo, peer, int(bwd_flags), tuple(aggrs)
+        ctx.storage_dtype = storage_dtype
         ctx.has_bias, ctx.has_comb_bias = bias is not None, comb_bias is not None
         return out
 
@@ -457,7 +475,7 @@ class _PartitionedEGConvFunction(torch.autograd.Function):
                 desc_t.n_dst, desc_t.n_src = pg.tpart.n_local + pg.tpart.n_halo, pg.tpart.n_local   # stream rows, own columns
                 t_width = n_target_streams(ctx.aggrs) * ctx.desc.bases * ctx.desc.dim
             if peer is None and use_t:
-                t_own = torch.empty((part.n_local, t_width), dtype=torch.float32, device=x.device)
+                t_own = torch.empty((part.n_local, t_width), dtype=ctx.storage_dtype, device=x.device)
                 d_w, _, d_bias, d_bc = F.aggregate_backward(ctx.desc, pg.graph, bases_ext, weightings, saved, saved_arg,
                                                             grad_out, want_b, ctx.bwd_flags, want_lin_colsum=True,
                                                             out_act=out_act, tstreams_out=t_own)
@@ -477,7 +495,7 @@ class _PartitionedEGConvFunction(torch.autograd.Function):
                 for t in (d_wb, d_wc, d_bc, d_bias):                          # parameters are replicated
                     if t is not None:
                         dist.all_reduce(t, op=dist.ReduceOp.SUM, group=pg.group)
-                return (d_x, d_wb, d_wc, d_bc, d_bias) + (None,) * 10
+                return (d_x, d_wb, d_wc, d_bc, d_bias) + (None,) * 11
             # ---- peer transport: flat parameter-gradient vector [d_wb | d_wc | d_bc | d_bias] in the exchange context
             n_wb, n_wc, hab = bases_weight.numel(), comb_weight.numel(), comb_weight.size(0)
             hd = ctx.desc.heads * ctx.desc.dim
@@ -503,7 +521,7 @@ class _PartitionedEGConvFunction(torch.autograd.Function):
                 d_w, _, _, _ = F.aggregate_backward(ctx.desc, pg.graph, bases_ext, weightings, saved, saved_arg, grad_out,
                                                     want_b, ctx.bwd_flags, want_lin_colsum=True, out_bias=v_b,
                                                     out_lin_colsum=v_bc, out_act=out_act, tstreams_out=peer.t_ext)
-                if pg.uses_overlap(ctx.aggrs):
+                if pg.uses_overlap(ctx.aggrs, ctx.storage_dtype):
                     peer.side_stream.wait_stream(main)
                     with torch.cuda.stream(peer.side_stream):
                         peer.push_t(dma=True)
@@ -539,7 +557,7 @@ class _PartitionedEGConvFunction(torch.autograd.Function):
             d_wc = total[n_wb:n_wb + n_wc].view_as(comb_weight).clone() if need_wc else None
             d_bc = total[n_wb + n_wc:n_wb + n_wc + hab].clone() if want_bc else None
             d_bias = total[n_wb + n_wc + hab:n_wb + n_wc + hab + hd].clone() if want_b else None
-        return (d_x, d_wb, d_wc, d_bc, d_bias) + (None,) * 10
+        return (d_x, d_wb, d_wc, d_bc, d_bias) + (None,) * 11
 
 
 def _bwd_flags_of(conv) -> int:
@@ -550,14 +568,18 @@ def _bwd_flags_of(conv) -> int:
 def partitioned_egconv(x_local: Tensor, pg: PartitionedGraph, conv, relu: bool = False) -> Tensor:
     """Run `conv` (an `egc_b200.EGConv` with replicated parameters) on this rank's rows of a partitioned graph.
     Output rows / input gradients are local; parameter gradients are summed over the ranks (= single-GPU values).
-    With the peer transport every layer keeps its own exchange buffers (keyed by the module), one step in flight."""
-    if getattr(conv, "storage_dtype", torch.float32) != torch.float32:
-        raise NotImplementedError("partitioned_egconv / PartitionedGraph: bf16 storage is not supported (the halo and peer "
-                                  "buffers are fp32); use storage_dtype=torch.float32")
+    With the peer transport every layer keeps its own exchange buffers (keyed by the module), one step in flight.
+    A layer with `storage_dtype=torch.bfloat16` needs a graph built with `storage_dtype=torch.bfloat16`; it returns this
+    rank's rows of the single-GPU bf16 layer's results."""
+    storage_dtype = getattr(conv, "storage_dtype", torch.float32)
+    if storage_dtype != torch.float32 and getattr(pg, "storage_dtype", None) != storage_dtype:
+        raise NotImplementedError("partitioned_egconv: a layer with storage_dtype=torch.bfloat16 needs a PartitionedGraph "
+                                  "built with storage_dtype=torch.bfloat16 (PartitionedGraph.from_global(..., "
+                                  "storage_dtype=torch.bfloat16))")
     return _PartitionedEGConvFunction.apply(x_local, conv.bases_weight, conv.comb_weight.weight, conv.comb_weight.bias,
                                             conv.bias, pg, conv.num_heads, conv.num_bases, tuple(conv.aggregators),
                                             bool(conv.sigmoid), int(conv.gemm_algo), id(conv), torch.is_grad_enabled(),
-                                            _bwd_flags_of(conv), bool(relu))
+                                            _bwd_flags_of(conv), bool(relu), storage_dtype)
 
 
 class GraphedStep:

@@ -179,8 +179,8 @@ def aggregate_backward(desc: LayerDesc, graph: GraphStructure, bases: Tensor, we
                                           torch.zeros(hab, dtype=torch.float32, device=dev))
         return d_w, d_bases, d_bias
     bf16 = bases.dtype == torch.bfloat16
-    if bf16 and (pass1_only or col_split is not None):
-        raise NotImplementedError("bf16 basis rows: column phases and the pass-1-only backward are not supported")
+    if pass1_only and tstreams_out.dtype != bases.dtype:
+        raise TypeError(f"tstreams_out must have the dtype of bases ({bases.dtype}, got {tstreams_out.dtype})")
     if not pass1_only:
         graph.ensure_csc()
     d_w = torch.empty((desc.n_dst, hab), dtype=torch.float32, device=dev)
@@ -192,18 +192,19 @@ def aggregate_backward(desc: LayerDesc, graph: GraphStructure, bases: Tensor, we
     csc_plan = graph.csc_plan.struct if not pass1_only else None
     if bf16:
         nbytes = lib.egc_aggregate_bwd_bf16_workspace_bytes(desc, csc_plan, flags)
-        ws = _ws(nbytes, dev)
-        check(lib.egc_aggregate_bwd_bf16(desc, ptr(graph.rowptr), ptr(graph.col), ptr(graph.colptr), ptr(graph.rowidx),
-                                         ptr(graph.csr2csc), ptr(graph.csc_val_sym), csc_plan, ptr(bases), ptr(weightings),
-                                         ptr(saved), ptr(saved_arg), ptr(grad_out), ptr(out_act), ptr(epi_scale), ptr(d_w),
-                                         ptr(d_bases), ptr(d_bias), ptr(d_lin_sum), flags, ptr(ws), nbytes, _stream()),
-              "egc_aggregate_bwd_bf16")
-        if want_lin_colsum:
-            return d_w, d_bases, d_bias, d_lin_sum
-        return d_w, d_bases, d_bias
-    nbytes = lib.egc_aggregate_bwd_workspace_bytes(desc, csc_plan, flags)
+    else:
+        nbytes = lib.egc_aggregate_bwd_workspace_bytes(desc, csc_plan, flags)
     ws = _ws(nbytes, dev)
     def call(phase_flags):
+        if bf16:
+            csc = (None,) * 4 if pass1_only else (ptr(graph.colptr), ptr(graph.rowidx), ptr(graph.csr2csc), ptr(graph.csc_val_sym))
+            check(lib.egc_aggregate_bwd_bf16_partitioned(desc, ptr(graph.rowptr), ptr(graph.col), *csc, csc_plan, ptr(bases),
+                                                         ptr(weightings), ptr(saved), ptr(saved_arg), ptr(grad_out),
+                                                         ptr(out_act), ptr(epi_scale), ptr(d_w), ptr(d_bases), ptr(d_bias),
+                                                         ptr(d_lin_sum), ptr(tstreams_out), flags | phase_flags,
+                                                         int(col_split or 0), ptr(ws), nbytes, _stream()),
+                  "egc_aggregate_bwd_bf16_partitioned")
+            return
         check(lib.egc_aggregate_bwd(desc, ptr(graph.rowptr), ptr(graph.col), ptr(graph.val_lin),
                                     *((None,) * 5 if pass1_only else (ptr(graph.colptr), ptr(graph.rowidx), ptr(graph.csr2csc),
                                                                       ptr(graph.csc_val_sym), ptr(graph.csc_val_lin))),
@@ -230,10 +231,15 @@ def aggregate_backward_cols(desc_t: LayerDesc, graph_t: GraphStructure, tstreams
                             d_bases: Optional[Tensor] = None, accumulate: bool = False) -> Tensor:
     """Pass 2 of the backward alone (`egc_aggregate_bwd_cols`): `graph_t` is the TRANSPOSED local adjacency in CSR form
     (rows = own source columns, column ids = rows of `tstreams`, values = the entries' weights), `desc_t` its descriptor
-    (n_dst of the descriptor = rows of `tstreams`, n_src = rows of `graph_t`).  Returns d_bases [n_src, B * D]."""
+    (n_dst of the descriptor = rows of `tstreams`, n_src = rows of `graph_t`).  Returns d_bases [n_src, B * D].
+    A bf16 `tstreams` (from a bf16 pass 1) runs `egc_aggregate_bwd_cols_bf16`: `bases` are then the bf16 basis rows and
+    d_bases stays fp32."""
     lib = _lib.load()
     dev = tstreams.device
     bd = desc_t.bases * desc_t.dim
+    bf16 = tstreams.dtype == torch.bfloat16
+    if bf16 and bases is not None and bases.dtype != torch.bfloat16:
+        raise TypeError(f"bf16 target-side streams need bf16 basis rows (got {bases.dtype})")
     if d_bases is None:
         d_bases = torch.empty((desc_t.n_src, bd), dtype=torch.float32, device=dev)
     if desc_t.n_src == 0:
@@ -241,9 +247,15 @@ def aggregate_backward_cols(desc_t: LayerDesc, graph_t: GraphStructure, tstreams
     plan = graph_t.plan.struct
     nbytes = lib.egc_aggregate_bwd_cols_workspace_bytes(desc_t, plan)
     ws = _ws(nbytes, dev)
+    flags = _lib.BWD_ACCUMULATE if accumulate else 0
+    if bf16:
+        check(lib.egc_aggregate_bwd_cols_bf16(desc_t, ptr(graph_t.rowptr), ptr(graph_t.col), ptr(graph_t.val_sym), plan,
+                                              ptr(tstreams), ptr(bases), ptr(d_bases), flags, ptr(ws), nbytes, _stream()),
+              "egc_aggregate_bwd_cols_bf16")
+        return d_bases
     check(lib.egc_aggregate_bwd_cols(desc_t, ptr(graph_t.rowptr), ptr(graph_t.col), ptr(graph_t.val_sym), ptr(graph_t.val_lin),
-                                     plan, ptr(tstreams), ptr(bases), ptr(d_bases), _lib.BWD_ACCUMULATE if accumulate else 0,
-                                     ptr(ws), nbytes, _stream()), "egc_aggregate_bwd_cols")
+                                     plan, ptr(tstreams), ptr(bases), ptr(d_bases), flags, ptr(ws), nbytes, _stream()),
+          "egc_aggregate_bwd_cols")
     return d_bases
 
 def project_backward(x: Tensor, bases_weight: Tensor, comb_weight: Tensor, d_bases: Tensor, d_lin: Tensor,

@@ -120,11 +120,16 @@ def _ptr_array(values: List[int]):
 
 
 class PeerLayerContext:
-    """Exchange state of one layer (basis width `bd`, `n_flat` replicated parameter-gradient floats) on one rank."""
+    """Exchange state of one layer (basis width `bd`, `n_flat` replicated parameter-gradient floats) on one rank.
+    storage_dtype=torch.bfloat16: the basis rows (`bases_ext`) and the target-side stream rows (`t_ext`) are stored and
+    pushed as bf16 - half the bytes per exchanged row; the halo partial sums (`staging`) and the parameter-gradient slots
+    stay fp32."""
 
     def __init__(self, part, bd: int, n_flat: int, device, group=None, timeout_ns: int = DEFAULT_TIMEOUT_NS,
-                 tpart=None, t_width: int = 0):
+                 tpart=None, t_width: int = 0, storage_dtype: torch.dtype = torch.float32):
         self.part, self.bd, self.device, self.group = part, int(bd), torch.device(device), group
+        self.storage_dtype = storage_dtype
+        elem = torch.empty((), dtype=storage_dtype).element_size()            # bytes per stored basis / stream value
         self.tpart, self.t_width = (tpart, int(t_width)) if tpart is not None and t_width else (None, 0)
         self.rank, self.world = part.rank, part.world_size
         self.timeout_ns = int(timeout_ns)
@@ -133,12 +138,16 @@ class PeerLayerContext:
         send_counts = [int(t.numel()) for t in part.send_rows]
         n_send = sum(send_counts) if self.tpart is None else 0     # T exchange: no partial sums, no staging
         n_ext_t = (self.tpart.n_local + self.tpart.n_halo) if self.tpart is not None else 0
-        self.seg = PeerSegment([("flags", 4 * N_SLOTS * self.world), ("bases_ext", 4 * n_ext * bd),
+        # the push kernels move 4-byte words: row widths of the stored tables in words (bf16 rows: whole 16-byte pieces)
+        if elem != 4 and (self.bd % 8 or self.t_width % 8):
+            raise ValueError(f"bf16 exchange rows need B*D % 8 == 0 (got {self.bd})")
+        self.bd_words, self.t_words = self.bd * elem // 4, self.t_width * elem // 4
+        self.seg = PeerSegment([("flags", 4 * N_SLOTS * self.world), ("bases_ext", elem * n_ext * bd),
                                 ("staging", 4 * max(n_send, 1) * bd), ("slots", 4 * self.world * self.n_flat),
-                                ("t_ext", 4 * n_ext_t * self.t_width)], device, group)
-        self.t_ext = self.seg.view("t_ext", (n_ext_t, self.t_width)) if self.tpart is not None else None
+                                ("t_ext", elem * n_ext_t * self.t_width)], device, group)
+        self.t_ext = self.seg.view("t_ext", (n_ext_t, self.t_width), storage_dtype) if self.tpart is not None else None
         self.flags = self.seg.view("flags", (N_SLOTS * self.world,), torch.int32)
-        self.bases_ext = self.seg.view("bases_ext", (n_ext, bd))
+        self.bases_ext = self.seg.view("bases_ext", (n_ext, bd), storage_dtype)
         self.staging = self.seg.view("staging", (max(n_send, 1), bd))
         self.slots = self.seg.view("slots", (self.world, self.n_flat))
         self.epoch = torch.zeros(1, dtype=torch.int32, device=self.device)
@@ -173,7 +182,7 @@ class PeerLayerContext:
             self.peers = [q for q in range(self.world) if q != self.rank]
         else:
             self.peers = [(self.rank + k) % self.world for k in range(1, self.world)]
-        row_bytes = 4 * bd
+        row_bytes = elem * bd
 
         # forward push: rows send_rows[q] of my basis table -> q's halo region, at q's offset for owner = me
         self.fwd_index = (torch.cat([part.send_rows[q] for q in self.peers]) if self.peers else
@@ -192,7 +201,7 @@ class PeerLayerContext:
         bwd_dst = []
         for s, q in enumerate(self.peers):
             self.bwd_seg_ptr[s + 1] = self.bwd_seg_ptr[s] + part.recv_counts[q]
-            bwd_dst.append(self.seg.peer_ptr(q, "staging", infos[q]["send_off"][self.rank] * row_bytes))
+            bwd_dst.append(self.seg.peer_ptr(q, "staging", infos[q]["send_off"][self.rank] * 4 * bd))
         self.bwd_dst = _ptr_array(bwd_dst)
 
         # T exchange: rows tpart.send_rows[q] of my stream table -> q's table, at q's offset for owner = me
@@ -204,14 +213,14 @@ class PeerLayerContext:
             t_dst = []
             for s, q in enumerate(self.peers):
                 self.t_seg_ptr[s + 1] = self.t_seg_ptr[s] + t_counts[q]
-                t_dst.append(self.seg.peer_ptr(q, "t_ext", (infos[q]["n_local"] + infos[q]["t_recv_off"][self.rank]) * 4 * self.t_width))
+                t_dst.append(self.seg.peer_ptr(q, "t_ext", (infos[q]["n_local"] + infos[q]["t_recv_off"][self.rank]) * elem * self.t_width))
             self.t_dst = _ptr_array(t_dst)
             self.t_dst_list, self.t_counts = t_dst, [t_counts[q] for q in self.peers]
             self.t_src = _ptr_array([self.t_ext.data_ptr()] * len(self.peers))
 
         # copy-engine pushes (overlapped exchanges): the rows are packed here first, then one contiguous copy per peer
-        pack = max(sum(send_counts) * bd, sum(self.t_counts) * self.t_width if self.tpart is not None else 0, 4)
-        self.send_buf = torch.empty(pack, dtype=torch.float32, device=self.device)
+        pack = max(sum(send_counts) * self.bd_words, sum(self.t_counts) * self.t_words if self.tpart is not None else 0, 4)
+        self.send_buf = torch.empty(pack, dtype=torch.float32, device=self.device)      # 4-byte words
 
         # deterministic reduce plan: local row -> its staging entries in ascending peer order
         if n_send:
@@ -287,7 +296,7 @@ class PeerLayerContext:
         if not fused:
             self.signal(*slots)
 
-    def _push_dma(self, table: torch.Tensor, index: torch.Tensor, counts, dst_ptrs, width: int, slots):
+    def _push_dma(self, table: torch.Tensor, index: torch.Tensor, counts, dst_ptrs, width: int, slots):      # width: words
         """The same transfer by the copy engine: pack the rows (egc_gather_rows, local), one contiguous copy per peer in
         the rotated order, then the flags.  No SM is busy while the bytes travel, so a compute kernel on another stream
         runs at full occupancy meanwhile (the posted-store kernel keeps 8 CTAs per SM resident for the whole transfer)."""
@@ -306,8 +315,9 @@ class PeerLayerContext:
     def push_forward(self, dma: bool = False):
         """My basis rows -> the halo regions of the peers that need them; the kernel's last CTA raises FWD."""
         if dma:
-            return self._push_dma(self.bases_ext, self.fwd_index, self.fwd_counts, self.fwd_dst_list, self.bd, (SLOT_FWD,))
-        self._push(len(self.peers), self.fwd_src, self.fwd_dst, self.fwd_seg_ptr, self.fwd_index.data_ptr(), self.bd,
+            return self._push_dma(self.bases_ext, self.fwd_index, self.fwd_counts, self.fwd_dst_list, self.bd_words,
+                                  (SLOT_FWD,))
+        self._push(len(self.peers), self.fwd_src, self.fwd_dst, self.fwd_seg_ptr, self.fwd_index.data_ptr(), self.bd_words,
                    (SLOT_FWD,))
 
     def push_backward(self, d_bases_ext: torch.Tensor):
@@ -321,8 +331,8 @@ class PeerLayerContext:
         """T exchange: the target-side stream rows my peers' source columns touch -> their stream tables; raises BWD and
         CONS (pass 1 is done: neither it nor the column pass reads my halo copy of the peers' basis rows)."""
         if dma:
-            return self._push_dma(self.t_ext, self.t_index, self.t_counts, self.t_dst_list, self.t_width, (SLOT_BWD, SLOT_CONS))
-        self._push(len(self.peers), self.t_src, self.t_dst, self.t_seg_ptr, self.t_index.data_ptr(), self.t_width,
+            return self._push_dma(self.t_ext, self.t_index, self.t_counts, self.t_dst_list, self.t_words, (SLOT_BWD, SLOT_CONS))
+        self._push(len(self.peers), self.t_src, self.t_dst, self.t_seg_ptr, self.t_index.data_ptr(), self.t_words,
                    (SLOT_BWD, SLOT_CONS))
 
     def reduce_into(self, d_bases_local: torch.Tensor):

@@ -291,9 +291,10 @@ int egc_aggregate_bwd(const egc_layer_desc* desc, const int32_t* rowptr, const i
 /* egc_aggregate_bwd for a layer whose forward ran on bf16 basis rows (egc_aggregate_fwd_bf16): `bases` is bf16 (read by the
  * var / std term 2 bases[j] t_sq[i]) and pass 1 stores the target-side streams t_sym / t_lin / t_sq as bf16 (round to
  * nearest even) in the workspace, which pass 2 widens and sums in fp32.  saved, the routed min/max gradients, d_weightings,
- * d_bases, d_bias and d_lin_colsum are fp32 as in egc_aggregate_bwd.  No per-entry linear weights (val_lin), no column
- * phases and no EGC_BWD_PASS1_ONLY; EGC_BWD_DETERMINISTIC and the tuning flags are honoured.  The basis rows must be
- * 36..128 values wide, a multiple of 4, 16-byte aligned.  Workspace: egc_aggregate_bwd_bf16_workspace_bytes(). */
+ * d_bases, d_bias and d_lin_colsum are fp32 as in egc_aggregate_bwd.  No per-entry linear weights (val_lin);
+ * EGC_BWD_DETERMINISTIC and the tuning flags are honoured.  The basis rows must be 36..128 values wide, a multiple of 4,
+ * 16-byte aligned.  Workspace: egc_aggregate_bwd_bf16_workspace_bytes().  Equivalent to
+ * egc_aggregate_bwd_bf16_partitioned(..., tstreams_out = NULL, flags, col_split = 0, ...). */
 size_t egc_aggregate_bwd_bf16_workspace_bytes(const egc_layer_desc* desc, const egc_row_plan* csc_plan, int32_t flags);
 int egc_aggregate_bwd_bf16(const egc_layer_desc* desc, const int32_t* rowptr, const int32_t* col, const int32_t* colptr,
                            const int32_t* rowidx, const int32_t* csr2csc, const float* csc_val_sym, const egc_row_plan* csc_plan,
@@ -301,6 +302,17 @@ int egc_aggregate_bwd_bf16(const egc_layer_desc* desc, const int32_t* rowptr, co
                            const float* grad_out, const float* out_act, const float* epi_scale, float* d_weightings,
                            float* d_bases, float* d_bias, float* d_lin_colsum, int32_t flags, void* workspace,
                            size_t workspace_bytes, void* stream);
+/* egc_aggregate_bwd_bf16 for row-partitioned callers: tstreams_out and col_split mean what they mean for egc_aggregate_bwd.
+ * EGC_BWD_PASS1_ONLY writes the target-side streams as bf16 (round to nearest even) into the first n_dst rows of
+ * tstreams_out [rows, L, B*D] (16-byte aligned) for egc_aggregate_bwd_cols_bf16; EGC_BWD_COLS_HEAD / EGC_BWD_COLS_TAIL split
+ * pass 2 at col_split (the routed min/max gradients come first and both pass-2 launches accumulate, as in fp32). */
+int egc_aggregate_bwd_bf16_partitioned(const egc_layer_desc* desc, const int32_t* rowptr, const int32_t* col,
+                                       const int32_t* colptr, const int32_t* rowidx, const int32_t* csr2csc,
+                                       const float* csc_val_sym, const egc_row_plan* csc_plan, const uint16_t* bases,
+                                       const float* weightings, const float* saved, const int32_t* saved_arg,
+                                       const float* grad_out, const float* out_act, const float* epi_scale, float* d_weightings,
+                                       float* d_bases, float* d_bias, float* d_lin_colsum, uint16_t* tstreams_out,
+                                       int32_t flags, int32_t col_split, void* workspace, size_t workspace_bytes, void* stream);
 
 /* Pass 2 alone, for row-partitioned callers that exchange the TARGET-SIDE STREAMS instead of partial sums (layers without
  * min / max; no reference counterpart, DESIGN.md "multi-GPU"): pass 1 runs through egc_aggregate_bwd with
@@ -318,12 +330,21 @@ int egc_aggregate_bwd_cols(const egc_layer_desc* desc, const int32_t* colptr, co
                            const float* csc_val_sym, const float* csc_val_lin, const egc_row_plan* csc_plan,
                            const float* tstreams, const float* bases, float* d_bases, int32_t flags,
                            void* workspace, size_t workspace_bytes, void* stream);
+/* egc_aggregate_bwd_cols over a bf16 stream table (from egc_aggregate_bwd_bf16_partitioned with EGC_BWD_PASS1_ONLY): the
+ * streams are widened and summed in fp32, `bases` are the bf16 basis rows of the columns (NULL without var / std), d_bases
+ * is fp32.  No per-entry linear weights.  Workspace: egc_aggregate_bwd_cols_workspace_bytes() (its partials are fp32). */
+int egc_aggregate_bwd_cols_bf16(const egc_layer_desc* desc, const int32_t* colptr, const int32_t* rowidx,
+                                const float* csc_val_sym, const egc_row_plan* csc_plan, const uint16_t* tstreams,
+                                const uint16_t* bases, float* d_bases, int32_t flags, void* workspace, size_t workspace_bytes,
+                                void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * Row exchange for row-partitioned graphs (no reference counterpart; see DESIGN.md "multi-GPU")
+ * egc_gather_rows and egc_peer_push_rows move rows without arithmetic: `width` counts 4-byte words, so a row of B*D bf16
+ * values (the *_bf16 entry points; B*D % 8 == 0) passes width = B*D / 2 and still moves in whole 16-byte pieces.
  * ---------------------------------------------------------------------------------------- */
 
-/* dst[k, :] = src[index[k], :]  (pack halo rows before a send / all-gather), width floats per row */
+/* dst[k, :] = src[index[k], :]  (pack halo rows before a send / all-gather), width 4-byte words per row */
 int egc_gather_rows(const float* src, const int32_t* index, int32_t n_index, int32_t width, float* dst, void* stream);
 
 /* ------------------------------------------------------------------------------------------
