@@ -13,6 +13,7 @@ LIB_PATH = os.path.join(_PKG_DIR, "libegc_b200.so")
 ABI_VERSION = 5
 EGC_MAX_AGGR = 8
 EGC_CHUNK_EDGES = 256
+MAX_PUSH_SEGMENTS = 64                     # EGC_MAX_PUSH_SEGMENTS: segments of one egc_peer_push_rows call
 META_SLOTS = 8
 META_NNZ, META_MAX_DEG, META_N_LONG, META_N_CHUNKS, META_N_LOOPS, META_ERRFLAGS = 0, 1, 2, 3, 4, 7
 LOOPS_NONE, LOOPS_ALL_NODES, LOOPS_UP_TO_MAX_ID = 0, 1, 2

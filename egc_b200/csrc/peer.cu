@@ -22,11 +22,13 @@ namespace egc {
 // ---- data movers ----------------------------------------------------------------------------------
 // One warp per row.  Segment s covers rows [seg_ptr[s], seg_ptr[s+1]) of the concatenated send list; row k of
 // segment s is  src[s] + index[k] * width  (index == null: the k-th row of the segment, counted from its start)
-// and lands at  dst[s] + (k - seg_ptr[s]) * width.
+// and lands at  dst[s] + (k - seg_ptr[s]) * width.  MAX_SEG: segment capacity of the parameter block - EGC_MAX_PEERS for
+// one table per peer (EGConv), EGC_MAX_PUSH_SEGMENTS for one segment per (peer, node type) of a heterogeneous layer.
+template <int MAX_SEG>
 struct PushParams {
-  const float* src[EGC_MAX_PEERS];
-  float* dst[EGC_MAX_PEERS];
-  int seg_ptr[EGC_MAX_PEERS + 1];
+  const float* src[MAX_SEG];
+  float* dst[MAX_SEG];
+  int seg_ptr[MAX_SEG + 1];
   int n_seg;
   const int32_t* index;
   int width;
@@ -49,8 +51,23 @@ __device__ __forceinline__ void raise_flags_of(uint32_t* const* flags, int world
   }
 }
 
-template <int VEC>
-__global__ void __launch_bounds__(256) k_peer_push(const __grid_constant__ PushParams p) {
+// The segment of list row k: the last s < n_seg with seg_ptr[s] <= k (empty segments are skipped because their successor
+// starts at the same row).  Up to EGC_MAX_PEERS segments an unrolled scan; beyond, a branchless binary search.
+template <int MAX_SEG>
+__device__ __forceinline__ int push_segment_of(const PushParams<MAX_SEG>& p, int k) {
+  int s = 0;
+  if constexpr (MAX_SEG <= EGC_MAX_PEERS) {
+#pragma unroll
+    for (int q = 1; q < MAX_SEG; ++q) s += (q < p.n_seg && k >= p.seg_ptr[q]) ? 1 : 0;
+  } else {
+#pragma unroll
+    for (int step = MAX_SEG / 2; step > 0; step >>= 1) s += (s + step < p.n_seg && k >= p.seg_ptr[s + step]) ? step : 0;
+  }
+  return s;
+}
+
+template <int VEC, int MAX_SEG>
+__global__ void __launch_bounds__(256) k_peer_push(const __grid_constant__ PushParams<MAX_SEG> p) {
   // A task = one VEC-float piece of one row; a thread keeps kPushUnroll pieces in flight (all loads, then all posted
   // stores), so narrow rows (256 B at the mag shape) use every lane and the copy runs at link speed instead of at the
   // latency of one  index -> row -> store  chain per warp.
@@ -67,9 +84,7 @@ __global__ void __launch_bounds__(256) k_peer_push(const __grid_constant__ PushP
       dst[u] = nullptr;
       if (t < total) {
         const int k = static_cast<int>(t / ppr), piece = static_cast<int>(t - static_cast<int64_t>(k) * ppr);
-        int s = 0;
-#pragma unroll
-        for (int q = 1; q < EGC_MAX_PEERS; ++q) s += (q < p.n_seg && k >= p.seg_ptr[q]) ? 1 : 0;
+        const int s = push_segment_of(p, k);
         const int local = k - p.seg_ptr[s];
         const int64_t row = p.index != nullptr ? __ldg(p.index + k) : local;
         const float* src = p.src[s] + row * p.width + piece * VEC;
@@ -260,6 +275,48 @@ __global__ void __launch_bounds__(256) k_peer_allreduce(const __grid_constant__ 
 
 static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 
+template <int MAX_SEG>
+static int launch_peer_push(int32_t n_seg, const float* const* src, float* const* dst, const int32_t* seg_ptr,
+                            const int32_t* index, int32_t width, uint32_t* const* flags, int32_t world, int32_t rank,
+                            uint32_t slot_mask, const uint32_t* epoch, uint32_t* counter, void* stream) {
+  PushParams<MAX_SEG> p{};
+  bool vec = width % 4 == 0;
+  p.n_seg = n_seg;
+  for (int s = 0; s < n_seg; ++s) {
+    p.src[s] = src[s];
+    p.dst[s] = dst[s];
+    p.seg_ptr[s] = seg_ptr[s];
+    EGC_REQUIRE(seg_ptr[s + 1] >= seg_ptr[s], "egc_peer_push_rows: seg_ptr must be non-decreasing");
+    if (seg_ptr[s + 1] > seg_ptr[s]) {
+      EGC_REQUIRE(src[s] && dst[s], "egc_peer_push_rows: null segment pointer");
+      vec = vec && aligned16(src[s]) && aligned16(dst[s]);
+    }
+  }
+  for (int s = n_seg; s <= MAX_SEG; ++s) p.seg_ptr[s] = seg_ptr[n_seg];
+  p.index = index;
+  p.width = width;
+  if (flags != nullptr && slot_mask != 0u && world > 1) {
+    EGC_REQUIRE(world <= EGC_MAX_PEERS && rank >= 0 && rank < world && epoch && counter && slot_mask < 256u,
+                "egc_peer_push_rows: bad signal arguments");
+    for (int q = 0; q < world; ++q) p.flags[q] = flags[q];
+    p.world = world; p.rank = rank; p.slot_mask = slot_mask; p.epoch = epoch; p.counter = counter;
+  }
+  const int total = seg_ptr[n_seg];
+  cudaStream_t st = as_stream(stream);
+  // one thread per 16-byte piece, 4 pieces in flight per thread (EGC_PEER_PUSH_CTAS_PER_SM: A/B runs; 1 CTA per SM measured
+  // 10 % slower on the mag shape, profiles/r02d)
+  static const int ctas_per_sm = [] { const char* e = getenv("EGC_PEER_PUSH_CTAS_PER_SM"); return e ? std::max(1, atoi(e)) : 8; }();
+  const int64_t pieces = static_cast<int64_t>(total) * (vec ? width / 4 : width);
+  const int grid = static_cast<int>(std::max<int64_t>(1, std::min<int64_t>((pieces + 1023) / 1024, static_cast<int64_t>(sm_count()) * ctas_per_sm)));
+  {
+    LaunchScope ls("k_peer_push", st);
+    if (vec) k_peer_push<4, MAX_SEG><<<grid, 256, 0, st>>>(p);
+    else k_peer_push<1, MAX_SEG><<<grid, 256, 0, st>>>(p);
+  }
+  EGC_LAUNCH_CHECK("k_peer_push");
+  return EGC_OK;
+}
+
 }  // namespace egc
 
 using namespace egc;
@@ -306,44 +363,14 @@ int egc_peer_close(void* ptr) {
 int egc_peer_push_rows(int32_t n_seg, const float* const* src, float* const* dst, const int32_t* seg_ptr,
                        const int32_t* index, int32_t width, uint32_t* const* flags, int32_t world, int32_t rank,
                        uint32_t slot_mask, const uint32_t* epoch, uint32_t* counter, void* stream) {
-  EGC_REQUIRE(n_seg >= 0 && n_seg <= EGC_MAX_PEERS && width > 0, "egc_peer_push_rows: n_seg=%d width=%d", n_seg, width);
+  EGC_REQUIRE(n_seg >= 0 && n_seg <= EGC_MAX_PUSH_SEGMENTS && width > 0, "egc_peer_push_rows: n_seg=%d width=%d", n_seg, width);
   EGC_REQUIRE(seg_ptr && (n_seg == 0 || (src && dst)), "egc_peer_push_rows: null pointer");
-  PushParams p{};
-  bool vec = width % 4 == 0;
-  p.n_seg = n_seg;
-  for (int s = 0; s < n_seg; ++s) {
-    p.src[s] = src[s];
-    p.dst[s] = dst[s];
-    p.seg_ptr[s] = seg_ptr[s];
-    EGC_REQUIRE(seg_ptr[s + 1] >= seg_ptr[s], "egc_peer_push_rows: seg_ptr must be non-decreasing");
-    if (seg_ptr[s + 1] > seg_ptr[s]) {
-      EGC_REQUIRE(src[s] && dst[s], "egc_peer_push_rows: null segment pointer");
-      vec = vec && aligned16(src[s]) && aligned16(dst[s]);
-    }
-  }
-  for (int s = n_seg; s <= EGC_MAX_PEERS; ++s) p.seg_ptr[s] = seg_ptr[n_seg];
-  p.index = index;
-  p.width = width;
-  if (flags != nullptr && slot_mask != 0u && world > 1) {
-    EGC_REQUIRE(world <= EGC_MAX_PEERS && rank >= 0 && rank < world && epoch && counter && slot_mask < 256u,
-                "egc_peer_push_rows: bad signal arguments");
-    for (int q = 0; q < world; ++q) p.flags[q] = flags[q];
-    p.world = world; p.rank = rank; p.slot_mask = slot_mask; p.epoch = epoch; p.counter = counter;
-  }
-  const int total = seg_ptr[n_seg];
-  cudaStream_t st = as_stream(stream);
-  // one thread per 16-byte piece, 4 pieces in flight per thread (EGC_PEER_PUSH_CTAS_PER_SM: A/B runs; 1 CTA per SM measured
-  // 10 % slower on the mag shape, profiles/r02d)
-  static const int ctas_per_sm = [] { const char* e = getenv("EGC_PEER_PUSH_CTAS_PER_SM"); return e ? std::max(1, atoi(e)) : 8; }();
-  const int64_t pieces = static_cast<int64_t>(total) * (vec ? width / 4 : width);
-  const int grid = static_cast<int>(std::max<int64_t>(1, std::min<int64_t>((pieces + 1023) / 1024, static_cast<int64_t>(sm_count()) * ctas_per_sm)));
-  {
-    LaunchScope ls("k_peer_push", st);
-    if (vec) k_peer_push<4><<<grid, 256, 0, st>>>(p);
-    else k_peer_push<1><<<grid, 256, 0, st>>>(p);
-  }
-  EGC_LAUNCH_CHECK("k_peer_push");
-  return EGC_OK;
+  // up to one segment per peer (EGConv) the parameter block and the segment scan of the 8-entry kernel
+  if (n_seg <= EGC_MAX_PEERS)
+    return launch_peer_push<EGC_MAX_PEERS>(n_seg, src, dst, seg_ptr, index, width, flags, world, rank, slot_mask, epoch,
+                                           counter, stream);
+  return launch_peer_push<EGC_MAX_PUSH_SEGMENTS>(n_seg, src, dst, seg_ptr, index, width, flags, world, rank, slot_mask,
+                                                 epoch, counter, stream);
 }
 
 int egc_peer_copy(void* dst, const void* src, size_t bytes, void* stream) {

@@ -20,8 +20,8 @@ Scheme (one process per GPU, torch.distributed; NCCL over NVLink on the B200 box
 go through NCCL: `transport="peer"` moves halo rows, halo gradient partial sums and the replicated parameter
 gradients with our own kernels over NVLink peer memory (`egc_b200/peer.py`, `csrc/peer.cu`).
 """
-from dataclasses import dataclass
-from typing import List, Optional
+from dataclasses import dataclass, replace
+from typing import Dict, List, Optional, Sequence, Tuple
 
 import torch
 import torch.distributed as dist
@@ -58,7 +58,9 @@ def transpose_csr(rowptr: Tensor, col: Tensor, *values: Optional[Tensor]):
 
 @dataclass
 class LocalPartition:
-    """What one rank needs (all index tensors int64 on CPU until `.to(device)`)."""
+    """What one rank needs (all index tensors int64 on CPU until `.to(device)`).  The column space is [own source rows
+    col_begin..col_end | halo rows]; a square graph owns the same range of rows and columns.  The per-type halo tables of
+    a `HeteroPartitionPlan` are LocalPartitions without a CSR (rowptr / col / interior / boundary rows are None)."""
     rank: int
     world_size: int
     row_begin: int
@@ -72,10 +74,16 @@ class LocalPartition:
     send_rows: List[Tensor]     # per peer: LOCAL row ids whose basis rows that peer needs
     interior_rows: Tensor       # local rows whose sources are all local
     boundary_rows: Tensor       # local rows that touch at least one halo source
+    col_begin: Optional[int] = None     # own source-column range (None: the row range)
+    col_end: Optional[int] = None
 
     @property
     def n_local(self) -> int:
         return self.row_end - self.row_begin
+
+    @property
+    def n_own_cols(self) -> int:
+        return self.n_local if self.col_begin is None else self.col_end - self.col_begin
 
     def split_by_column(self):
         """The local CSR cut by column locality: (entries whose column is an OWN row, entries whose column is a HALO row),
@@ -83,7 +91,7 @@ class LocalPartition:
         row = the sum over the first part (computable while the halo rows are still in flight) + the sum over the second."""
         n = self.n_local
         rows = torch.repeat_interleave(torch.arange(n), self.rowptr[1:] - self.rowptr[:-1])
-        is_own = self.col < n
+        is_own = self.col < self.n_own_cols
         parts = []
         for m in (is_own, ~is_own):
             rowptr = torch.zeros(n + 1, dtype=torch.long)
@@ -99,10 +107,13 @@ class LocalPartition:
 
 class PartitionPlan:
     """Host-side partition of a prepared global CSR (after self-loops / gcn_norm), so that symnorm
-    weights and nnz counts are the GLOBAL ones on every rank."""
+    weights and nnz counts are the GLOBAL ones on every rank.  `col_bounds`: owner ranges of the source columns of a
+    rectangular CSR (one relation of a heterogeneous graph: rows = target type, columns = source type); by default the
+    columns are owned like the rows."""
 
     def __init__(self, rowptr: Tensor, col: Tensor, world_size: int, val_sym: Optional[Tensor] = None,
-                 val_lin: Optional[Tensor] = None, bounds: Optional[List[int]] = None):
+                 val_lin: Optional[Tensor] = None, bounds: Optional[List[int]] = None,
+                 col_bounds: Optional[List[int]] = None):
         self.rowptr, self.col = rowptr.long().cpu(), col.long().cpu()
         self.val_sym = val_sym.cpu() if val_sym is not None else None
         self.val_lin = val_lin.cpu() if val_lin is not None else None
@@ -111,24 +122,29 @@ class PartitionPlan:
         if self.n < world_size:
             raise ValueError(f"cannot partition {self.n} rows over {world_size} ranks: every rank needs at least one row")
         self.bounds = bounds or balanced_row_bounds(self.rowptr, world_size)
-        self._bounds_t = torch.tensor(self.bounds, dtype=torch.long)
+        self.col_bounds = list(col_bounds) if col_bounds is not None else self.bounds
+        if len(self.bounds) != world_size + 1 or len(self.col_bounds) != world_size + 1:
+            raise ValueError(f"row / column bounds need {world_size + 1} entries")
+        self._bounds_t = torch.tensor(self.col_bounds, dtype=torch.long)
         self._needs = [self._needed_remote(r) for r in range(world_size)]      # [rank][owner] -> ids
 
     def owner_of(self, ids: Tensor) -> Tensor:
+        """Rank that owns each source column id."""
         return torch.searchsorted(self._bounds_t, ids, right=True) - 1
 
     def transposed(self) -> "PartitionPlan":
         """The same node ranges over the TRANSPOSED adjacency: rank p's rows are its own SOURCE columns, its halo the
         remote TARGETS that aggregate them - what the backward's T exchange needs (see the module docstring)."""
-        if int(self.col.max()) >= self.n if self.col.numel() else False:
+        if (int(self.col.max()) >= self.n if self.col.numel() else False) or self.col_bounds != self.bounds:
             raise ValueError("the transposed plan needs a square adjacency")
         rowptr_t, col_t, sym_t, lin_t = transpose_csr(self.rowptr, self.col, self.val_sym, self.val_lin)
         return PartitionPlan(rowptr_t, col_t, self.world_size, val_sym=sym_t, val_lin=lin_t, bounds=list(self.bounds))
 
     def _needed_remote(self, rank: int) -> List[Tensor]:
         b, e = self.bounds[rank], self.bounds[rank + 1]
+        cb, ce = self.col_bounds[rank], self.col_bounds[rank + 1]
         cols = self.col[self.rowptr[b]:self.rowptr[e]]
-        remote = torch.unique(cols[(cols < b) | (cols >= e)])
+        remote = torch.unique(cols[(cols < cb) | (cols >= ce)])
         owner = self.owner_of(remote)
         return [remote[owner == q] for q in range(self.world_size)]
 
@@ -137,22 +153,93 @@ class PartitionPlan:
         lo, hi = int(self.rowptr[b]), int(self.rowptr[e])
         rowptr = self.rowptr[b:e + 1] - lo
         cols = self.col[lo:hi]
+        cb, ce = self.col_bounds[rank], self.col_bounds[rank + 1]
         halo_ids = torch.cat(self._needs[rank]) if self.world_size > 1 else cols.new_zeros(0)
         n_local = e - b
-        is_local = (cols >= b) & (cols < e)
-        col_ext = torch.where(is_local, cols - b, n_local + torch.searchsorted(halo_ids, cols)
-                              if halo_ids.numel() else cols - b)
+        is_local = (cols >= cb) & (cols < ce)
+        col_ext = torch.where(is_local, cols - cb, (ce - cb) + torch.searchsorted(halo_ids, cols)
+                              if halo_ids.numel() else cols - cb)
         # halo_ids is sorted globally because owners are contiguous ascending ranges
         rows = torch.repeat_interleave(torch.arange(n_local), rowptr[1:] - rowptr[:-1])
         touches = torch.zeros(n_local, dtype=torch.bool)
         touches[rows[~is_local]] = True
-        send_rows = [self._needs[q][rank] - b for q in range(self.world_size)]
+        send_rows = [self._needs[q][rank] - cb for q in range(self.world_size)]
         return LocalPartition(
             rank=rank, world_size=self.world_size, row_begin=b, row_end=e, rowptr=rowptr, col=col_ext,
             val_sym=self.val_sym[lo:hi] if self.val_sym is not None else None,
             val_lin=self.val_lin[lo:hi] if self.val_lin is not None else None,
             halo_ids=halo_ids, recv_counts=[int(t.numel()) for t in self._needs[rank]], send_rows=send_rows,
-            interior_rows=torch.nonzero(~touches).flatten(), boundary_rows=torch.nonzero(touches).flatten())
+            interior_rows=torch.nonzero(~touches).flatten(), boundary_rows=torch.nonzero(touches).flatten(),
+            col_begin=cb, col_end=ce)
+
+
+@dataclass
+class HeteroLocalPartition:
+    """One rank's share of a heterogeneous graph: per node type the exchange table (own rows + the union halo of every
+    relation that reads that type, a `LocalPartition` without CSR), per relation the local CSR over this rank's target
+    rows whose column ids point into the [own | halo] table of its source type (halo fields = those of that table)."""
+    tables: Dict[str, LocalPartition]
+    relations: Dict[Tuple[str, str, str], LocalPartition]
+
+
+class HeteroPartitionPlan:
+    """Row partition of a heterogeneous graph {(src, rel, dst): (rowptr [n_dst + 1], col)} over node types `sizes`: every
+    type gets its own contiguous row ranges, balanced by the rows + nnz of the relations that target it, so every rank
+    owns rows of every type.  Each relation is a rectangular `PartitionPlan` (rows owned like its target type, columns
+    like its source type); a rank's halo of type s is the union of the remote s ids its target rows reference in every
+    relation (s, r, t), grouped by owner and ascending - ONE halo per source type, shared by all relations reading it."""
+
+    def __init__(self, csr_dict, sizes: Dict[str, int], world_size: int, values=None):
+        self.types, self.keys, self.world_size = list(sizes), list(csr_dict), world_size
+        for t, n in sizes.items():
+            if n < world_size:
+                raise ValueError(f"cannot partition {n} rows of node type {t!r} over {world_size} ranks: every rank "
+                                 "needs at least one row of every type")
+        csr = {}
+        for k, (rowptr, col) in csr_dict.items():
+            if k[0] not in sizes or k[2] not in sizes:
+                raise ValueError(f"relation {k} names a node type outside {self.types}")
+            if rowptr.numel() != sizes[k[2]] + 1:
+                raise ValueError(f"relation {k} has {rowptr.numel() - 1} rows, node type {k[2]!r} has {sizes[k[2]]}")
+            csr[k] = (rowptr.long().cpu(), col.long().cpu())
+        self.bounds = {}
+        for t in self.types:
+            rowptr = torch.zeros(sizes[t] + 1, dtype=torch.long)
+            for k, (rp, _) in csr.items():
+                if k[2] == t:
+                    rowptr = rowptr + rp
+            self.bounds[t] = balanced_row_bounds(rowptr, world_size)
+        values = values or {}
+        self.plans = {k: PartitionPlan(rp, col, world_size, val_lin=values.get(k), bounds=self.bounds[k[2]],
+                                       col_bounds=self.bounds[k[0]]) for k, (rp, col) in csr.items()}
+
+    def _type_needs(self, s: str, reader: int, owner: int) -> Tensor:
+        """Ascending ids of type s owned by `owner` that `reader` reads, over every relation with source s."""
+        parts = [p._needs[reader][owner] for k, p in self.plans.items() if k[0] == s]
+        return torch.unique(torch.cat(parts)) if parts else torch.zeros(0, dtype=torch.long)
+
+    def local(self, rank: int) -> HeteroLocalPartition:
+        w = self.world_size
+        tables = {}
+        for s in self.types:
+            cb, ce = self.bounds[s][rank], self.bounds[s][rank + 1]
+            needs = [self._type_needs(s, rank, q) for q in range(w)]
+            halo_ids = torch.cat(needs) if w > 1 else torch.zeros(0, dtype=torch.long)
+            send_rows = [self._type_needs(s, q, rank) - cb for q in range(w)]
+            tables[s] = LocalPartition(rank=rank, world_size=w, row_begin=cb, row_end=ce, rowptr=None, col=None,
+                                       val_sym=None, val_lin=None, halo_ids=halo_ids,
+                                       recv_counts=[int(t.numel()) for t in needs], send_rows=send_rows,
+                                       interior_rows=None, boundary_rows=None, col_begin=cb, col_end=ce)
+        relations = {}
+        for k, plan in self.plans.items():
+            lp, tab = plan.local(rank), tables[k[0]]
+            n_own = tab.n_local
+            is_halo = lp.col >= n_own                   # relation halo slot -> the same id's slot in the type's halo
+            col = lp.col.clone()
+            col[is_halo] = n_own + torch.searchsorted(tab.halo_ids, lp.halo_ids[lp.col[is_halo] - n_own])
+            relations[k] = replace(lp, col=col, halo_ids=tab.halo_ids, recv_counts=tab.recv_counts,
+                                   send_rows=tab.send_rows)
+        return HeteroLocalPartition(tables, relations)
 
 
 class HaloExchange:
@@ -580,6 +667,177 @@ def partitioned_egconv(x_local: Tensor, pg: PartitionedGraph, conv, relu: bool =
                                             conv.bias, pg, conv.num_heads, conv.num_bases, tuple(conv.aggregators),
                                             bool(conv.sigmoid), int(conv.gemm_algo), id(conv), torch.is_grad_enabled(),
                                             _bwd_flags_of(conv), bool(relu), storage_dtype)
+
+
+class PartitionedHeteroGraph:
+    """Device-side state of one rank of a row-partitioned heterogeneous graph (`REGConv`): per relation the local CSR
+    ([own target rows] x [own | halo] rows of its source type), per node type the halo exchange.  Pass it to
+    `REGConv.forward` in place of the adjacency dict; the layer then returns this rank's rows of every type.
+
+    transport = "peer" (default): every layer gets one peer segment holding the [own | halo] basis table of every node
+    type; ONE push moves the halo rows of all types, ONE push sends their partial sums home, ONE reduce adds them in fixed
+    peer order, ONE kernel all-reduces the parameter gradients (`egc_b200.peer`).  transport = "nccl": one
+    `CudaHaloExchange` per node type and `dist.all_reduce` (the library baseline)."""
+
+    def __init__(self, part: HeteroLocalPartition, device, group=None, transport: str = "peer"):
+        from .graph import GraphStructure
+        if transport not in ("peer", "nccl"):
+            raise ValueError(f"unknown transport {transport!r}")
+        self.part, self.device, self.group, self.transport = part, torch.device(device), group, transport
+        self.types = list(part.tables)
+        self.edge_types = list(part.relations)          # the order of the adjacency dict: the accumulation order
+        self.graphs = {}
+        for k, rel in part.relations.items():
+            tab = part.tables[k[0]]
+            self.graphs[k] = GraphStructure.from_prepared(rel.rowptr, rel.col, tab.n_local + tab.n_halo,
+                                                          val_lin=rel.val_lin, device=self.device)
+        self.exchanges = {t: CudaHaloExchange(tab, self.device, group) for t, tab in part.tables.items()}
+        self._peer_ctx = {}
+
+    @staticmethod
+    def from_global(adj_t_dict, sizes: Dict[str, int], rank: int, world_size: int, device, group=None,
+                    transport: str = "peer") -> "PartitionedHeteroGraph":
+        """Partition a dict of whole-graph adjacencies {(src, rel, dst): adj_t} (rows = targets) over node types with
+        `sizes` rows each (every rank builds the same plan).  Raises ValueError, on every rank alike and before anything
+        collective, when a type has fewer rows than there are ranks."""
+        from .graph import adjacency_to_csr
+        csr, values = {}, {}
+        for k, adj in adj_t_dict.items():
+            rowptr, col, value, n_src = adjacency_to_csr(adj)
+            if k[0] in sizes and n_src != sizes[k[0]]:
+                raise ValueError(f"adjacency of {k} has {n_src} columns, node type {k[0]!r} has {sizes[k[0]]} rows")
+            csr[k] = (rowptr.cpu(), col.cpu())
+            if value is not None:
+                values[k] = value.cpu()
+        plan = HeteroPartitionPlan(csr, sizes, world_size, values)
+        return PartitionedHeteroGraph(plan.local(rank), device, group, transport)
+
+    def row_range(self, node_type: str) -> Tuple[int, int]:
+        """(begin, end) of the global rows of `node_type` this rank owns."""
+        tab = self.part.tables[node_type]
+        return tab.row_begin, tab.row_end
+
+    def peer_context(self, key, bd: int, n_flat: int):
+        """Exchange state of one layer (collective on first use: every rank must reach it in the same order)."""
+        k = (key, int(bd), int(n_flat))
+        ctx = self._peer_ctx.get(k)
+        if ctx is None:
+            from .peer import PeerLayerContext
+            ctx = PeerLayerContext([self.part.tables[t] for t in self.types], bd, n_flat, self.device, self.group)
+            self._peer_ctx[k] = ctx
+        return ctx
+
+    def exchange(self, key, n_flat: int, bases: Dict[str, Tensor]) -> Dict[str, Tensor]:
+        """{type: own basis rows} -> {type: [own | halo] rows}, differentiable (backward: halo partial sums go home)."""
+        tables = _HeteroHaloFunction.apply(self, key, int(n_flat), torch.is_grad_enabled(), *[bases[t] for t in self.types])
+        return dict(zip(self.types, tables))
+
+    def replicated(self, key, params: Sequence[Tensor]) -> Tuple[Tensor, ...]:
+        """The same parameters; their gradients are summed over the ranks (one flat all-reduce per layer)."""
+        return _ReplicatedParamsFunction.apply(self, key, *params)
+
+    def end_forward(self, key, bd: int, n_flat: int) -> None:
+        """After the last relation launch of a forward that saved nothing for a backward: release the peers' rows (CONS)."""
+        from . import peer as P
+        ctx = self._peer_ctx.get((key, int(bd), int(n_flat)))
+        if ctx is not None and not ctx.outstanding:
+            ctx.signal(P.SLOT_CONS)
+
+    def check(self):
+        """Raise if any exchange of this graph timed out on the device (synchronises)."""
+        for ctx in self._peer_ctx.values():
+            ctx.check()
+
+    def close(self):
+        for ctx in self._peer_ctx.values():
+            ctx.close()
+        self._peer_ctx = {}
+
+
+class _HeteroHaloFunction(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, phg, key, n_flat, grad_mode, *bases):
+        from . import peer as P
+        types = phg.types
+        tabs = [phg.part.tables[t] for t in types]
+        bd = bases[0].size(1)
+        for t, b, tab in zip(types, bases, tabs):
+            if b.dtype != torch.float32 or not b.is_cuda or tuple(b.shape) != (tab.n_local, bd):
+                raise ValueError(f"bases of node type {t!r} must be CUDA fp32 [{tab.n_local}, {bd}] (got {b.dtype} "
+                                 f"{tuple(b.shape)} on {b.device})")
+        needs_grad = grad_mode and any(ctx.needs_input_grad[4:])       # needs_input_grad ignores torch.no_grad()
+        peer = None
+        with torch.cuda.device(bases[0].device):
+            if phg.transport == "peer":
+                peer = phg.peer_context(key, bd, n_flat)
+                ctx.step_id = peer.begin_step(needs_grad)       # every peer is done with the halo rows of my last step
+                out = [peer.table(i) for i in range(len(types))]
+                for o, b, tab in zip(out, bases, tabs):
+                    o[:tab.n_local].copy_(b)
+                peer.push_forward()                             # every type's halo rows to every peer, then FWD flag
+                peer.wait(P.SLOT_FWD)
+            else:
+                out = [torch.cat([b, phg.exchanges[t].forward(b)]) for t, b in zip(types, bases)]
+        ctx.phg, ctx.peer, ctx.bd = phg, peer, bd
+        return tuple(out)
+
+    @staticmethod
+    def backward(ctx, *d_ext):
+        from . import peer as P
+        phg, peer = ctx.phg, ctx.peer
+        tabs = [phg.part.tables[t] for t in phg.types]
+        dev = phg.device
+        d_ext = [d.contiguous() if d is not None else torch.zeros((tab.n_local + tab.n_halo, ctx.bd), device=dev)
+                 for d, tab in zip(d_ext, tabs)]
+        with torch.cuda.device(dev):
+            if peer is None:
+                d_own = []
+                for t, d, tab in zip(phg.types, d_ext, tabs):
+                    own = d[:tab.n_local].clone()
+                    phg.exchanges[t].reverse(d[tab.n_local:], own)       # halo partial sums go home
+                    d_own.append(own)
+                return (None,) * 4 + tuple(d_own)
+            peer.begin_backward(ctx.step_id)
+            stacked = torch.cat([d[:tab.n_local] for d, tab in zip(d_ext, tabs)])     # [own t0 | own t1 | ...]
+            peer.push_backward(*d_ext)                          # every type's halo partial sums home, BWD + CONS flags
+            peer.wait(P.SLOT_BWD)
+            peer.reduce_into(stacked)                           # fixed peer order: deterministic
+        return (None,) * 4 + tuple(stacked.split([tab.n_local for tab in tabs]))
+
+
+class _ReplicatedParamsFunction(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, phg, key, *params):
+        ctx.phg, ctx.key, ctx.sizes = phg, key, [p.numel() for p in params]
+        ctx.set_materialize_grads(False)
+        return tuple(p.view_as(p) for p in params)
+
+    @staticmethod
+    def backward(ctx, *grads):
+        phg, n = ctx.phg, sum(ctx.sizes)
+        with torch.cuda.device(phg.device):
+            if phg.transport == "peer":                  # the layer's exchange context (made by its forward)
+                peer = next(c for k, c in phg._peer_ctx.items() if k[0] == ctx.key and k[2] == n)
+                flat = peer.flat
+            else:
+                flat = torch.empty(n, dtype=torch.float32, device=phg.device)
+            off = 0
+            for g, m in zip(grads, ctx.sizes):           # fixed layout [param 0 | param 1 | ...], unused ones zero
+                if g is not None:
+                    flat[off:off + m].copy_(g.reshape(-1))
+                else:
+                    flat[off:off + m].zero_()
+                off += m
+            if phg.transport == "peer":
+                total = peer.allreduce_flat()
+            else:
+                dist.all_reduce(flat, op=dist.ReduceOp.SUM, group=phg.group)
+                total = flat
+            out, off = [], 0
+            for g, m in zip(grads, ctx.sizes):
+                out.append(total[off:off + m].view_as(g).clone() if g is not None else None)
+                off += m
+        return (None, None) + tuple(out)
 
 
 class GraphedStep:

@@ -39,7 +39,10 @@ EdgeType = Tuple[str, str, str]
 class REGConv(torch.nn.Module):
     def __init__(self, in_channels: int, out_channels: int, num_heads: int, num_bases: int,
                  node_types: Sequence[str] = NODE_TYPES, edge_types: Sequence[EdgeType] = EDGE_TYPES,
-                 cached: bool = True, gemm_algo: int = _lib.GEMM_AUTO, *, storage_dtype: torch.dtype = torch.float32):
+                 cached: bool = True, gemm_algo: int = _lib.GEMM_AUTO, *, storage_dtype: torch.dtype = torch.float32,
+                 deterministic: bool = False):
+        """deterministic: route the max gradients of the relations without fp32 atomics, so the backward gives the same
+        bits on every run (as `EGConv(..., deterministic=True)`)."""
         super().__init__()
         if storage_dtype != torch.float32:
             raise NotImplementedError("REGConv: bf16 storage is not supported; use storage_dtype=torch.float32")
@@ -49,6 +52,7 @@ class REGConv(torch.nn.Module):
         self.num_heads, self.num_bases = num_heads, num_bases
         self.node_types, self.edge_types = tuple(node_types), tuple(tuple(k) for k in edge_types)
         self.cached, self.gemm_algo = cached, gemm_algo
+        self.deterministic = deterministic
         self.bases_weight = Parameter(torch.empty(in_channels, (out_channels // num_heads) * num_bases))
         self.rel_combs = ModuleDict({f"{k[0]}_{k[1]}_{k[2]}": Linear(in_channels, 2 * num_heads * num_bases)
                                      for k in self.edge_types})                                  # ref :89-97
@@ -88,35 +92,58 @@ class REGConv(torch.nn.Module):
             self._graphs[key] = (adj_t, g)
         return g
 
-    def forward(self, x_dict: Dict[str, Tensor], adj_t_dict: Dict[EdgeType, object]) -> Dict[str, Tensor]:
+    def forward(self, x_dict: Dict[str, Tensor], adj_t_dict) -> Dict[str, Tensor]:
+        """`adj_t_dict`: {(src, rel, dst): adj_t} over whole node sets, or an `egc_b200.dist.PartitionedHeteroGraph` with
+        `x_dict` holding this rank's rows of every type (`row_range`): the result is then this rank's rows of the
+        single-GPU layer's output, and the parameter gradients are summed over the ranks."""
+        from .dist import PartitionedHeteroGraph
+        phg = adj_t_dict if isinstance(adj_t_dict, PartitionedHeteroGraph) else None
+        keys = phg.edge_types if phg is not None else list(adj_t_dict)
         h, b = self.num_heads, self.num_bases
         hb = h * b
+        bwd_flags = _lib.BWD_DETERMINISTIC if self.deterministic else 0
+        names, params = map(list, zip(*self.named_parameters()))
+        if phg is not None:
+            unknown = [k for k in keys if k not in self.edge_types]
+            if unknown:
+                raise ValueError(f"REGConv: relations {unknown} of the partitioned graph are not among the layer's edge types")
+            if set(x_dict) != set(phg.types):
+                raise ValueError(f"REGConv: x_dict has node types {sorted(x_dict)}, the partitioned graph {sorted(phg.types)}")
+            key, n_flat = id(self), sum(p.numel() for p in params)
+            params = phg.replicated(key, params)        # gradients summed over the ranks
+        P = dict(zip(names, params))
         # relations grouped by the node type they write to, in adj_t_dict order (the reference's accumulation order)
-        incoming = {t: [k for k in adj_t_dict if k[2] == t] for t in x_dict}
+        incoming = {t: [k for k in keys if k[2] == t] for t in x_dict}
         bases, weights = {}, {}
         for t, x in x_dict.items():
             if not x.is_cuda:
                 raise RuntimeError("egc_b200.REGConv runs on CUDA (sm_100a) only; move the module and inputs to the GPU")
-            lins = [self.root_combs[t]] + [self.rel_combs[f"{k[0]}_{k[1]}_{k[2]}"] for k in incoming[t]]
-            w_cat = torch.cat([lin.weight for lin in lins], 0) if len(lins) > 1 else lins[0].weight
-            b_cat = torch.cat([lin.bias for lin in lins], 0) if len(lins) > 1 else lins[0].bias
-            bases[t], weights[t] = project_autograd(x, self.bases_weight, w_cat, b_cat, self.gemm_algo)
+            lins = [f"root_combs.{t}"] + [f"rel_combs.{k[0]}_{k[1]}_{k[2]}" for k in incoming[t]]
+            w_cat = torch.cat([P[n + ".weight"] for n in lins], 0) if len(lins) > 1 else P[lins[0] + ".weight"]
+            b_cat = torch.cat([P[n + ".bias"] for n in lins], 0) if len(lins) > 1 else P[lins[0] + ".bias"]
+            bases[t], weights[t] = project_autograd(x, P["bases_weight"], w_cat, b_cat, self.gemm_algo)
+        # source tables: the own rows, or [own | halo] rows of every type after the halo exchange
+        src = phg.exchange(key, n_flat, bases) if phg is not None else bases
         out = {}
         for t, x in x_dict.items():
             w_root = weights[t][:, :hb].contiguous()
             if x.size(0) == 0:                                  # a node type without nodes (ref handles empty tensors)
                 out[t] = x.new_zeros((0, self.out_channels)) + weights[t].sum() * 0.0
                 continue
-            out[t] = aggregate_combine_autograd(bases[t], w_root, None, self._identity(x.size(0), x.device), h, b, ("sum",))
+            own = src[t] if src[t].size(0) == x.size(0) else src[t][:x.size(0)]
+            out[t] = aggregate_combine_autograd(own, w_root, None, self._identity(x.size(0), x.device), h, b, ("sum",))
             for i, k in enumerate(incoming[t]):
-                if bases[k[0]].size(0) == 0:                    # relation from an empty node type: contributes nothing
+                if src[k[0]].size(0) == 0:                      # relation from an empty node type: contributes nothing
                     continue
-                g = self._relation(k, adj_t_dict[k], x.device)
-                if g.n_dst != x.size(0) or g.n_src != bases[k[0]].size(0):
-                    raise ValueError(f"adjacency of {k} is {g.n_dst} x {g.n_src}, expected {x.size(0)} x {bases[k[0]].size(0)}")
+                g = phg.graphs[k] if phg is not None else self._relation(k, adj_t_dict[k], x.device)
+                if g.n_dst != x.size(0) or g.n_src != src[k[0]].size(0):
+                    raise ValueError(f"adjacency of {k} is {g.n_dst} x {g.n_src}, expected {x.size(0)} x {src[k[0]].size(0)}")
                 w_rel = weights[t][:, hb + 2 * hb * i: hb + 2 * hb * (i + 1)].contiguous()
                 # root_combined[t] += ... (ref :146): the running sum is the `add` input of the kernel's epilogue
-                out[t] = aggregate_combine_autograd(bases[k[0]], w_rel, None, g, h, b, ("mean", "max"), add=out[t])
+                out[t] = aggregate_combine_autograd(src[k[0]], w_rel, None, g, h, b, ("mean", "max"), bwd_flags,
+                                                    add=out[t])
+        if phg is not None:
+            phg.end_forward(key, bases[phg.types[0]].size(1), n_flat)
         return out
 
     def __repr__(self):

@@ -121,34 +121,54 @@ def _ptr_array(values: List[int]):
 
 class PeerLayerContext:
     """Exchange state of one layer (basis width `bd`, `n_flat` replicated parameter-gradient floats) on one rank.
+    `part` is one `LocalPartition` (EGConv: one [own | halo] basis table) or a list of them, one table per node type of a
+    heterogeneous layer (`egc_b200.dist.PartitionedHeteroGraph`): every table gets its own [own | halo] region and staging
+    rows, and each exchange moves the rows of ALL tables in one push - segments per (peer, table), peers in the rotated
+    order outside, tables inside - with one flag; the reduce adds the partial sums into the stacked own rows
+    [own 0 | own 1 | ...].  The T exchange and the copy-engine pushes take one table.
     storage_dtype=torch.bfloat16: the basis rows (`bases_ext`) and the target-side stream rows (`t_ext`) are stored and
     pushed as bf16 - half the bytes per exchanged row; the halo partial sums (`staging`) and the parameter-gradient slots
     stay fp32."""
 
     def __init__(self, part, bd: int, n_flat: int, device, group=None, timeout_ns: int = DEFAULT_TIMEOUT_NS,
                  tpart=None, t_width: int = 0, storage_dtype: torch.dtype = torch.float32):
-        self.part, self.bd, self.device, self.group = part, int(bd), torch.device(device), group
+        tables = list(part) if isinstance(part, (list, tuple)) else [part]
+        self.tables = tables
+        self.part, self.bd, self.device, self.group = tables[0], int(bd), torch.device(device), group
         self.storage_dtype = storage_dtype
         elem = torch.empty((), dtype=storage_dtype).element_size()            # bytes per stored basis / stream value
         self.tpart, self.t_width = (tpart, int(t_width)) if tpart is not None and t_width else (None, 0)
-        self.rank, self.world = part.rank, part.world_size
+        if len(tables) > 1 and self.tpart is not None:
+            raise ValueError("the T exchange takes one table")
+        self.rank, self.world = self.part.rank, self.part.world_size
+        if (self.world - 1) * len(tables) > _lib.MAX_PUSH_SEGMENTS:           # same on every rank, nothing collective yet
+            raise ValueError(f"{len(tables)} tables over {self.world} ranks need {(self.world - 1) * len(tables)} push "
+                             f"segments, more than {_lib.MAX_PUSH_SEGMENTS}")
         self.timeout_ns = int(timeout_ns)
         self.n_flat = _align(int(n_flat), 128)                     # rows of 128 floats for the slot pushes
-        n_ext = part.n_local + part.n_halo
-        send_counts = [int(t.numel()) for t in part.send_rows]
-        n_send = sum(send_counts) if self.tpart is None else 0     # T exchange: no partial sums, no staging
+        n_ext = [t.n_local + t.n_halo for t in tables]
+        send_counts = [[int(r.numel()) for r in t.send_rows] for t in tables]
+        n_send = [sum(c) if self.tpart is None else 0 for c in send_counts]     # T exchange: no partial sums, no staging
+        stage_off = [0]                                            # staging rows of table i start at stage_off[i]
+        for c in n_send:
+            stage_off.append(stage_off[-1] + c)
+        own_off = [0]                                              # stacked own rows [own 0 | own 1 | ...]
+        for t in tables:
+            own_off.append(own_off[-1] + t.n_local)
         n_ext_t = (self.tpart.n_local + self.tpart.n_halo) if self.tpart is not None else 0
         # the push kernels move 4-byte words: row widths of the stored tables in words (bf16 rows: whole 16-byte pieces)
         if elem != 4 and (self.bd % 8 or self.t_width % 8):
             raise ValueError(f"bf16 exchange rows need B*D % 8 == 0 (got {self.bd})")
         self.bd_words, self.t_words = self.bd * elem // 4, self.t_width * elem // 4
-        self.seg = PeerSegment([("flags", 4 * N_SLOTS * self.world), ("bases_ext", elem * n_ext * bd),
-                                ("staging", 4 * max(n_send, 1) * bd), ("slots", 4 * self.world * self.n_flat),
+        self.seg = PeerSegment([("flags", 4 * N_SLOTS * self.world)] +
+                               [(f"bases_ext{i}", elem * n * bd) for i, n in enumerate(n_ext)] +
+                               [("staging", 4 * max(stage_off[-1], 1) * bd), ("slots", 4 * self.world * self.n_flat),
                                 ("t_ext", elem * n_ext_t * self.t_width)], device, group)
         self.t_ext = self.seg.view("t_ext", (n_ext_t, self.t_width), storage_dtype) if self.tpart is not None else None
         self.flags = self.seg.view("flags", (N_SLOTS * self.world,), torch.int32)
-        self.bases_ext = self.seg.view("bases_ext", (n_ext, bd), storage_dtype)
-        self.staging = self.seg.view("staging", (max(n_send, 1), bd))
+        self.n_ext = n_ext
+        self.bases_ext = self.table(0)
+        self.staging = self.seg.view("staging", (max(stage_off[-1], 1), bd))
         self.slots = self.seg.view("slots", (self.world, self.n_flat))
         self.epoch = torch.zeros(1, dtype=torch.int32, device=self.device)
         self.err = torch.zeros(1, dtype=torch.int32, device=self.device)
@@ -161,20 +181,23 @@ class PeerLayerContext:
         self.outstanding = False
         self.side_stream = torch.cuda.Stream(device=self.device)      # carries the backward push next to pass 2
 
-        # what every rank must know about the others: local row counts, halo layout, staging layout
-        recv_off = [0]
-        for c in part.recv_counts:
-            recv_off.append(recv_off[-1] + c)
-        send_off = [0]
-        for c in send_counts:
-            send_off.append(send_off[-1] + c)
+        # what every rank must know about the others: local row counts, halo layout, staging layout (per table)
+        recv_off, send_off = [], []
+        for t, counts in zip(tables, send_counts):
+            r_off, s_off = [0], [0]
+            for c in t.recv_counts:
+                r_off.append(r_off[-1] + c)
+            for c in counts:
+                s_off.append(s_off[-1] + c)
+            recv_off.append(r_off)
+            send_off.append(s_off)
         self.recv_off, self.send_off = recv_off, send_off
         infos = [None] * self.world
         t_recv_off = [0]
         for c in (self.tpart.recv_counts if self.tpart is not None else []):
             t_recv_off.append(t_recv_off[-1] + c)
-        dist.all_gather_object(infos, {"n_local": part.n_local, "recv_off": recv_off, "send_off": send_off,
-                                       "t_recv_off": t_recv_off}, group=group)
+        dist.all_gather_object(infos, {"n_local": [t.n_local for t in tables], "recv_off": recv_off, "send_off": send_off,
+                                       "stage_off": stage_off, "t_recv_off": t_recv_off}, group=group)
         # Destination order of every push: rank + 1, rank + 2, ... (mod world).  The push kernel walks its segments in
         # this order, so at any moment the ranks write to DIFFERENT destinations; with the ascending order every rank
         # started on rank 0 (7 senders into one ingress port), then rank 1, ...  (EGC_PEER_ORDER=ascending: A/B)
@@ -182,26 +205,29 @@ class PeerLayerContext:
             self.peers = [q for q in range(self.world) if q != self.rank]
         else:
             self.peers = [(self.rank + k) % self.world for k in range(1, self.world)]
+        self.segments = [(q, i) for q in self.peers for i in range(len(tables))]      # peers outside, tables inside
         row_bytes = elem * bd
 
-        # forward push: rows send_rows[q] of my basis table -> q's halo region, at q's offset for owner = me
-        self.fwd_index = (torch.cat([part.send_rows[q] for q in self.peers]) if self.peers else
+        # forward push: rows send_rows[q] of my table i -> q's halo region of table i, at q's offset for owner = me
+        self.fwd_index = (torch.cat([tables[i].send_rows[q] for q, i in self.segments]) if self.segments else
                           torch.zeros(0, dtype=torch.long)).to(self.device, torch.int32)
-        self.fwd_seg_ptr = (ctypes.c_int32 * (len(self.peers) + 1))()
+        self.fwd_seg_ptr = (ctypes.c_int32 * (len(self.segments) + 1))()
         fwd_dst = []
-        for s, q in enumerate(self.peers):
-            self.fwd_seg_ptr[s + 1] = self.fwd_seg_ptr[s] + send_counts[q]
-            fwd_dst.append(self.seg.peer_ptr(q, "bases_ext", (infos[q]["n_local"] + infos[q]["recv_off"][self.rank]) * row_bytes))
+        for s, (q, i) in enumerate(self.segments):
+            self.fwd_seg_ptr[s + 1] = self.fwd_seg_ptr[s] + send_counts[i][q]
+            fwd_dst.append(self.seg.peer_ptr(q, f"bases_ext{i}",
+                                             (infos[q]["n_local"][i] + infos[q]["recv_off"][i][self.rank]) * row_bytes))
         self.fwd_dst = _ptr_array(fwd_dst)
-        self.fwd_dst_list, self.fwd_counts = fwd_dst, [send_counts[q] for q in self.peers]
-        self.fwd_src = _ptr_array([self.bases_ext.data_ptr()] * len(self.peers))
+        self.fwd_dst_list, self.fwd_counts = fwd_dst, [send_counts[i][q] for q, i in self.segments]
+        self.fwd_src = _ptr_array([self.seg.peer_ptr(self.rank, f"bases_ext{i}") for _, i in self.segments])
 
-        # backward push: my halo segment owned by q (contiguous) -> q's staging, at q's offset for sender = me
-        self.bwd_seg_ptr = (ctypes.c_int32 * (len(self.peers) + 1))()
+        # backward push: my halo rows of table i owned by q (contiguous) -> q's staging, at q's offset for sender = me
+        self.bwd_seg_ptr = (ctypes.c_int32 * (len(self.segments) + 1))()
         bwd_dst = []
-        for s, q in enumerate(self.peers):
-            self.bwd_seg_ptr[s + 1] = self.bwd_seg_ptr[s] + part.recv_counts[q]
-            bwd_dst.append(self.seg.peer_ptr(q, "staging", infos[q]["send_off"][self.rank] * 4 * bd))
+        for s, (q, i) in enumerate(self.segments):
+            self.bwd_seg_ptr[s + 1] = self.bwd_seg_ptr[s] + tables[i].recv_counts[q]
+            bwd_dst.append(self.seg.peer_ptr(q, "staging",
+                                             (infos[q]["stage_off"][i] + infos[q]["send_off"][i][self.rank]) * 4 * bd))
         self.bwd_dst = _ptr_array(bwd_dst)
 
         # T exchange: rows tpart.send_rows[q] of my stream table -> q's table, at q's offset for owner = me
@@ -213,26 +239,33 @@ class PeerLayerContext:
             t_dst = []
             for s, q in enumerate(self.peers):
                 self.t_seg_ptr[s + 1] = self.t_seg_ptr[s] + t_counts[q]
-                t_dst.append(self.seg.peer_ptr(q, "t_ext", (infos[q]["n_local"] + infos[q]["t_recv_off"][self.rank]) * elem * self.t_width))
+                t_dst.append(self.seg.peer_ptr(q, "t_ext", (infos[q]["n_local"][0] + infos[q]["t_recv_off"][self.rank]) * elem * self.t_width))
             self.t_dst = _ptr_array(t_dst)
             self.t_dst_list, self.t_counts = t_dst, [t_counts[q] for q in self.peers]
             self.t_src = _ptr_array([self.t_ext.data_ptr()] * len(self.peers))
 
         # copy-engine pushes (overlapped exchanges): the rows are packed here first, then one contiguous copy per peer
-        pack = max(sum(send_counts) * self.bd_words, sum(self.t_counts) * self.t_words if self.tpart is not None else 0, 4)
+        pack = max(sum(send_counts[0]) * self.bd_words, sum(self.t_counts) * self.t_words if self.tpart is not None else 0, 4)
         self.send_buf = torch.empty(pack, dtype=torch.float32, device=self.device)      # 4-byte words
 
-        # deterministic reduce plan: local row -> its staging entries in ascending peer order
-        if n_send:
-            rows_cat = torch.cat([part.send_rows[q] for q in range(self.world)])        # staging order = peer order
+        # deterministic reduce plan: stacked own row -> its staging entries in ascending peer order
+        red_rows, red_cnt, red_entry = [], [], []
+        for i, t in enumerate(tables):
+            if not n_send[i]:
+                continue
+            rows_cat = torch.cat([t.send_rows[q] for q in range(self.world)])           # staging order = peer order
             order = torch.argsort(rows_cat, stable=True)
-            rows_sorted = rows_cat[order]
-            uniq, counts = torch.unique_consecutive(rows_sorted, return_counts=True)
-            ptr = torch.zeros(uniq.numel() + 1, dtype=torch.long)
+            uniq, counts = torch.unique_consecutive(rows_cat[order], return_counts=True)
+            red_rows.append(uniq + own_off[i])
+            red_cnt.append(counts)
+            red_entry.append(order + stage_off[i])
+        if red_rows:
+            counts = torch.cat(red_cnt)
+            ptr = torch.zeros(counts.numel() + 1, dtype=torch.long)
             ptr[1:] = torch.cumsum(counts, 0)
-            self.red_rows = uniq.to(self.device, torch.int32)
+            self.red_rows = torch.cat(red_rows).to(self.device, torch.int32)
             self.red_ptr = ptr.to(self.device, torch.int32)
-            self.red_entry = order.to(self.device, torch.int32)
+            self.red_entry = torch.cat(red_entry).to(self.device, torch.int32)
         else:
             self.red_rows = self.red_ptr = self.red_entry = None
 
@@ -244,6 +277,10 @@ class PeerLayerContext:
         self.grad_dst = _ptr_array([self.seg.peer_ptr(q, "slots", self.rank * self.n_flat * 4) for q in range(self.world)])
         self.grad_src = _ptr_array([self.flat.data_ptr()] * self.world)
         self.flag_ptrs = _ptr_array([self.seg.peer_ptr(q, "flags") for q in range(self.world)])
+
+    def table(self, i: int) -> torch.Tensor:
+        """[own | halo] rows of table i in this rank's segment (a new view object on every call)."""
+        return self.seg.view(f"bases_ext{i}", (self.n_ext[i], self.bd), self.storage_dtype)
 
     # -- step protocol -----------------------------------------------------------------------------------
     def begin_step(self, needs_grad: bool) -> int:
@@ -317,15 +354,15 @@ class PeerLayerContext:
         if dma:
             return self._push_dma(self.bases_ext, self.fwd_index, self.fwd_counts, self.fwd_dst_list, self.bd_words,
                                   (SLOT_FWD,))
-        self._push(len(self.peers), self.fwd_src, self.fwd_dst, self.fwd_seg_ptr, self.fwd_index.data_ptr(), self.bd_words,
-                   (SLOT_FWD,))
+        self._push(len(self.segments), self.fwd_src, self.fwd_dst, self.fwd_seg_ptr, self.fwd_index.data_ptr(),
+                   self.bd_words, (SLOT_FWD,))
 
-    def push_backward(self, d_bases_ext: torch.Tensor):
-        """Halo partial sums -> their owners' staging; raises BWD and CONS (my halo copy of the peers' basis rows is
-        no longer needed once the local backward passes are done)."""
-        base = d_bases_ext.data_ptr() + self.part.n_local * self.bd * 4
-        src = _ptr_array([base + self.recv_off[q] * self.bd * 4 for q in self.peers])
-        self._push(len(self.peers), src, self.bwd_dst, self.bwd_seg_ptr, None, self.bd, (SLOT_BWD, SLOT_CONS))
+    def push_backward(self, *d_bases_ext: torch.Tensor):
+        """Halo partial sums -> their owners' staging (one contiguous fp32 [own | halo] gradient per table); raises BWD
+        and CONS (my halo copy of the peers' basis rows is no longer needed once the local backward passes are done)."""
+        src = _ptr_array([d_bases_ext[i].data_ptr() + (self.tables[i].n_local + self.recv_off[i][q]) * self.bd * 4
+                          for q, i in self.segments])
+        self._push(len(self.segments), src, self.bwd_dst, self.bwd_seg_ptr, None, self.bd, (SLOT_BWD, SLOT_CONS))
 
     def push_t(self, dma: bool = False):
         """T exchange: the target-side stream rows my peers' source columns touch -> their stream tables; raises BWD and
@@ -336,6 +373,7 @@ class PeerLayerContext:
                    (SLOT_BWD, SLOT_CONS))
 
     def reduce_into(self, d_bases_local: torch.Tensor):
+        """d_bases_local (fp32, the stacked own rows of every table) += the peers' partial sums, in fixed peer order."""
         if self.red_rows is None:
             return
         check(_lib.load().egc_peer_reduce_rows(self.staging.data_ptr(), self.red_rows.data_ptr(), self.red_ptr.data_ptr(),

@@ -355,6 +355,8 @@ int egc_gather_rows(const float* src, const int32_t* index, int32_t n_index, int
  * The epoch is a device-resident counter advanced by a kernel, so a step can be replayed from a CUDA graph.
  * ---------------------------------------------------------------------------------------- */
 #define EGC_MAX_PEERS 8
+/* segments of one egc_peer_push_rows call: one per (peer, table), e.g. 7 peers x 4 node types of a heterogeneous layer */
+#define EGC_MAX_PUSH_SEGMENTS 64
 typedef struct egc_ipc_handle { unsigned char bytes[64]; } egc_ipc_handle;
 
 /* cudaMalloc + zero-fill + cudaIpcGetMemHandle (setup time; synchronises) */
@@ -364,7 +366,7 @@ int egc_peer_free(void* ptr);
 int egc_peer_open(const egc_ipc_handle* handle, void** ptr);
 int egc_peer_close(void* ptr);
 
-/* For each segment s < n_seg (HOST arrays src/dst/seg_ptr, n_seg <= EGC_MAX_PEERS): rows k in
+/* For each segment s < n_seg (HOST arrays src/dst/seg_ptr, n_seg <= EGC_MAX_PUSH_SEGMENTS): rows k in
  * [seg_ptr[s], seg_ptr[s+1]) of the concatenated list:  dst[s][(k - seg_ptr[s]), :] = src[s][index[k], :]
  * (index == NULL: src[s][k - seg_ptr[s], :]).  dst may point into a mapped peer segment.
  * Fused signal (flags != NULL, slot_mask != 0): the last CTA to finish, after a system-scope fence, raises
