@@ -38,6 +38,11 @@ class Epilogue(Structure):
     _fields_ = [("scale", c_void_p), ("shift", c_void_p), ("add", c_void_p), ("agg_init", c_void_p)]
 
 
+class Dropout(Structure):
+    """mirrors `egc_dropout`"""
+    _fields_ = [("seed", c_void_p), ("p", c_float), ("row_offset", c_int64)]
+
+
 class RowPlan(Structure):
     """mirrors `egc_row_plan`"""
     _fields_ = [("n_long", c_int32), ("n_chunks", c_int32), ("long_rows", c_void_p),
@@ -75,6 +80,10 @@ SIGNATURES = {
                                     _P, _P, _P, _P, _P, _P, c_size_t, _P]),
     "egc_aggregate_fwd_bf16": (c_int32, [POINTER(LayerDesc), _P, _P, _P, POINTER(RowPlan), _P, _P, _P, POINTER(Epilogue),
                                          _P, _P, _P, _P, _P, _P, c_size_t, _P]),
+    "egc_aggregate_fwd_dropout": (c_int32, [POINTER(LayerDesc), _P, _P, _P, _P, POINTER(RowPlan), _P, _P, _P, POINTER(Epilogue),
+                                            POINTER(Dropout), _P, c_int32, _P, _P, _P, _P, _P, _P, c_size_t, _P]),
+    "egc_aggregate_fwd_bf16_dropout": (c_int32, [POINTER(LayerDesc), _P, _P, _P, POINTER(RowPlan), _P, _P, _P, POINTER(Epilogue),
+                                                 POINTER(Dropout), _P, _P, _P, _P, _P, _P, c_size_t, _P]),
     "egc_aggregate_bwd_bf16_workspace_bytes": (c_size_t, [POINTER(LayerDesc), POINTER(RowPlan), c_int32]),
     "egc_aggregate_bwd_bf16": (c_int32, [POINTER(LayerDesc), _P, _P, _P, _P, _P, _P, POINTER(RowPlan), _P, _P, _P, _P, _P, _P, _P,
                                          _P, _P, _P, _P, c_int32, _P, c_size_t, _P]),

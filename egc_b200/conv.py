@@ -102,12 +102,15 @@ class EGConv(torch.nn.Module):
         return g
 
     def forward(self, x: Tensor, edge_index, relu: bool = False, scale: Optional[Tensor] = None,
-                shift: Optional[Tensor] = None, residual: Optional[Tensor] = None) -> Tensor:
+                shift: Optional[Tensor] = None, residual: Optional[Tensor] = None, dropout: float = 0.0,
+                dropout_seed: Optional[Tensor] = None) -> Tensor:
         """Extensions (keyword arguments the reference does not have; used by `egc_b200.EGC` / `egc_b200.EGCBlock`): the
         stack around the layer fused into the aggregation kernel's epilogue -
         `relu(layer(x) * scale + shift) + residual`, with `scale` / `shift` an eval-mode BatchNorm folded to constants
         (`egc_b200.fold_batchnorm`).  Same values as the separate torch ops; the backward masks / scales the incoming
-        gradient inside its first pass."""
+        gradient inside its first pass.  `dropout` = p > 0 (with relu=True): dropout after the ReLU in the same epilogue,
+        applied whenever p > 0 - the caller decides on training mode, as with F.dropout(training=...); its mask is the
+        counter-based one of `egc_b200.functional.egconv` (`dropout_seed`: see there), not torch's random stream."""
         if not x.is_cuda:
             raise RuntimeError("egc_b200.EGConv runs on CUDA (sm_100a) only; move the module and inputs to the GPU")
         if x.size(self.node_dim) == 0:                         # zero-node batch: empty output, zero parameter gradients
@@ -117,7 +120,7 @@ class EGConv(torch.nn.Module):
         flags = (_lib.BWD_DETERMINISTIC if self.deterministic else 0) | int(getattr(self, "bwd_flags", 0))
         return egconv(x, graph, self.bases_weight, self.comb_weight.weight, self.comb_weight.bias, self.bias,
                       self.num_heads, self.num_bases, self.aggregators, self.sigmoid, self.gemm_algo, flags, relu,
-                      scale, shift, residual, self.storage_dtype)
+                      scale, shift, residual, self.storage_dtype, dropout, dropout_seed)
 
     def __repr__(self):                                                                          # ref :280-286
         return "{}({}, {}, {})".format(self.__class__.__name__, self.in_channels, self.out_channels,

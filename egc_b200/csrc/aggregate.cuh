@@ -72,6 +72,13 @@ struct AggParams {
   int sm_agg, sm_w, sm_per_warp;
   int mode;      // 0: chunk tasks then row tasks, 1: merge tasks (one per long row)
   int rows_per_task;   // row-block kernel: consecutive rows per task (<= EGC_ROWS_PER_TASK); fewer when the launch is small
+  // fused dropout after the ReLU (egc_dropout), read only by the kernels instantiated with DROP = true: keep (row, c) iff
+  // Philox4x32-10 word c & 3 of counter (c >> 2, drop_row0 + row, 0, 0) under key *drop_seed is < drop_thresh; kept
+  // values are scaled by drop_scale
+  const uint64_t* drop_seed;   // null: no dropout
+  uint32_t drop_thresh;
+  float drop_scale;
+  int64_t drop_row0;           // global id of local row 0
 };
 
 // ---------------------------------------------------------------------------------------------
@@ -141,6 +148,41 @@ __device__ __forceinline__ void cp_async_16(void* smem_dst, const void* gmem_src
   asm volatile("cp.async.cg.shared.global [%0], [%1], 16;\n" ::"r"(d), "l"(gmem_src));
 }
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;\n" ::: "memory"); }
+
+// ---------------------------------------------------------------------------------------------
+// fused dropout: Philox4x32-10 (Salmon et al., SC'11; the Random123 constants), one call per 4 output columns
+// ---------------------------------------------------------------------------------------------
+__device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k) {
+#pragma unroll
+  for (int r = 0; r < 10; ++r) {
+    if (r > 0) { k.x += 0x9E3779B9u; k.y += 0xBB67AE85u; }
+    const uint32_t lo0 = 0xD2511F53u * c.x, hi0 = __umulhi(0xD2511F53u, c.x);
+    const uint32_t lo1 = 0xCD9E8D57u * c.z, hi1 = __umulhi(0xCD9E8D57u, c.z);
+    c = make_uint4(hi1 ^ c.y ^ k.x, lo1, hi0 ^ c.w ^ k.y, lo0);
+  }
+  return c;
+}
+
+// keep bits of columns 4q .. 4q + 3 of global row `grow` (bit w = column 4q + w).  Out of line, and the key is read here
+// (an L1-resident word): the forward kernels run at their register caps, and a key held from kernel start, or the
+// Philox rounds inlined into the epilogue loops, made the dropout instantiations spill in their gather loops
+static __device__ __noinline__ uint32_t dropout_keep4(const uint64_t* seed, uint32_t thresh, uint32_t q, uint32_t grow) {
+  const uint64_t s = __ldg(reinterpret_cast<const unsigned long long*>(seed));
+  const uint4 u = philox4x32_10(make_uint4(q, grow, 0u, 0u), make_uint2(static_cast<uint32_t>(s), static_cast<uint32_t>(s >> 32)));
+  return (u.x < thresh ? 1u : 0u) | (u.y < thresh ? 2u : 0u) | (u.z < thresh ? 4u : 0u) | (u.w < thresh ? 8u : 0u);
+}
+
+// columns c0 .. c0 + 3 (c0 % 4 == 0) of local row `row`, after the ReLU
+__device__ __forceinline__ void dropout4(const AggParams& p, float (&r)[4], int64_t row, int c0) {
+  const uint32_t m = dropout_keep4(p.drop_seed, p.drop_thresh, static_cast<uint32_t>(c0) >> 2, static_cast<uint32_t>(p.drop_row0 + row));
+#pragma unroll
+  for (int w = 0; w < 4; ++w) r[w] = (m >> w) & 1u ? __fmul_rn(r[w], p.drop_scale) : 0.f;
+}
+// one column (the scalar tails, D % 4 != 0): the same word of the same draw
+__device__ __forceinline__ float dropout1(const AggParams& p, float r, int64_t row, int c) {
+  const uint32_t m = dropout_keep4(p.drop_seed, p.drop_thresh, static_cast<uint32_t>(c) >> 2, static_cast<uint32_t>(p.drop_row0 + row));
+  return (m >> (c & 3)) & 1u ? __fmul_rn(r, p.drop_scale) : 0.f;
+}
 
 // ---------------------------------------------------------------------------------------------
 // accumulator of the aggregation primitives for VEC features
@@ -392,7 +434,9 @@ inline int n_saved_slots(const egc_layer_desc& d) { return d.n_aggr + (has_var_l
 // host: fill shape / geometry / smem layout fields; returns dynamic smem bytes per CTA
 int fill_agg_params(AggParams& p, const egc_layer_desc& d, bool vec4);
 
-// launchers (one translation unit per VEC/ARG combination to keep compile times parallel)
+// launchers (one translation unit per VEC/ARG combination to keep compile times parallel).  The *_dropout launchers run the
+// same kernels instantiated with DROP = true (fused dropout after the ReLU, p.drop_seed != null; *_dropout.cu); every
+// other launch runs kernels without a line of dropout code
 int launch_aggregate_v4(const AggParams& p, int mask, bool linw, bool arg, int smem_bytes, cudaStream_t st);
 int launch_aggregate_v1(const AggParams& p, int mask, bool linw, bool arg, int smem_bytes, cudaStream_t st);
 // fast path (aggregate_fast.cuh): vec4 rows of <= 128 floats, no per-nnz linear weights, mode 0 only
@@ -409,5 +453,16 @@ int rows_kernel_smem_bytes(const AggParams& p);
 int launch_aggregate_rows_bf16_static(int cfg_index, const AggParams& p, bool arg, int* task_counter, cudaStream_t st);
 int launch_aggregate_rows_bf16_g8(const AggParams& p, int mask, bool arg, int* task_counter, cudaStream_t st);
 int launch_aggregate_rows_bf16_g16(const AggParams& p, int mask, bool arg, int* task_counter, cudaStream_t st);
+int launch_aggregate_v4_dropout(const AggParams& p, int mask, bool linw, bool arg, int smem_bytes, cudaStream_t st);
+int launch_aggregate_v1_dropout(const AggParams& p, int mask, bool linw, bool arg, int smem_bytes, cudaStream_t st);
+int launch_aggregate_fast_g32_dropout(const AggParams& p, int mask, bool arg, int smem_bytes, cudaStream_t st);
+int launch_aggregate_fast_g16_dropout(const AggParams& p, int mask, bool arg, int smem_bytes, cudaStream_t st);
+int launch_aggregate_fast_static_dropout(int cfg_index, const AggParams& p, bool arg, int smem_bytes, cudaStream_t st);
+int launch_aggregate_rows_static_dropout(int cfg_index, const AggParams& p, bool arg, int* task_counter, cudaStream_t st);
+int launch_aggregate_rows_g32_dropout(const AggParams& p, int mask, bool arg, int* task_counter, cudaStream_t st);
+int launch_aggregate_rows_g16_dropout(const AggParams& p, int mask, bool arg, int* task_counter, cudaStream_t st);
+int launch_aggregate_rows_bf16_static_dropout(int cfg_index, const AggParams& p, bool arg, int* task_counter, cudaStream_t st);
+int launch_aggregate_rows_bf16_g8_dropout(const AggParams& p, int mask, bool arg, int* task_counter, cudaStream_t st);
+int launch_aggregate_rows_bf16_g16_dropout(const AggParams& p, int mask, bool arg, int* task_counter, cudaStream_t st);
 
 }  // namespace egc

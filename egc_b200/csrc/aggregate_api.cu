@@ -5,6 +5,7 @@
 #include <stdlib.h>
 
 #include <algorithm>
+#include <cmath>
 
 #include "aggregate_fast.cuh"
 #include "colsum.cuh"
@@ -62,6 +63,27 @@ static int validate_plan(const egc_row_plan* plan, const char* who) {
   if (plan == nullptr || plan->n_long == 0) return EGC_OK;
   EGC_REQUIRE(plan->n_long > 0 && plan->n_chunks >= 2 * plan->n_long, "%s: inconsistent row plan", who);
   EGC_REQUIRE(plan->long_rows && plan->long_chunk_ptr && plan->chunk_row && plan->chunk_begin, "%s: row plan with null arrays", who);
+  return EGC_OK;
+}
+
+// egc_dropout -> p.drop_*: threshold and scale from the fp32 p widened to double (include/egc_b200.h)
+static int set_dropout(AggParams& p, const egc_layer_desc& d, const egc_epilogue* epi, const egc_dropout* dropout,
+                       const float* out, const char* who) {
+  p.drop_seed = nullptr;
+  if (dropout == nullptr || dropout->p == 0.f) return EGC_OK;
+  EGC_REQUIRE(dropout->p > 0.f && dropout->p < 1.f, "%s: dropout p=%g outside [0, 1)", who, static_cast<double>(dropout->p));
+  EGC_REQUIRE(dropout->seed != nullptr, "%s: dropout without a seed", who);
+  EGC_REQUIRE(d.relu != 0, "%s: dropout is fused after the ReLU: it needs desc->relu", who);
+  EGC_REQUIRE(out != nullptr, "%s: dropout applies to the `out` output, which is not requested", who);
+  EGC_REQUIRE(epi == nullptr || (epi->scale == nullptr && epi->shift == nullptr && epi->add == nullptr),
+              "%s: dropout cannot be combined with the epilogue's scale / shift / add", who);
+  EGC_REQUIRE(dropout->row_offset >= 0 && dropout->row_offset + d.n_dst <= (int64_t{1} << 32),
+              "%s: dropout row_offset=%lld outside [0, 2^32 - n_dst]", who, static_cast<long long>(dropout->row_offset));
+  const double keep = 1.0 - static_cast<double>(dropout->p);
+  p.drop_seed = dropout->seed;
+  p.drop_thresh = static_cast<uint32_t>(std::min(std::floor(keep * 4294967296.0), 4294967295.0));   // p < 2^-53: 1 - p == 1
+  p.drop_scale = static_cast<float>(1.0 / keep);
+  p.drop_row0 = dropout->row_offset;
   return EGC_OK;
 }
 
@@ -227,6 +249,16 @@ int egc_aggregate_fwd(const egc_layer_desc* desc, const int32_t* rowptr, const i
                       const float* bias, const egc_epilogue* epilogue, const int32_t* row_subset, int32_t n_subset, float* out, float* agg_out,
                       int32_t* arg_out, float* saved, int32_t* saved_arg, void* workspace, size_t workspace_bytes,
                       void* stream) {
+  return egc_aggregate_fwd_dropout(desc, rowptr, col, val_sym, val_lin, plan, bases, weightings, bias, epilogue, nullptr,
+                                   row_subset, n_subset, out, agg_out, arg_out, saved, saved_arg, workspace, workspace_bytes,
+                                   stream);
+}
+
+int egc_aggregate_fwd_dropout(const egc_layer_desc* desc, const int32_t* rowptr, const int32_t* col, const float* val_sym,
+                              const float* val_lin, const egc_row_plan* plan, const float* bases, const float* weightings,
+                              const float* bias, const egc_epilogue* epilogue, const egc_dropout* dropout,
+                              const int32_t* row_subset, int32_t n_subset, float* out, float* agg_out, int32_t* arg_out,
+                              float* saved, int32_t* saved_arg, void* workspace, size_t workspace_bytes, void* stream) {
   if (int rc = validate_desc(desc, "egc_aggregate_fwd")) return rc;
   if (int rc = validate_plan(plan, "egc_aggregate_fwd")) return rc;
   EGC_REQUIRE(rowptr && col && bases, "egc_aggregate_fwd: null graph / bases pointer");
@@ -267,12 +299,16 @@ int egc_aggregate_fwd(const egc_layer_desc* desc, const int32_t* rowptr, const i
       p.agg_init = epilogue->agg_init;
     }
   }
+  if (int rc = set_dropout(p, *desc, epilogue, dropout, out, "egc_aggregate_fwd")) return rc;
   p.out = out; p.agg_out = agg_out; p.arg_out = arg_out; p.saved = saved; p.saved_arg = saved_arg;
   cudaStream_t st = as_stream(stream);
   const bool want_arg = (arg_out != nullptr || saved_arg != nullptr) && n_arg > 0;
   if (arg_out != nullptr && !want_arg && row_subset == nullptr)   // no min/max slot: every arg is "none"
     EGC_CUDA(cudaMemsetAsync(arg_out, 0xff, static_cast<size_t>(desc->n_dst) * desc->n_aggr * bd * sizeof(int32_t), st));
-  auto launch = vec4 ? launch_aggregate_v4 : launch_aggregate_v1;
+  // dropout runs the DROP = true instantiations (*_dropout.cu); every other call the kernels without dropout code
+  const bool drop = p.drop_seed != nullptr;
+  auto launch = drop ? (vec4 ? launch_aggregate_v4_dropout : launch_aggregate_v1_dropout)
+                     : (vec4 ? launch_aggregate_v4 : launch_aggregate_v1);
   p.mode = 0;
   const int hd = desc->heads * desc->dim;
   // (agg_init - the opt-in split launches of a row-partitioned caller - is served by the general kernel only)
@@ -289,13 +325,17 @@ int egc_aggregate_fwd(const egc_layer_desc* desc, const int32_t* rowptr, const i
   if (row_blocks) EGC_CUDA(cudaMemsetAsync(p.long_counter, 0, counter_off + sizeof(int), st));
   else if (fast && p.n_long > 0) EGC_CUDA(cudaMemsetAsync(p.long_counter, 0, static_cast<size_t>(p.n_long) * sizeof(int), st));
   if (row_blocks && static_idx >= 0) {
-    if (int rc = launch_aggregate_rows_static(static_idx, p, want_arg, task_counter, st)) return rc;
+    if (int rc = (drop ? launch_aggregate_rows_static_dropout : launch_aggregate_rows_static)(static_idx, p, want_arg, task_counter, st)) return rc;
   } else if (row_blocks) {
-    if (int rc = (p.G == 32 ? launch_aggregate_rows_g32 : launch_aggregate_rows_g16)(p, mask, want_arg, task_counter, st)) return rc;
+    auto rows = drop ? (p.G == 32 ? launch_aggregate_rows_g32_dropout : launch_aggregate_rows_g16_dropout)
+                     : (p.G == 32 ? launch_aggregate_rows_g32 : launch_aggregate_rows_g16);
+    if (int rc = rows(p, mask, want_arg, task_counter, st)) return rc;
   } else if (static_idx >= 0) {
-    if (int rc = launch_aggregate_fast_static(static_idx, p, want_arg, smem, st)) return rc;
+    if (int rc = (drop ? launch_aggregate_fast_static_dropout : launch_aggregate_fast_static)(static_idx, p, want_arg, smem, st)) return rc;
   } else if (fast) {
-    if (int rc = (p.G == 32 ? launch_aggregate_fast_g32 : launch_aggregate_fast_g16)(p, mask, want_arg, smem, st)) return rc;
+    auto fast_fam = drop ? (p.G == 32 ? launch_aggregate_fast_g32_dropout : launch_aggregate_fast_g16_dropout)
+                         : (p.G == 32 ? launch_aggregate_fast_g32 : launch_aggregate_fast_g16);
+    if (int rc = fast_fam(p, mask, want_arg, smem, st)) return rc;
   } else {
     if (int rc = launch(p, mask, val_lin != nullptr, want_arg, smem, st)) return rc;
   }
@@ -310,6 +350,15 @@ int egc_aggregate_fwd_bf16(const egc_layer_desc* desc, const int32_t* rowptr, co
                            const egc_row_plan* plan, const uint16_t* bases, const float* weightings, const float* bias,
                            const egc_epilogue* epilogue, float* out, float* agg_out, int32_t* arg_out, float* saved,
                            int32_t* saved_arg, void* workspace, size_t workspace_bytes, void* stream) {
+  return egc_aggregate_fwd_bf16_dropout(desc, rowptr, col, val_sym, plan, bases, weightings, bias, epilogue, nullptr, out,
+                                        agg_out, arg_out, saved, saved_arg, workspace, workspace_bytes, stream);
+}
+
+int egc_aggregate_fwd_bf16_dropout(const egc_layer_desc* desc, const int32_t* rowptr, const int32_t* col, const float* val_sym,
+                                   const egc_row_plan* plan, const uint16_t* bases, const float* weightings, const float* bias,
+                                   const egc_epilogue* epilogue, const egc_dropout* dropout, float* out, float* agg_out,
+                                   int32_t* arg_out, float* saved, int32_t* saved_arg, void* workspace, size_t workspace_bytes,
+                                   void* stream) {
   if (int rc = validate_desc(desc, "egc_aggregate_fwd_bf16")) return rc;
   if (int rc = validate_plan(plan, "egc_aggregate_fwd_bf16")) return rc;
   EGC_REQUIRE(rowptr && col && bases, "egc_aggregate_fwd_bf16: null graph / bases pointer");
@@ -353,6 +402,7 @@ int egc_aggregate_fwd_bf16(const egc_layer_desc* desc, const int32_t* rowptr, co
   }
   EGC_REQUIRE(desc->dim % 4 != 0 || (aligned16(bias) && aligned16(p.epi_scale) && aligned16(p.epi_shift) && aligned16(p.epi_add)),
               "egc_aggregate_fwd_bf16: bias / epilogue tensors must be 16-byte aligned");
+  if (int rc = set_dropout(p, *desc, epilogue, dropout, out, "egc_aggregate_fwd_bf16")) return rc;
   p.out = out; p.agg_out = agg_out; p.arg_out = arg_out; p.saved = saved; p.saved_arg = saved_arg;
   cudaStream_t st = as_stream(stream);
   const bool want_arg = (arg_out != nullptr || saved_arg != nullptr) && n_arg > 0;
@@ -363,6 +413,10 @@ int egc_aggregate_fwd_bf16(const egc_layer_desc* desc, const int32_t* rowptr, co
   int* task_counter = reinterpret_cast<int*>(reinterpret_cast<char*>(p.long_counter) + counter_off);
   EGC_CUDA(cudaMemsetAsync(p.long_counter, 0, counter_off + sizeof(int), st));
   const int static_idx = static_cfg_index(*desc);
+  if (p.drop_seed != nullptr) {                       // the DROP = true instantiations (*_dropout.cu)
+    if (static_idx >= 0) return launch_aggregate_rows_bf16_static_dropout(static_idx, p, want_arg, task_counter, st);
+    return (p.G == 16 ? launch_aggregate_rows_bf16_g16_dropout : launch_aggregate_rows_bf16_g8_dropout)(p, mask, want_arg, task_counter, st);
+  }
   if (static_idx >= 0) return launch_aggregate_rows_bf16_static(static_idx, p, want_arg, task_counter, st);
   return (p.G == 16 ? launch_aggregate_rows_bf16_g16 : launch_aggregate_rows_bf16_g8)(p, mask, want_arg, task_counter, st);
 }

@@ -42,21 +42,26 @@ __device__ __forceinline__ void stg_f4_hint(float* p, const float (&v)[4], uint6
                ::"l"(p), "f"(v[0]), "f"(v[1]), "f"(v[2]), "f"(v[3]), "l"(pol) : "memory");
 }
 
-// tail of the output epilogue after bias: BatchNorm-eval affine -> ReLU -> post-activation add (egc_epilogue order)
+// tail of the output epilogue after bias: BatchNorm-eval affine -> ReLU -> [DROP: dropout] -> post-activation add
+// (egc_epilogue order)
+template <bool DROP = false>
 __device__ __forceinline__ void epilogue_tail4(const AggParams& p, float (&r)[4], int64_t row, int o, int HD) {
   if (p.epi_scale != nullptr) {
     const float4 sc = __ldg(reinterpret_cast<const float4*>(p.epi_scale + o)), sh = __ldg(reinterpret_cast<const float4*>(p.epi_shift + o));
     r[0] = fmaf(r[0], sc.x, sh.x); r[1] = fmaf(r[1], sc.y, sh.y); r[2] = fmaf(r[2], sc.z, sh.z); r[3] = fmaf(r[3], sc.w, sh.w);
   }
   if (p.relu) { r[0] = fmaxf(r[0], 0.f); r[1] = fmaxf(r[1], 0.f); r[2] = fmaxf(r[2], 0.f); r[3] = fmaxf(r[3], 0.f); }
+  if constexpr (DROP) dropout4(p, r, row, o);
   if (p.epi_add != nullptr) {
     const float4 a = *reinterpret_cast<const float4*>(p.epi_add + row * HD + o);
     r[0] += a.x; r[1] += a.y; r[2] += a.z; r[3] += a.w;
   }
 }
+template <bool DROP = false>
 __device__ __forceinline__ float epilogue_tail1(const AggParams& p, float r, int64_t row, int o, int HD) {
   if (p.epi_scale != nullptr) r = fmaf(r, __ldg(p.epi_scale + o), __ldg(p.epi_shift + o));
   if (p.relu) r = fmaxf(r, 0.f);
+  if constexpr (DROP) r = dropout1(p, r, row, o);
   if (p.epi_add != nullptr) r += p.epi_add[row * HD + o];
   return r;
 }
@@ -207,7 +212,7 @@ __device__ __forceinline__ void add_edge(Acc<MASK, 4, false, ARG>& acc, const fl
   }
 }
 
-template <class Cfg, bool ARG>
+template <class Cfg, bool ARG, bool DROP = false>
 __global__ void __launch_bounds__(kAggThreads, 4) k_aggregate_fast(const __grid_constant__ AggParams p) {
   extern __shared__ __align__(16) float smem_all[];
   constexpr int MASK = Cfg::MASK, G = Cfg::G;
@@ -429,14 +434,14 @@ __global__ void __launch_bounds__(kAggThreads, 4) k_aggregate_fast(const __grid_
               const float4 b = __ldg(reinterpret_cast<const float4*>(p.bias + o));
               r[0] += b.x; r[1] += b.y; r[2] += b.z; r[3] += b.w;
             }
-            epilogue_tail4(p, r, row, o, GC::HD(p));
+            epilogue_tail4<DROP>(p, r, row, o, GC::HD(p));
             stg_f4_hint(out + o, r, pol_stream);
           } else {
             float r = 0.f;
 #pragma unroll 4
             for (int ab = 0; ab < AB; ++ab) r = fmaf(wh[ab], ad[ab * D], r);
             if (p.bias != nullptr) r += __ldg(p.bias + o);
-            r = epilogue_tail1(p, r, row, o, GC::HD(p));
+            r = epilogue_tail1<DROP>(p, r, row, o, GC::HD(p));
             __stcs(out + o, r);
           }
         }
@@ -449,9 +454,9 @@ __global__ void __launch_bounds__(kAggThreads, 4) k_aggregate_fast(const __grid_
 // ---------------------------------------------------------------------------------------------
 // dispatch
 // ---------------------------------------------------------------------------------------------
-template <class Cfg, bool ARG>
+template <class Cfg, bool ARG, bool DROP = false>
 int launch_fast_one(const AggParams& p, int smem_bytes, cudaStream_t st) {
-  auto kern = k_aggregate_fast<Cfg, ARG>;
+  auto kern = k_aggregate_fast<Cfg, ARG, DROP>;
   if (smem_bytes > 48 * 1024) {
     EGC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
   }
@@ -466,22 +471,22 @@ int launch_fast_one(const AggParams& p, int smem_bytes, cudaStream_t st) {
   return EGC_OK;
 }
 
-template <class Cfg>
+template <class Cfg, bool DROP = false>
 int launch_fast_arg(const AggParams& p, bool arg, int smem_bytes, cudaStream_t st) {
   if constexpr ((Cfg::MASK & (P_MAX | P_MIN)) != 0) {
-    if (arg) return launch_fast_one<Cfg, true>(p, smem_bytes, st);
+    if (arg) return launch_fast_one<Cfg, true, DROP>(p, smem_bytes, st);
   }
-  return launch_fast_one<Cfg, false>(p, smem_bytes, st);
+  return launch_fast_one<Cfg, false, DROP>(p, smem_bytes, st);
 }
 
 #define EGC_FAST_MASK_CASES(X) \
   X(1) X(2) X(3) X(5) X(7) X(8) X(9) X(10) X(11) X(13) X(15) X(16) X(17) X(18) X(19) X(21) X(23) \
   X(24) X(25) X(26) X(27) X(29) X(31)
 
-template <int G>
+template <int G, bool DROP = false>
 int launch_fast_family(const AggParams& p, int mask, bool arg, int smem_bytes, cudaStream_t st) {
   switch (mask) {
-#define X(M) case M: return launch_fast_arg<DynCfg<M, G>>(p, arg, smem_bytes, st);
+#define X(M) case M: return launch_fast_arg<DynCfg<M, G>, DROP>(p, arg, smem_bytes, st);
     EGC_FAST_MASK_CASES(X)
 #undef X
   }

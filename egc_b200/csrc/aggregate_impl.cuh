@@ -10,7 +10,7 @@ namespace egc {
 // forward epilogue: out[row, h*D+d] = sum_ab w[h*AB+ab] * agg[ab*D+d] (+ bias)     (ref :195-208)
 // agg rows live in this warp's shared memory as [A][BD] == [A*B][D].
 // ---------------------------------------------------------------------------------------------
-template <int EV>
+template <int EV, bool DROP = false>
 __device__ __forceinline__ void combine_epilogue(const AggParams& p, const float* sm, int row, int lane) {
   const float* agg = sm + p.sm_agg;
   const float* w = sm + p.sm_w;
@@ -38,7 +38,15 @@ __device__ __forceinline__ void combine_epilogue(const AggParams& p, const float
     for (int k = 0; k < EV; ++k) {                            // BatchNorm-eval affine -> ReLU -> post-activation add
       if (p.epi_scale != nullptr) acc[k] = fmaf(acc[k], __ldg(p.epi_scale + o0 + k), __ldg(p.epi_shift + o0 + k));
       if (p.relu) acc[k] = fmaxf(acc[k], 0.f);
-      if (p.epi_add != nullptr) acc[k] += p.epi_add[static_cast<int64_t>(row) * p.HD + o0 + k];
+      if constexpr (!DROP) { if (p.epi_add != nullptr) acc[k] += p.epi_add[static_cast<int64_t>(row) * p.HD + o0 + k]; }
+    }
+    if constexpr (DROP) {                                     // ReLU -> dropout (one Philox draw per 4 columns) -> add
+      if constexpr (EV == 4) dropout4(p, acc, row, o0);
+      else acc[0] = dropout1(p, acc[0], row, o0);
+      if (p.epi_add != nullptr) {
+#pragma unroll
+        for (int k = 0; k < EV; ++k) acc[k] += p.epi_add[static_cast<int64_t>(row) * p.HD + o0 + k];
+      }
     }
     st_stream<EV>(out + o0, acc);
   }
@@ -47,7 +55,7 @@ __device__ __forceinline__ void combine_epilogue(const AggParams& p, const float
 // ---------------------------------------------------------------------------------------------
 // the kernel
 // ---------------------------------------------------------------------------------------------
-template <int MASK, int VEC, bool LINW, bool ARG>
+template <int MASK, int VEC, bool LINW, bool ARG, bool DROP = false>
 __global__ void __launch_bounds__(kAggThreads, 3) k_aggregate(const __grid_constant__ AggParams p) {
   extern __shared__ __align__(16) float smem_all[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -157,16 +165,16 @@ __global__ void __launch_bounds__(kAggThreads, 3) k_aggregate(const __grid_const
 
   cp_async_wait_all();
   __syncwarp();
-  if (p.D % 4 == 0) combine_epilogue<4>(p, sm, row, lane);
-  else combine_epilogue<1>(p, sm, row, lane);
+  if (p.D % 4 == 0) combine_epilogue<4, DROP>(p, sm, row, lane);
+  else combine_epilogue<1, DROP>(p, sm, row, lane);
 }
 
 // ---------------------------------------------------------------------------------------------
 // dispatch over the primitive mask
 // ---------------------------------------------------------------------------------------------
-template <int MASK, int VEC, bool LINW, bool ARG>
+template <int MASK, int VEC, bool LINW, bool ARG, bool DROP = false>
 int launch_one(const AggParams& p, int smem_bytes, cudaStream_t st) {
-  auto kern = k_aggregate<MASK, VEC, LINW, ARG>;
+  auto kern = k_aggregate<MASK, VEC, LINW, ARG, DROP>;
   if (smem_bytes > 48 * 1024) {
     EGC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
   }
@@ -188,25 +196,25 @@ int launch_one(const AggParams& p, int smem_bytes, cudaStream_t st) {
 // masks without SYM: the only ones that can carry per-nnz linear weights
 #define EGC_MASK_CASES_NOSYM(X) X(1) X(5) X(8) X(9) X(13) X(16) X(17) X(21) X(24) X(25) X(29)
 
-template <int MASK, int VEC, bool LINW>
+template <int MASK, int VEC, bool LINW, bool DROP = false>
 int launch_arg(const AggParams& p, bool arg, int smem_bytes, cudaStream_t st) {
   if constexpr ((MASK & (P_MAX | P_MIN)) != 0) {
-    if (arg) return launch_one<MASK, VEC, LINW, true>(p, smem_bytes, st);
+    if (arg) return launch_one<MASK, VEC, LINW, true, DROP>(p, smem_bytes, st);
   }
-  return launch_one<MASK, VEC, LINW, false>(p, smem_bytes, st);
+  return launch_one<MASK, VEC, LINW, false, DROP>(p, smem_bytes, st);
 }
 
-template <int VEC>
+template <int VEC, bool DROP = false>
 int launch_family(const AggParams& p, int mask, bool linw, bool arg, int smem_bytes, cudaStream_t st) {
   if (!linw) {
     switch (mask) {
-#define X(M) case M: return launch_arg<M, VEC, false>(p, arg, smem_bytes, st);
+#define X(M) case M: return launch_arg<M, VEC, false, DROP>(p, arg, smem_bytes, st);
       EGC_MASK_CASES(X)
 #undef X
     }
   } else {
     switch (mask) {
-#define X(M) case M: return launch_arg<M, VEC, true>(p, arg, smem_bytes, st);
+#define X(M) case M: return launch_arg<M, VEC, true, DROP>(p, arg, smem_bytes, st);
       EGC_MASK_CASES_NOSYM(X)
 #undef X
     }

@@ -90,7 +90,7 @@ struct Bf16Cfg : Cfg {
   static_assert(Cfg::BD % 8 == 0 && nvec <= 16, "Bf16Cfg: basis rows of at most 128 values, a multiple of 8");
 };
 
-template <class Cfg, bool ARG, class ST = float>
+template <class Cfg, bool ARG, class ST = float, bool DROP = false>
 __global__ void __launch_bounds__(kAggThreads, EGC_ROWS_CTAS) k_aggregate_rows(const __grid_constant__ AggParams p, int* __restrict__ task_counter) {
   extern __shared__ __align__(16) float smem_all[];
   constexpr int MASK = Cfg::MASK, G = Cfg::G;
@@ -246,14 +246,14 @@ __global__ void __launch_bounds__(kAggThreads, EGC_ROWS_CTAS) k_aggregate_rows(c
             const float4 b = __ldg(reinterpret_cast<const float4*>(p.bias + o));
             r[0] += b.x; r[1] += b.y; r[2] += b.z; r[3] += b.w;
           }
-          epilogue_tail4(p, r, row, o, GC::HD(p));
+          epilogue_tail4<DROP>(p, r, row, o, GC::HD(p));
           stg_f4_hint(out + o, r, pol_stream);
         } else {
           float r = 0.f;
 #pragma unroll 4
           for (int ab = 0; ab < AB; ++ab) r = fmaf(wh[ab], ad[ab * D], r);
           if (p.bias != nullptr) r += __ldg(p.bias + o);
-          r = epilogue_tail1(p, r, row, o, GC::HD(p));
+          r = epilogue_tail1<DROP>(p, r, row, o, GC::HD(p));
           __stcs(out + o, r);
         }
       }
@@ -478,11 +478,11 @@ inline int pick_rows_per_task(int n_row_tasks) {
   return rpt;
 }
 
-template <class Cfg, bool ARG, class ST = float>
+template <class Cfg, bool ARG, class ST = float, bool DROP = false>
 int launch_rows_one(const AggParams& p_in, int* task_counter, cudaStream_t st) {
   AggParams p = p_in;
   p.rows_per_task = pick_rows_per_task(p.n_row_tasks);
-  auto kern = k_aggregate_rows<Cfg, ARG, ST>;
+  auto kern = k_aggregate_rows<Cfg, ARG, ST, DROP>;
   const int smem_bytes = rows_smem_bytes(p);
   if (smem_bytes > 48 * 1024) {
     EGC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
@@ -498,18 +498,18 @@ int launch_rows_one(const AggParams& p_in, int* task_counter, cudaStream_t st) {
   return EGC_OK;
 }
 
-template <class Cfg, class ST = float>
+template <class Cfg, class ST = float, bool DROP = false>
 int launch_rows_arg(const AggParams& p, bool arg, int* task_counter, cudaStream_t st) {
   if constexpr ((Cfg::MASK & (P_MAX | P_MIN)) != 0) {
-    if (arg) return launch_rows_one<Cfg, true, ST>(p, task_counter, st);
+    if (arg) return launch_rows_one<Cfg, true, ST, DROP>(p, task_counter, st);
   }
-  return launch_rows_one<Cfg, false, ST>(p, task_counter, st);
+  return launch_rows_one<Cfg, false, ST, DROP>(p, task_counter, st);
 }
 
-template <int G, class ST = float>
+template <int G, class ST = float, bool DROP = false>
 int launch_rows_family(const AggParams& p, int mask, bool arg, int* task_counter, cudaStream_t st) {
   switch (mask) {
-#define X(M) case M: return launch_rows_arg<DynCfg<M, G>, ST>(p, arg, task_counter, st);
+#define X(M) case M: return launch_rows_arg<DynCfg<M, G>, ST, DROP>(p, arg, task_counter, st);
     EGC_FAST_MASK_CASES(X)
 #undef X
   }

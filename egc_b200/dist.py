@@ -472,11 +472,14 @@ def n_target_streams(aggrs) -> int:
 class _PartitionedEGConvFunction(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, bases_weight, comb_weight, comb_bias, bias, pg, heads, num_bases, aggrs, sigmoid, algo, key,
-                grad_mode=True, bwd_flags=0, relu=False, storage_dtype=torch.float32):
+                grad_mode=True, bwd_flags=0, relu=False, storage_dtype=torch.float32, dropout=0.0, dropout_seed=None):
         from . import functional as F
         from . import peer as P
         part, g = pg.part, pg.graph
         x = F._require_cuda_f32("x", x)
+        dropout = F.check_dropout(dropout)
+        if dropout > 0.0 and not relu:
+            raise ValueError("the fused dropout follows the fused ReLU: dropout > 0 needs relu=True")
         bd = bases_weight.size(1)
         desc = F.make_desc(g, heads, num_bases, bd // num_bases, aggrs, sigmoid, relu)
         bf16 = storage_dtype == torch.bfloat16
@@ -499,10 +502,14 @@ class _PartitionedEGConvFunction(torch.autograd.Function):
             _, weightings = F.project(x, bases_weight.contiguous(), comb_weight.contiguous(), comb_bias, sigmoid, algo,
                                       bases_out=bases_ext[:part.n_local])
             outs = F.alloc_aggregate_outputs(desc, x.device, want_out=True, want_saved=needs_grad)
+            drop = None                                    # this rank's rows of the single-GPU mask: keyed by global row
+            if dropout > 0.0:
+                seed = F.check_dropout_seed(dropout_seed, x.device) if dropout_seed is not None else F.draw_dropout_seed(x.device)
+                drop = (seed, dropout, part.row_begin)
             def interior():
                 if rows_split:
                     F.aggregate_combine(desc, g, bases_ext, weightings, bias, row_subset=pg.interior, use_plan=False,
-                                        outputs=outs)
+                                        outputs=outs, dropout=drop)
 
             overlap = peer is not None and pg.uses_overlap(aggrs, storage_dtype)
             if overlap:
@@ -517,7 +524,7 @@ class _PartitionedEGConvFunction(torch.autograd.Function):
                 main.wait_stream(peer.side_stream)
                 peer.wait(P.SLOT_FWD)
                 F.aggregate_combine(desc, g_halo, bases_ext, weightings, bias, outputs=outs,
-                                    epilogue=(None, None, None, partial))
+                                    epilogue=(None, None, None, partial), dropout=drop)
             elif peer is not None:
                 peer.push_forward()                        # posted stores into the peers' halo regions, then FWD flag
                 interior()
@@ -532,14 +539,17 @@ class _PartitionedEGConvFunction(torch.autograd.Function):
                 pass
             elif rows_split:
                 F.aggregate_combine(desc, g, bases_ext, weightings, bias, row_subset=pg.boundary, use_plan=True,
-                                    outputs=outs)
+                                    outputs=outs, dropout=drop)
             else:                                          # one contiguous launch over every local row
-                F.aggregate_combine(desc, g, bases_ext, weightings, bias, outputs=outs)
+                F.aggregate_combine(desc, g, bases_ext, weightings, bias, outputs=outs, dropout=drop)
             if peer is not None and not needs_grad:
                 peer.signal(P.SLOT_CONS)
         out, _, _, saved, saved_arg = outs
         if needs_grad:
-            ctx.save_for_backward(x, bases_weight, comb_weight, bases_ext, weightings, saved, saved_arg, out if relu else None)
+            # dropout: out > 0 = ReLU open and kept, so the ReLU's mask scaled by k is the backward (functional.egconv)
+            k = (torch.full((desc.heads * desc.dim,), F.dropout_constants(dropout)[1], dtype=torch.float32, device=x.device)
+                 if dropout > 0.0 else None)
+            ctx.save_for_backward(x, bases_weight, comb_weight, bases_ext, weightings, saved, saved_arg, out if relu else None, k)
         ctx.pg, ctx.desc, ctx.algo, ctx.peer, ctx.bwd_flags, ctx.aggrs = pg, desc, algo, peer, int(bwd_flags), tuple(aggrs)
         ctx.storage_dtype = storage_dtype
         ctx.has_bias, ctx.has_comb_bias = bias is not None, comb_bias is not None
@@ -549,7 +559,7 @@ class _PartitionedEGConvFunction(torch.autograd.Function):
     def backward(ctx, grad_out):
         from . import functional as F
         from . import peer as P
-        x, bases_weight, comb_weight, bases_ext, weightings, saved, saved_arg, out_act = ctx.saved_tensors
+        x, bases_weight, comb_weight, bases_ext, weightings, saved, saved_arg, out_act, epi_scale = ctx.saved_tensors
         pg, part, peer = ctx.pg, ctx.pg.part, ctx.peer
         grad_out = F._require_cuda_f32("grad_out", grad_out)
         need_x, need_wb, need_wc, need_bc, need_b = ctx.needs_input_grad[:5]
@@ -565,13 +575,13 @@ class _PartitionedEGConvFunction(torch.autograd.Function):
                 t_own = torch.empty((part.n_local, t_width), dtype=ctx.storage_dtype, device=x.device)
                 d_w, _, d_bias, d_bc = F.aggregate_backward(ctx.desc, pg.graph, bases_ext, weightings, saved, saved_arg,
                                                             grad_out, want_b, ctx.bwd_flags, want_lin_colsum=True,
-                                                            out_act=out_act, tstreams_out=t_own)
+                                                            out_act=out_act, epi_scale=epi_scale, tstreams_out=t_own)
                 t_ext = torch.cat([t_own, pg.exchange_t.forward(t_own)])      # stream rows of the remote targets
                 d_bases = F.aggregate_backward_cols(desc_t, pg.graph_t, t_ext, bases_ext[:part.n_local])
             elif peer is None:
                 d_w, d_bases_ext, d_bias, d_bc = F.aggregate_backward(ctx.desc, pg.graph, bases_ext, weightings, saved,
                                                                       saved_arg, grad_out, want_b, ctx.bwd_flags,
-                                                                      want_lin_colsum=True, out_act=out_act)
+                                                                      want_lin_colsum=True, out_act=out_act, epi_scale=epi_scale)
                 d_bases = d_bases_ext[:part.n_local]
                 pg.exchange.reverse(d_bases_ext[part.n_local:], d_bases)     # halo partial sums go home
             if peer is None:
@@ -582,7 +592,7 @@ class _PartitionedEGConvFunction(torch.autograd.Function):
                 for t in (d_wb, d_wc, d_bc, d_bias):                          # parameters are replicated
                     if t is not None:
                         dist.all_reduce(t, op=dist.ReduceOp.SUM, group=pg.group)
-                return (d_x, d_wb, d_wc, d_bc, d_bias) + (None,) * 11
+                return (d_x, d_wb, d_wc, d_bc, d_bias) + (None,) * 13
             # ---- peer transport: flat parameter-gradient vector [d_wb | d_wc | d_bc | d_bias] in the exchange context
             n_wb, n_wc, hab = bases_weight.numel(), comb_weight.numel(), comb_weight.size(0)
             hd = ctx.desc.heads * ctx.desc.dim
@@ -607,7 +617,7 @@ class _PartitionedEGConvFunction(torch.autograd.Function):
                 # to them (BWD + CONS flags); once theirs are here the column pass over my own columns is complete
                 d_w, _, _, _ = F.aggregate_backward(ctx.desc, pg.graph, bases_ext, weightings, saved, saved_arg, grad_out,
                                                     want_b, ctx.bwd_flags, want_lin_colsum=True, out_bias=v_b,
-                                                    out_lin_colsum=v_bc, out_act=out_act, tstreams_out=peer.t_ext)
+                                                    out_lin_colsum=v_bc, out_act=out_act, epi_scale=epi_scale, tstreams_out=peer.t_ext)
                 if pg.uses_overlap(ctx.aggrs, ctx.storage_dtype):
                     peer.side_stream.wait_stream(main)
                     with torch.cuda.stream(peer.side_stream):
@@ -626,12 +636,12 @@ class _PartitionedEGConvFunction(torch.autograd.Function):
                 d_w, d_bases_ext, _, _ = F.aggregate_backward(ctx.desc, pg.graph, bases_ext, weightings, saved, saved_arg,
                                                               grad_out, want_b, ctx.bwd_flags, want_lin_colsum=True,
                                                               out_bias=v_b, out_lin_colsum=v_bc, col_split=part.n_local,
-                                                              between_phases=push_halo, out_act=out_act)
+                                                              between_phases=push_halo, out_act=out_act, epi_scale=epi_scale)
                 main.wait_stream(peer.side_stream)
             else:
                 d_w, d_bases_ext, _, _ = F.aggregate_backward(ctx.desc, pg.graph, bases_ext, weightings, saved, saved_arg,
                                                               grad_out, want_b, ctx.bwd_flags, want_lin_colsum=True,
-                                                              out_bias=v_b, out_lin_colsum=v_bc, out_act=out_act)
+                                                              out_bias=v_b, out_lin_colsum=v_bc, out_act=out_act, epi_scale=epi_scale)
                 peer.push_backward(d_bases_ext)
             if not use_t:
                 peer.wait(P.SLOT_BWD)
@@ -644,7 +654,7 @@ class _PartitionedEGConvFunction(torch.autograd.Function):
             d_wc = total[n_wb:n_wb + n_wc].view_as(comb_weight).clone() if need_wc else None
             d_bc = total[n_wb + n_wc:n_wb + n_wc + hab].clone() if want_bc else None
             d_bias = total[n_wb + n_wc + hab:n_wb + n_wc + hab + hd].clone() if want_b else None
-        return (d_x, d_wb, d_wc, d_bc, d_bias) + (None,) * 11
+        return (d_x, d_wb, d_wc, d_bc, d_bias) + (None,) * 13
 
 
 def _bwd_flags_of(conv) -> int:
@@ -652,12 +662,17 @@ def _bwd_flags_of(conv) -> int:
     return (_lib.BWD_DETERMINISTIC if getattr(conv, "deterministic", False) else 0) | int(getattr(conv, "bwd_flags", 0))
 
 
-def partitioned_egconv(x_local: Tensor, pg: PartitionedGraph, conv, relu: bool = False) -> Tensor:
+def partitioned_egconv(x_local: Tensor, pg: PartitionedGraph, conv, relu: bool = False, dropout: float = 0.0,
+                       dropout_seed: Optional[Tensor] = None) -> Tensor:
     """Run `conv` (an `egc_b200.EGConv` with replicated parameters) on this rank's rows of a partitioned graph.
     Output rows / input gradients are local; parameter gradients are summed over the ranks (= single-GPU values).
     With the peer transport every layer keeps its own exchange buffers (keyed by the module), one step in flight.
     A layer with `storage_dtype=torch.bfloat16` needs a graph built with `storage_dtype=torch.bfloat16`; it returns this
-    rank's rows of the single-GPU bf16 layer's results."""
+    rank's rows of the single-GPU bf16 layer's results.
+    `dropout` = p > 0 (with relu=True): the fused dropout of `egc_b200.functional.egconv`, keyed by the GLOBAL row, so each
+    rank gets its rows of the single-GPU mask for the same seed.  Without `dropout_seed` every rank draws it from its own
+    default CUDA generator: the ranks must be seeded identically (torch.manual_seed with the same value, as every
+    multi-rank driver of this project does), or their masks are not one mask."""
     storage_dtype = getattr(conv, "storage_dtype", torch.float32)
     if storage_dtype != torch.float32 and getattr(pg, "storage_dtype", None) != storage_dtype:
         raise NotImplementedError("partitioned_egconv: a layer with storage_dtype=torch.bfloat16 needs a PartitionedGraph "
@@ -666,7 +681,7 @@ def partitioned_egconv(x_local: Tensor, pg: PartitionedGraph, conv, relu: bool =
     return _PartitionedEGConvFunction.apply(x_local, conv.bases_weight, conv.comb_weight.weight, conv.comb_weight.bias,
                                             conv.bias, pg, conv.num_heads, conv.num_bases, tuple(conv.aggregators),
                                             bool(conv.sigmoid), int(conv.gemm_algo), id(conv), torch.is_grad_enabled(),
-                                            _bwd_flags_of(conv), bool(relu), storage_dtype)
+                                            _bwd_flags_of(conv), bool(relu), storage_dtype, float(dropout), dropout_seed)
 
 
 class PartitionedHeteroGraph:

@@ -6,6 +6,7 @@
 the hand-written one (CSR pass, atomic-free CSC pass, projection gradients).  PyTorch only owns
 the memory and the stream.
 """
+import ctypes
 from typing import Optional, Sequence
 
 import torch
@@ -69,6 +70,36 @@ def check_bf16_layer(desc: LayerDesc, graph: GraphStructure) -> None:
         raise ValueError("storage_dtype=torch.bfloat16 does not support an adjacency with edge values (without symnorm)")
 
 
+def check_dropout(p) -> float:
+    """The drop probability of the fused dropout: 0 <= p < 1 (0 = no dropout), else ValueError."""
+    p = float(p)
+    if not 0.0 <= p < 1.0:
+        raise ValueError(f"dropout probability has to be in [0, 1), got {p}")
+    return p
+
+
+def dropout_constants(p: float):
+    """(threshold, scale) of the fused dropout (include/egc_b200.h, egc_dropout): p is rounded to fp32 first, as the C
+    call receives it; keep iff the Philox word < threshold = floor((1 - p) * 2^32), kept values times scale = fp32(1 / (1 - p))."""
+    keep = 1.0 - float(ctypes.c_float(p).value)
+    return min(int(keep * 4294967296.0), 0xFFFFFFFF), float(ctypes.c_float(1.0 / keep).value)
+
+
+def check_dropout_seed(seed: Tensor, device) -> Tensor:
+    """A caller-supplied seed of the fused dropout: one int64 word on `device` (the kernel reads it from there)."""
+    if not (isinstance(seed, Tensor) and seed.is_cuda and seed.dtype == torch.int64 and seed.numel() == 1 and
+            seed.device == torch.device(device)):
+        raise ValueError("dropout_seed must be a one-element int64 tensor on the device of x")
+    return seed.contiguous()
+
+
+def draw_dropout_seed(device) -> Tensor:
+    """The per-call seed of the fused dropout: one draw from the default CUDA generator of `device`, so it follows
+    torch.manual_seed and - inside a CUDA graph - is drawn afresh at every replay.  Every layer call that applies dropout
+    draws exactly one seed, in layer order."""
+    return torch.randint(0, 2 ** 63 - 1, (1,), dtype=torch.int64, device=device)
+
+
 def project(x: Tensor, bases_weight: Tensor, comb_weight: Tensor, comb_bias: Optional[Tensor], sigmoid: bool,
             algo: int = _lib.GEMM_AUTO, bases_out: Optional[Tensor] = None, storage_dtype: torch.dtype = torch.float32):
     """bases = x @ W_b ; weightings = act(x @ W_c^T + b_c)   (ref :180-184).  `bases_out` lets a caller
@@ -103,12 +134,13 @@ def alloc_aggregate_outputs(desc: LayerDesc, device, want_out=True, want_agg=Fal
 def aggregate_combine(desc: LayerDesc, graph: GraphStructure, bases: Tensor, weightings: Optional[Tensor],
                       bias: Optional[Tensor], want_out: bool = True, want_agg: bool = False, want_arg: bool = False,
                       want_saved: bool = False, row_subset: Optional[Tensor] = None, use_plan: bool = True,
-                      outputs=None, epilogue=None):
+                      outputs=None, epilogue=None, dropout=None):
     """Fused SpMM + combination (ref :191-208).  Returns (out, agg, arg, saved, saved_arg); unrequested ones
     are None.  `saved` / `saved_arg` are what the backward pass consumes (see include/egc_b200.h).
     `row_subset` (int32 device tensor) restricts the row tasks; `outputs` reuses buffers of a previous call.
     `epilogue` = (scale, shift, add[, agg_init]) tensors or None each: the fused tail  y*scale+shift -> relu (desc.relu) ->
-    +add; agg_init [n_dst, A, B*D] = partial aggregates of an earlier call over another entry subset (sum / symnorm only)."""
+    +add; agg_init [n_dst, A, B*D] = partial aggregates of an earlier call over another entry subset (sum / symnorm only).
+    `dropout` = (seed [1] int64 CUDA tensor, p, global id of row 0) or None: dropout after the ReLU (egc_dropout)."""
     lib = _lib.load()
     dev = bases.device
     bf16 = bases.dtype == torch.bfloat16
@@ -126,13 +158,18 @@ def aggregate_combine(desc: LayerDesc, graph: GraphStructure, bases: Tensor, wei
     plan = graph.plan.struct if use_plan else None
     nbytes = lib.egc_aggregate_fwd_workspace_bytes(desc, plan)
     ws = _ws(nbytes, dev)
+    drop = None
+    if dropout is not None:
+        seed, p, row_offset = dropout
+        drop = _lib.Dropout(seed.data_ptr(), p, int(row_offset))
     if bf16:
         epi = None
         if epilogue is not None and any(t is not None for t in epilogue):
             epi = _lib.Epilogue(*(t.data_ptr() if t is not None else None for t in tuple(epilogue)[:3]), None)
-        check(lib.egc_aggregate_fwd_bf16(desc, ptr(graph.rowptr), ptr(graph.col), ptr(graph.val_sym), plan, ptr(bases),
-                                         ptr(weightings), ptr(bias), epi, ptr(out), ptr(agg), ptr(arg), ptr(saved),
-                                         ptr(saved_arg), ptr(ws), nbytes, _stream()), "egc_aggregate_fwd_bf16")
+        check(lib.egc_aggregate_fwd_bf16_dropout(desc, ptr(graph.rowptr), ptr(graph.col), ptr(graph.val_sym), plan,
+                                                 ptr(bases), ptr(weightings), ptr(bias), epi, drop, ptr(out), ptr(agg),
+                                                 ptr(arg), ptr(saved), ptr(saved_arg), ptr(ws), nbytes, _stream()),
+              "egc_aggregate_fwd_bf16")
         return outputs
     n_subset = int(row_subset.numel()) if row_subset is not None else 0
     if row_subset is not None and n_subset == 0 and not (use_plan and graph.plan.n_long):
@@ -141,9 +178,10 @@ def aggregate_combine(desc: LayerDesc, graph: GraphStructure, bases: Tensor, wei
     if epilogue is not None and any(t is not None for t in epilogue):
         scale, shift, add, agg_init = tuple(epilogue) + (None,) * (4 - len(epilogue))
         epi = _lib.Epilogue(*(t.data_ptr() if t is not None else None for t in (scale, shift, add, agg_init)))
-    check(lib.egc_aggregate_fwd(desc, ptr(graph.rowptr), ptr(graph.col), ptr(graph.val_sym), ptr(graph.val_lin), plan,
-                                ptr(bases), ptr(weightings), ptr(bias), epi, ptr(row_subset) if n_subset else None, n_subset,
-                                ptr(out), ptr(agg), ptr(arg), ptr(saved), ptr(saved_arg), ptr(ws), nbytes, _stream()),
+    check(lib.egc_aggregate_fwd_dropout(desc, ptr(graph.rowptr), ptr(graph.col), ptr(graph.val_sym), ptr(graph.val_lin),
+                                        plan, ptr(bases), ptr(weightings), ptr(bias), epi, drop,
+                                        ptr(row_subset) if n_subset else None, n_subset, ptr(out), ptr(agg), ptr(arg),
+                                        ptr(saved), ptr(saved_arg), ptr(ws), nbytes, _stream()),
           "egc_aggregate_fwd")
     return outputs
 
@@ -287,8 +325,14 @@ class _EGConvFunction(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, bases_weight, comb_weight, comb_bias, bias, graph, heads, num_bases, aggrs, sigmoid, algo,
                 bwd_flags, grad_mode=True, relu=False, epi_scale=None, epi_shift=None, epi_add=None,
-                storage_dtype=torch.float32):
+                storage_dtype=torch.float32, dropout=0.0, dropout_seed=None):
         x = _require_cuda_f32("x", x)
+        dropout = check_dropout(dropout)
+        if dropout > 0.0:
+            if not relu:
+                raise ValueError("the fused dropout follows the fused ReLU: dropout > 0 needs relu=True")
+            if epi_scale is not None or epi_shift is not None or epi_add is not None:
+                raise ValueError("the fused dropout cannot be combined with `scale`, `shift` or `residual`")
         epi_scale, epi_shift = _require_cuda_f32("scale", epi_scale), _require_cuda_f32("shift", epi_shift)
         epi_add = _require_cuda_f32("residual", epi_add)
         if (epi_scale is None) != (epi_shift is None):
@@ -313,14 +357,22 @@ class _EGConvFunction(torch.autograd.Function):
             for name, t, shape in (("scale", epi_scale, (hd,)), ("shift", epi_shift, (hd,)), ("residual", epi_add, (graph.n_dst, hd))):
                 if t is not None and tuple(t.shape) != shape:
                     raise ValueError(f"`{name}` of the fused epilogue must have shape {shape} (got {tuple(t.shape)})")
+            drop = None
+            if dropout > 0.0:
+                seed = check_dropout_seed(dropout_seed, x.device) if dropout_seed is not None else draw_dropout_seed(x.device)
+                drop = (seed, dropout, 0)
             out, _, _, saved, saved_arg = aggregate_combine(desc, graph, bases, weightings, bias, want_saved=needs_grad,
-                                                            epilogue=(epi_scale, epi_shift, epi_add))
+                                                            epilogue=(epi_scale, epi_shift, epi_add), dropout=drop)
         if needs_grad or (epi_add is not None and ctx.needs_input_grad[16] and grad_mode):
             # the fused ReLU's backward needs the sign of the post-activation value: `out` itself (the next layer's input
             # anyway, nothing extra is written) - or out - add when a residual was added after the activation
             act = None
             if relu:
                 act = out if epi_add is None else out - epi_add
+            if dropout > 0.0:
+                # out > 0 exactly where the ReLU was open and the element kept: pass 1's mask-and-scale with scale = k is
+                # the exact ReLU + dropout backward, and no mask is stored
+                epi_scale = torch.full((heads * dim,), dropout_constants(dropout)[1], dtype=torch.float32, device=x.device)
             ctx.save_for_backward(x, bases_weight, comb_weight, bases, weightings, saved, saved_arg, act, epi_scale)
         ctx.graph, ctx.desc, ctx.algo, ctx.bwd_flags = graph, desc, algo, bwd_flags
         ctx.has_bias, ctx.has_comb_bias = bias is not None, comb_bias is not None
@@ -333,7 +385,7 @@ class _EGConvFunction(torch.autograd.Function):
         need_x, need_wb, need_wc, need_bc, need_b = ctx.needs_input_grad[:5]
         d_add = grad_out if ctx.needs_input_grad[16] else None      # the residual is added after the activation
         if saved is None:                                           # only the residual needed a gradient
-            return (None,) * 16 + (d_add, None)
+            return (None,) * 16 + (d_add, None, None, None)
         with torch.cuda.device(x.device):
             want_bc = bool(need_bc and ctx.has_comb_bias)
             d_w, d_bases, d_bias, d_bc = aggregate_backward(ctx.desc, ctx.graph, bases, weightings, saved, saved_arg,
@@ -343,24 +395,29 @@ class _EGConvFunction(torch.autograd.Function):
                                                   need_wc, False, ctx.algo)
             if not want_bc:
                 d_bc = None
-        return (d_x, d_wb, d_wc, d_bc, d_bias) + (None,) * 11 + (d_add, None)
+        return (d_x, d_wb, d_wc, d_bc, d_bias) + (None,) * 11 + (d_add, None, None, None)
 
 
 def egconv(x: Tensor, graph: GraphStructure, bases_weight: Tensor, comb_weight: Tensor, comb_bias: Optional[Tensor],
            bias: Optional[Tensor], num_heads: int, num_bases: int, aggrs: Sequence[str], sigmoid: bool = False,
            algo: int = _lib.GEMM_AUTO, bwd_flags: int = 0, relu: bool = False, scale: Optional[Tensor] = None,
            shift: Optional[Tensor] = None, residual: Optional[Tensor] = None,
-           storage_dtype: torch.dtype = torch.float32) -> Tensor:
+           storage_dtype: torch.dtype = torch.float32, dropout: float = 0.0,
+           dropout_seed: Optional[Tensor] = None) -> Tensor:
     """Differentiable EGConv layer body on a prepared graph.  storage_dtype=torch.bfloat16 stores the basis rows and the
     backward's target-side streams as bf16 (half the gathered bytes); x, parameters, weightings, out, the saved aggregates,
     all accumulation and every gradient stay fp32.  Fused epilogue of the stack around the layer (SURVEY 8 f-1):
     `scale` / `shift` [F_out] = an eval-mode BatchNorm folded to an affine map (constants), `relu=True` the ReLU that
     follows (mag/models.py:63, arxiv/norm_models.py:35-36), `residual` [N, F_out] added after the activation (:38-39):
     out = relu(layer(x) * scale + shift) + residual, all inside the aggregation kernel's epilogue; the backward masks and
-    scales grad_out while its first pass stages the row."""
+    scales grad_out while its first pass stages the row.
+    `dropout` = p > 0 (with relu=True, without scale / shift / residual): training-mode dropout after the ReLU in the same
+    epilogue, out = keep ? relu(y) / (1 - p) : 0, with the counter-based mask of include/egc_b200.h (egc_dropout) keyed by
+    `dropout_seed` (a one-element int64 CUDA tensor; drawn by `draw_dropout_seed` when None).  The caller decides on training
+    mode, as with F.dropout(training=...).  The random stream is not torch's F.dropout stream."""
     return _EGConvFunction.apply(x, bases_weight, comb_weight, comb_bias, bias, graph, num_heads, num_bases,
                                  tuple(aggrs), bool(sigmoid), int(algo), int(bwd_flags), torch.is_grad_enabled(), bool(relu),
-                                 scale, shift, residual, check_storage_dtype(storage_dtype))
+                                 scale, shift, residual, check_storage_dtype(storage_dtype), float(dropout), dropout_seed)
 
 
 class _ProjectFunction(torch.autograd.Function):

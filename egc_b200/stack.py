@@ -12,7 +12,10 @@ Differences in execution only:
   * every layer of the stack uses the same aggregator list, so the prepared graph (CSR, CSC, symnorm weights, plans)
     is built ONCE and shared by the layers (the reference caches one copy per layer, `cached=True`);
   * `forward` also accepts a `PartitionedGraph` (row-partitioned multi-GPU run, `egc_b200.dist`): `x` then holds
-    this rank's rows and the result is this rank's rows of the single-GPU result.
+    this rank's rows and the result is this rank's rows of the single-GPU result;
+  * opt-in (`fused_dropout=True`): in training mode the dropout after every hidden layer runs in the same epilogue, after
+    the ReLU, and its backward is the ReLU's mask scaled by 1 / (1 - p) - no separate kernels, no stored mask.  Its random
+    stream is a counter-based one (`egc_b200.functional.egconv`), not torch's F.dropout stream, so it is not the default.
 """
 from typing import Iterable
 
@@ -21,6 +24,7 @@ import torch.nn.functional as F
 from torch import Tensor
 
 from .conv import EGConv
+from .functional import draw_dropout_seed
 from .graph import GraphStructure
 
 IN_FEATURES = 128        # ref mag/models.py:8-10
@@ -31,7 +35,7 @@ OUT_TRUE = 349
 class EGC(torch.nn.Module):
     def __init__(self, hidden_channels: int, num_layers: int, dropout: float, num_heads: int, num_bases: int,
                  aggrs: Iterable[str], in_features: int = IN_FEATURES, out_rounded: int = OUT_ROUNDED,
-                 out_true: int = OUT_TRUE, **conv_kwargs):
+                 out_true: int = OUT_TRUE, *, fused_dropout: bool = False, **conv_kwargs):
         super().__init__()
         if num_layers < 2:
             raise ValueError("EGC needs at least two layers (ref mag/models.py:22-54)")
@@ -42,6 +46,10 @@ class EGC(torch.nn.Module):
             for i in range(num_layers))
         self.dropout = dropout
         self.out_true = out_true
+        self.fused_dropout = bool(fused_dropout)
+        # seed tensors of the fused dropout drawn by the last forward, in layer order (inside a captured CUDA graph: the
+        # graph's buffers, which hold each replay's seeds) - enough to rebuild the masks exactly
+        self.last_dropout_seeds = []
 
     def reset_parameters(self):
         for conv in self.convs:
@@ -58,15 +66,24 @@ class EGC(torch.nn.Module):
     def forward(self, x: Tensor, adj_t) -> Tensor:
         from .dist import PartitionedGraph, partitioned_egconv
         g = self.prepare(x, adj_t)
-        if isinstance(g, PartitionedGraph):
-            def run(conv, h, relu):
-                return partitioned_egconv(h, g, conv, relu=relu)
-        else:
-            def run(conv, h, relu):
-                return conv(h, g, relu=relu)
+        seeds = []
+
+        def run(conv, h, relu, dropout=0.0):
+            seed = None
+            if dropout > 0.0:                                          # one seed per layer call, in layer order
+                seed = draw_dropout_seed(h.device)
+                seeds.append(seed)
+            if isinstance(g, PartitionedGraph):
+                return partitioned_egconv(h, g, conv, relu=relu, dropout=dropout, dropout_seed=seed)
+            return conv(h, g, relu=relu, dropout=dropout, dropout_seed=seed)
+        fused = self.fused_dropout and self.training and self.dropout > 0
         for conv in self.convs[:-1]:                                   # ref :61-65
-            x = run(conv, x, True)                                     # conv + ReLU: fused epilogue / backward mask
-            x = F.dropout(x, p=self.dropout, training=self.training)
+            if fused:                                                  # conv + ReLU + dropout: one epilogue
+                x = run(conv, x, True, self.dropout)
+            else:
+                x = run(conv, x, True)                                 # conv + ReLU: fused epilogue / backward mask
+                x = F.dropout(x, p=self.dropout, training=self.training)
+        self.last_dropout_seeds = seeds
         x = run(self.convs[-1], x, False)[:, :self.out_true]            # ref :68
         return x.log_softmax(dim=-1)                                   # ref :69
 

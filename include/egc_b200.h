@@ -250,6 +250,36 @@ int egc_aggregate_fwd_bf16(const egc_layer_desc* desc, const int32_t* rowptr, co
                            const egc_epilogue* epilogue, float* out, float* agg_out, int32_t* arg_out, float* saved,
                            int32_t* saved_arg, void* workspace, size_t workspace_bytes, void* stream);
 
+/* Training-mode dropout after the fused ReLU (ref mag/models.py:63-64), applied to `out` inside the same epilogue.  The mask
+ * is a pure function of (seed, global row, column):
+ *   key     = (low 32 bits of *seed, high 32 bits of *seed)         (*seed is read by the kernel: a replayed CUDA graph
+ *                                                                    sees whatever the seed buffer holds at replay time)
+ *   r       = word (c & 3) of Philox4x32-10(counter = (c >> 2, row_offset + i, 0, 0), key)   for output (i, c), c < H*D
+ *   keep    = r < min(floor((1 - p) * 2^32), 2^32 - 1),  k = fp32(1 / (1 - p)),  both from the fp32 `p` widened to double
+ *   out     = keep ? relu(y) * k : 0
+ * A row-partitioned caller passes its first global row as row_offset and gets its rows of the single-GPU mask.  p == 0 is no
+ * dropout; 0 < p < 1 needs desc->relu, `out`, and an epilogue without scale / shift / add (agg_init is allowed: it continues
+ * the sums before the combination).  Anything else returns EGC_ERR_INVALID_ARGUMENT.  The backward needs no mask:
+ * out > 0 exactly where the ReLU was open and the element kept, so egc_aggregate_bwd with out_act = out and epi_scale = a
+ * [H*D] vector filled with k is the exact ReLU + dropout backward. */
+typedef struct egc_dropout {
+  const uint64_t* seed;          /* device, one word                                              */
+  float p;                       /* drop probability, 0 <= p < 1                                  */
+  int64_t row_offset;            /* global id of local row 0; row_offset + n_dst <= 2^32          */
+} egc_dropout;
+
+/* egc_aggregate_fwd / egc_aggregate_fwd_bf16 with dropout (NULL: the calls above, which are these with dropout = NULL). */
+int egc_aggregate_fwd_dropout(const egc_layer_desc* desc, const int32_t* rowptr, const int32_t* col, const float* val_sym,
+                              const float* val_lin, const egc_row_plan* plan, const float* bases, const float* weightings,
+                              const float* bias, const egc_epilogue* epilogue, const egc_dropout* dropout,
+                              const int32_t* row_subset, int32_t n_subset, float* out, float* agg_out, int32_t* arg_out,
+                              float* saved, int32_t* saved_arg, void* workspace, size_t workspace_bytes, void* stream);
+int egc_aggregate_fwd_bf16_dropout(const egc_layer_desc* desc, const int32_t* rowptr, const int32_t* col, const float* val_sym,
+                                   const egc_row_plan* plan, const uint16_t* bases, const float* weightings, const float* bias,
+                                   const egc_epilogue* epilogue, const egc_dropout* dropout, float* out, float* agg_out,
+                                   int32_t* arg_out, float* saved, int32_t* saved_arg, void* workspace, size_t workspace_bytes,
+                                   void* stream);
+
 /* Backward of the above (ref: autograd of :191-208; torch_sparse spmm backward over the cached CSC).
  * Pass 1 (per target, streaming over `saved`): d_weightings (times sigmoid' when desc->sigmoid; = gradient
  * w.r.t. the Linear output) and the target-side streams t_sym / t_lin / t_sq; min/max gradients are routed
