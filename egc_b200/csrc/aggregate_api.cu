@@ -620,10 +620,10 @@ static int aggregate_bwd_impl(const egc_layer_desc* desc, const int32_t* rowptr,
   }
 
   if (!tail && !fuse_colsum) {
-    EGC_REQUIRE((out_act == nullptr && epi_scale == nullptr) || d_bias == nullptr,
-                "egc_aggregate_bwd: a fused epilogue needs the bias gradient from pass 1 (layer too wide for the fused column sums)");
+    // a layer too wide for the fused column sums: with a fused epilogue, d_bias sums grad_out masked with out_act > 0 and
+    // multiplied by epi_scale, the gradient pass 1 staged
     if (d_bias != nullptr) {
-      if (int rc = colsum_f32(grad_out, desc->n_dst, hd, d_bias, colsum_ws, L.colsum_bytes, st)) return rc;
+      if (int rc = colsum_f32(grad_out, desc->n_dst, hd, d_bias, colsum_ws, L.colsum_bytes, st, out_act, epi_scale)) return rc;
     }
     if (d_lin_colsum != nullptr) {
       if (int rc = colsum_f32(d_weightings, desc->n_dst, hab, d_lin_colsum, colsum_ws, L.colsum_bytes, st)) return rc;

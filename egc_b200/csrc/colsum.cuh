@@ -1,5 +1,6 @@
 // Deterministic two-stage column sum of a row-major fp32 matrix: out[c] = sum_r in[r, c].
-// Used for d_bias = colsum(grad_out) and d_b_comb = colsum(d_lin).
+// Used for d_bias = colsum(grad_out) and d_b_comb = colsum(d_lin).  With a gate and / or a scale (the backward of a fused
+// ReLU / affine epilogue) each term is first masked and scaled as backward pass 1 does it: (gate[r, c] > 0 ? in : 0) * scale[c].
 #pragma once
 
 #include <algorithm>
@@ -18,15 +19,25 @@ inline size_t colsum_workspace_bytes(int n_rows, int n_cols) {
   return static_cast<size_t>(colsum_slabs(n_rows)) * n_cols * sizeof(float) + 256;
 }
 
-static __global__ void k_colsum_stage1(const float* __restrict__ in, int n_rows, int n_cols, int rows_per_slab,
-                                float* __restrict__ partial) {
+template <bool EPI>
+static __global__ void k_colsum_stage1(const float* __restrict__ in, const float* __restrict__ gate, const float* __restrict__ scale,
+                                       int n_rows, int n_cols, int rows_per_slab, float* __restrict__ partial) {
   __shared__ float red[kColsumRowsPerCta][33];
   const int r0 = blockIdx.x * rows_per_slab, r1 = min(r0 + rows_per_slab, n_rows);
   for (int c0 = 0; c0 < n_cols; c0 += 32) {
     const int c = c0 + threadIdx.x;
     float s = 0.f;
-    if (c < n_cols)
-      for (int r = r0 + threadIdx.y; r < r1; r += kColsumRowsPerCta) s += __ldg(in + static_cast<int64_t>(r) * n_cols + c);
+    if (c < n_cols) {
+      for (int r = r0 + threadIdx.y; r < r1; r += kColsumRowsPerCta) {
+        const int64_t i = static_cast<int64_t>(r) * n_cols + c;
+        float v = __ldg(in + i);
+        if constexpr (EPI) {
+          if (gate != nullptr) v = __ldg(gate + i) > 0.f ? v : 0.f;
+          if (scale != nullptr) v *= __ldg(scale + c);
+        }
+        s += v;
+      }
+    }
     red[threadIdx.y][threadIdx.x] = s;
     __syncthreads();
     if (threadIdx.y == 0 && c < n_cols) {
@@ -50,7 +61,8 @@ static __global__ void k_colsum_stage2(const float* __restrict__ partial, int n_
   if (lane == 0) out[c] = t;
 }
 
-inline int colsum_f32(const float* in, int n_rows, int n_cols, float* out, void* ws, size_t ws_bytes, cudaStream_t st) {
+inline int colsum_f32(const float* in, int n_rows, int n_cols, float* out, void* ws, size_t ws_bytes, cudaStream_t st,
+                      const float* gate = nullptr, const float* scale = nullptr) {
   EGC_REQUIRE(in && out && ws && n_rows > 0 && n_cols > 0, "colsum: bad arguments");
   EGC_REQUIRE(ws_bytes >= colsum_workspace_bytes(n_rows, n_cols), "colsum: workspace too small");
   const int slabs = colsum_slabs(n_rows);
@@ -58,7 +70,10 @@ inline int colsum_f32(const float* in, int n_rows, int n_cols, float* out, void*
   float* partial = static_cast<float*>(ws);
   {
     LaunchScope egc_ls_("k_colsum_stage1", st);
-    k_colsum_stage1<<<slabs, dim3(32, kColsumRowsPerCta), 0, st>>>(in, n_rows, n_cols, rows_per_slab, partial);
+    if (gate != nullptr || scale != nullptr)
+      k_colsum_stage1<true><<<slabs, dim3(32, kColsumRowsPerCta), 0, st>>>(in, gate, scale, n_rows, n_cols, rows_per_slab, partial);
+    else
+      k_colsum_stage1<false><<<slabs, dim3(32, kColsumRowsPerCta), 0, st>>>(in, nullptr, nullptr, n_rows, n_cols, rows_per_slab, partial);
   }
   EGC_LAUNCH_CHECK("k_colsum_stage1");
   {

@@ -295,7 +295,10 @@ int egc_aggregate_fwd_bf16_dropout(const egc_layer_desc* desc, const int32_t* ro
  * NULL): pass 1 uses grad_out[i, c] * (out_act[i, c] > 0) - with an epilogue `add`, pass the post-activation value
  * BEFORE the add (out - add).  epi_scale (or NULL): the forward epilogue's scale; pass 1 multiplies the masked gradient
  * by it (scale / shift themselves are constants: no gradient is produced for them); the gradient w.r.t. `add` is
- * grad_out itself.  d_bias then is the gradient of the bias INSIDE the epilogue (masked and scaled).  tstreams_out (or NULL):
+ * grad_out itself.  d_bias then is the gradient of the bias INSIDE the epilogue (masked and scaled).  Column sums: pass 1
+ * accumulates d_bias and d_lin_colsum in registers while H*A*B <= 128 and H*D <= 512 (<= 128 when D % 4 != 0); wider
+ * layers take a two-stage column sum after the passes, which applies the same mask and scale to grad_out - so the fused
+ * epilogue has no width limit of its own.  tstreams_out (or NULL):
  * where pass 1 writes the target-side streams [n_dst, L, B*D] instead of the workspace (see egc_aggregate_bwd_cols).
  * flags: EGC_BWD_*. */
 #define EGC_BWD_DETERMINISTIC 1 /* route min/max gradients with a compare-and-add gather over the CSC instead of fp32
