@@ -68,6 +68,20 @@ struct Carver {
 // number of SMs of the current device (cached)
 int sm_count();
 
+// Raises cudaFuncAttributeMaxDynamicSharedMemorySize of `func` to `bytes` once per device: the attribute belongs to the
+// function in the current device's context, so a process that launches on several devices sets it on each.  `done` holds
+// the call site's per-device flags.
+constexpr int kMaxDevices = 64;
+inline cudaError_t max_dynamic_smem_once(const void* func, int bytes, bool (&done)[kMaxDevices]) {
+  int dev = 0;
+  if (cudaError_t e = cudaGetDevice(&dev)) return e;
+  const bool cached = dev >= 0 && dev < kMaxDevices;
+  if (cached && done[dev]) return cudaSuccess;
+  const cudaError_t e = cudaFuncSetAttribute(func, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+  if (e == cudaSuccess && cached) done[dev] = true;
+  return e;
+}
+
 // Every kernel launch goes through a LaunchScope: counts the launch and, when profiling is on,
 // brackets it with CUDA events on the launching stream (api.cu).
 struct LaunchScope {

@@ -223,12 +223,14 @@ int egc_project_fwd(const float* x, const float* w_bases, const float* w_comb, c
   EGC_REQUIRE(x && w_bases && w_comb && bases && weightings, "egc_project_fwd: null pointer");
   EGC_REQUIRE(algo >= EGC_GEMM_AUTO && algo <= EGC_GEMM_TF32, "egc_project_fwd: unknown algo %d", algo);
   cudaStream_t st = as_stream(stream);
-  if (algo != EGC_GEMM_FP32_SIMT && project_tc_supported(n, f_in, bd, hab)) {
+  const bool tc = algo != EGC_GEMM_FP32_SIMT && project_tc_supported(n, f_in, bd, hab);
+  if (tc && tc_aligned(x, bases, weightings, b_comb)) {
     return project_fwd_tc(x, w_bases, w_comb, b_comb, n, f_in, bd, hab, sigmoid, bases, weightings,
                           algo == EGC_GEMM_TF32 ? 1 : 3, st);
   }
   if (algo == EGC_GEMM_3XTF32 || algo == EGC_GEMM_TF32) {
-    set_error("egc_project_fwd: tensor-core path does not support n=%d f_in=%d bd=%d hab=%d", n, f_in, bd, hab);
+    if (tc) set_error("egc_project_fwd: tensor-core path does not support tensors that are not 16-byte aligned");
+    else set_error("egc_project_fwd: tensor-core path does not support n=%d f_in=%d bd=%d hab=%d", n, f_in, bd, hab);
     return EGC_ERR_UNSUPPORTED;
   }
   return project_fwd_simt(x, w_bases, w_comb, b_comb, n, f_in, bd, hab, sigmoid, bases, weightings, st);
@@ -241,12 +243,14 @@ int egc_project_fwd_bf16(const float* x, const float* w_bases, const float* w_co
   EGC_REQUIRE(x && w_bases && w_comb && bases && weightings, "egc_project_fwd_bf16: null pointer");
   EGC_REQUIRE(algo >= EGC_GEMM_AUTO && algo <= EGC_GEMM_TF32, "egc_project_fwd_bf16: unknown algo %d", algo);
   cudaStream_t st = as_stream(stream);
-  if (algo != EGC_GEMM_FP32_SIMT && project_tc_supported(n, f_in, bd, hab)) {
+  const bool tc = algo != EGC_GEMM_FP32_SIMT && project_tc_supported(n, f_in, bd, hab);
+  if (tc && tc_aligned(x, bases, weightings, b_comb)) {
     return project_fwd_tc_bf16(x, w_bases, w_comb, b_comb, n, f_in, bd, hab, sigmoid, bases, weightings,
                                algo == EGC_GEMM_TF32 ? 1 : 3, st);
   }
   if (algo == EGC_GEMM_3XTF32 || algo == EGC_GEMM_TF32) {
-    set_error("egc_project_fwd_bf16: tensor-core path does not support n=%d f_in=%d bd=%d hab=%d", n, f_in, bd, hab);
+    if (tc) set_error("egc_project_fwd_bf16: tensor-core path does not support tensors that are not 16-byte aligned");
+    else set_error("egc_project_fwd_bf16: tensor-core path does not support n=%d f_in=%d bd=%d hab=%d", n, f_in, bd, hab);
     return EGC_ERR_UNSUPPORTED;
   }
   return project_fwd_simt_bf16(x, w_bases, w_comb, b_comb, n, f_in, bd, hab, sigmoid, bases, weightings, st);
@@ -266,6 +270,10 @@ int egc_project_bwd(const float* x, const float* w_bases, const float* w_comb, c
   EGC_REQUIRE(algo >= EGC_GEMM_AUTO && algo <= EGC_GEMM_TF32, "egc_project_bwd: unknown algo %d", algo);
   cudaStream_t st = as_stream(stream);
   if (algo != EGC_GEMM_FP32_SIMT && project_tc_supported(n, f_in, bd, hab)) {
+    if ((algo == EGC_GEMM_3XTF32 || algo == EGC_GEMM_TF32) && d_x != nullptr && !tc_aligned(d_bases, d_lin, d_x)) {
+      set_error("egc_project_bwd: tensor-core path does not support tensors that are not 16-byte aligned");
+      return EGC_ERR_UNSUPPORTED;
+    }
     return project_bwd_tc(x, w_bases, w_comb, d_bases, d_lin, n, f_in, bd, hab, d_x, d_w_bases, d_w_comb, d_b_comb,
                           algo == EGC_GEMM_TF32 ? 1 : 3, workspace, workspace_bytes, st);
   }

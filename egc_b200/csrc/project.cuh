@@ -16,6 +16,9 @@ int project_bwd_simt(const float* x, const float* w_bases, const float* w_comb, 
 
 // tensor-core (tcgen05, kind::tf32) path; n_terms = 3 -> 3xTF32 split (fp32-level accuracy), 1 -> plain TF32
 bool project_tc_supported(int n, int f_in, int bd, int hab);
+// the operands and outputs of k_project_tc are read and written in 16-byte pieces: true when every non-NULL pointer is
+// 16-byte aligned
+bool tc_aligned(const void* a, const void* b, const void* c, const void* d = nullptr);
 int project_fwd_tc(const float* x, const float* w_bases, const float* w_comb, const float* b_comb, int n, int f_in,
                    int bd, int hab, int sigmoid, float* bases, float* weightings, int n_terms, cudaStream_t st);
 // the same with the basis rows stored as bf16 (round to nearest even); the weightings stay fp32

@@ -244,6 +244,12 @@ __global__ void __launch_bounds__(kTcThreads, 1) k_project_tc(const __grid_const
     int stage = cw % R;
     uint32_t phase = 0, lo_phase = 0;
     for (int c = cw; c < total_chunks; c += kConvWarps) {
+      // When R is not a multiple of 4 the slot's previous chunk (c - R) belongs to another converter warp, and its copy may
+      // still be in flight: raw_full would then be one phase behind, and a parity wait for this chunk would pass at once on
+      // the completed phase of chunk c - 2R.  So first wait until the MMA has consumed chunk c - R (raw_empty cannot be a
+      // phase ahead: chunk c is not consumed before it is converted).  The producer waits for the same before it copies
+      // chunk c, so this never delays the conversion.
+      mbar_wait(raw_empty(stage), phase ^ 1u);
       mbar_wait(raw_full(stage), phase);
       const uint32_t src = raw_addr + stage * kChunkBytes + lane * 16;
       float4 v[16];
@@ -457,6 +463,10 @@ static bool tc_plan(int k, int n, TcPlan& out) {
 
 static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 
+bool tc_aligned(const void* a, const void* b, const void* c, const void* d) {
+  return aligned16(a) && aligned16(b) && aligned16(c) && aligned16(d);
+}
+
 bool project_tc_supported(int n, int f_in, int bd, int hab) {
   if (n < 1 || f_in % 4 || bd % 4 || hab % 4) return false;
   TcPlan a, b;
@@ -523,11 +533,8 @@ static int launch_tc(TcParams& p, cudaStream_t st) {
   p.raw_stages = plan.raw_stages;
   p.num_tiles = ceil_div(p.M, kTileM);
   if (const char* ab = getenv("EGC_TC_ABLATE")) p.ablate = atoi(ab);
-  static bool attr_set = false;
-  if (!attr_set) {
-    EGC_CUDA(cudaFuncSetAttribute(k_project_tc<BF16_C1>, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxSmem));
-    attr_set = true;
-  }
+  static bool attr_set[kMaxDevices] = {};
+  EGC_CUDA(max_dynamic_smem_once(reinterpret_cast<const void*>(k_project_tc<BF16_C1>), kMaxSmem, attr_set));
   // TMA feed of the A operand (default; EGC_TC_NO_TMA=1 keeps the cp.async producers): needs the driver's tensor-map
   // encoder and 16-byte aligned rows.  Measured on B200: arxiv shape 0.106 -> 0.088 ms, mag shape 0.217 -> 0.159 ms.
   alignas(64) CUtensorMap tm1, tm2;
@@ -599,8 +606,9 @@ size_t project_bwd_tc_workspace(int n, int f_in, int bd, int hab) {
 int project_bwd_tc(const float* x, const float* w_bases, const float* w_comb, const float* d_bases, const float* d_lin,
                    int n, int f_in, int bd, int hab, float* d_x, float* d_w_bases, float* d_w_comb, float* d_b_comb,
                    int n_terms, void* workspace, size_t workspace_bytes, cudaStream_t st) {
-  if (d_x != nullptr) {
-    EGC_REQUIRE(aligned16(d_bases) && aligned16(d_lin) && aligned16(d_x), "tensor-core projection needs 16-byte aligned tensors");
+  // d_x from unaligned tensors: the FFMA kernel below (egc_project_bwd refuses this for a forced tensor-core algorithm)
+  float* d_x_simt = d_x != nullptr && !tc_aligned(d_bases, d_lin, d_x) ? d_x : nullptr;
+  if (d_x != nullptr && d_x_simt == nullptr) {
     TcParams p{};
     p.a1 = d_bases; p.lda1 = bd; p.k1 = bd; p.a2 = d_lin; p.lda2 = hab; p.k2 = hab; p.M = n;
     p.b[0][0] = w_bases; p.b_sn[0][0] = bd; p.b_sk[0][0] = 1;         // k < bd : B(n,k) = W_b[n][k]
@@ -628,7 +636,7 @@ int project_bwd_tc(const float* x, const float* w_bases, const float* w_comb, co
     workspace = static_cast<char*>(workspace) + wg_bytes;
     workspace_bytes -= wg_bytes;
   }
-  return project_bwd_simt(x, w_bases, w_comb, d_bases, d_lin, n, f_in, bd, hab, nullptr, d_w_bases, d_w_comb, d_b_comb,
+  return project_bwd_simt(x, w_bases, w_comb, d_bases, d_lin, n, f_in, bd, hab, d_x_simt, d_w_bases, d_w_comb, d_b_comb,
                           workspace, workspace_bytes, st);
 }
 

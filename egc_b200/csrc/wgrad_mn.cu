@@ -307,11 +307,8 @@ static int wgrad_mn_part(const float* x, const float* d1, int n1, int ld1, const
               (n1 == 0 || make_mn_map(&tm1, d1, n1, ld1, n)), "wgrad_mn: tensor-map encoding failed");
   if (n1 == 0) tm1 = tm2;                                      // never used: no d1 boxes are issued
   const size_t smem = static_cast<size_t>(p.raw_stages + kMnLoStages) * p.stage_bytes + (3 * kMnMaxRaw + kMnLoStages + 4) * 8 + 64 + 1024;
-  static bool attr_set = false;
-  if (!attr_set) {
-    EGC_CUDA(cudaFuncSetAttribute(k_wgrad_mn, cudaFuncAttributeMaxDynamicSharedMemorySize, kMnMaxSmem));
-    attr_set = true;
-  }
+  static bool attr_set[kMaxDevices] = {};
+  EGC_CUDA(max_dynamic_smem_once(reinterpret_cast<const void*>(k_wgrad_mn), kMnMaxSmem, attr_set));
   {
     LaunchScope ls("k_wgrad_tc", st);
     k_wgrad_mn<<<grid, kMnThreads, smem, st>>>(p, tmx, tm1, tm2);

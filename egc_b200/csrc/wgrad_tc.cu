@@ -329,11 +329,8 @@ int wgrad_tc(const float* x, const float* d_bases, const float* d_lin, int n, in
   p.partial = static_cast<float*>(workspace);
   const size_t op = 2 * (static_cast<size_t>(kWgM) * kWgChunk * 4 + static_cast<size_t>(p.n_pad) * kWgChunk * 4);
   const size_t smem = kWgOpStages * op + static_cast<size_t>(p.raw_stages) * kWgChunk * width * 4 + (2 * kWgMaxRaw + 8) * 8 + 64;
-  static bool attr_set = false;
-  if (!attr_set) {
-    EGC_CUDA(cudaFuncSetAttribute(k_wgrad_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, kWgMaxSmem));
-    attr_set = true;
-  }
+  static bool attr_set[kMaxDevices] = {};
+  EGC_CUDA(max_dynamic_smem_once(reinterpret_cast<const void*>(k_wgrad_tc), kWgMaxSmem, attr_set));
   {
     LaunchScope ls("k_wgrad_tc", st);
     k_wgrad_tc<<<grid, kWgThreads, smem, st>>>(p);

@@ -23,8 +23,11 @@
  *   EGC_FWD_WARP_PER_ROW=1     forward aggregation: warp-per-row kernel instead of the row-block kernel
  *   EGC_BWD_WARP_PER_COLUMN=1  backward CSC pass: warp-per-column kernel instead of the column-block kernel
  *   EGC_TC_NO_TMA=1            projection GEMM: cp.async producers instead of TMA tensor copies for the A operand
+ *   EGC_TC_NO_SWIZZLE=1        projection GEMM: four 16-byte TMA boxes per A chunk instead of one 64-byte-swizzled box
  *   EGC_TC_TMA_STORE=1         projection GEMM: TMA tensor-store epilogue (measured equal to the default)
- *   EGC_TC_MAX_RAW_STAGES=n    projection GEMM: cap the A ring depth
+ *   EGC_TC_MAX_RAW_STAGES=n    projection GEMM: cap the A ring depth (at least 4)
+ *   EGC_WGRAD_TRANSPOSE=1      parameter gradients: the transposing kernel (k_wgrad_tc) instead of the MN-major one
+ *                              (k_wgrad_mn); it partitions the nodes differently, so results differ in the last bits
  *   EGC_TC_ABLATE=bits         projection GEMM: switch pipeline stages off for timing (WRONG results; tools/gemm_ablate.sh)
  */
 #ifndef EGC_B200_H_
@@ -182,6 +185,15 @@ size_t egc_plan_build_workspace_bytes(int32_t n_rows);
 #define EGC_GEMM_FP32_SIMT 1    /* exact fp32 FFMA tiles (any shape)                               */
 #define EGC_GEMM_3XTF32 2       /* tcgen05 kind::tf32, 3-term split: fp32-level accuracy           */
 #define EGC_GEMM_TF32 3         /* tcgen05 kind::tf32, single pass (~1e-3 relative)                */
+
+/* Shapes and alignment of the tensor-core path: f_in, bd and hab multiples of 4 and the weights resident in shared memory
+ * next to the operand ring (the forward's and d_x's); the tensors a tensor-core kernel streams 16-byte aligned:
+ *   forward: x, bases, weightings and b_comb (when not NULL);
+ *   d_x:     d_bases, d_lin and d_x;
+ *   d_w_bases / d_w_comb: x, d_bases and d_lin.
+ * Contiguous tensors at a storage offset need not be.  EGC_GEMM_AUTO takes the fp32 FFMA kernels for a product whose
+ * shape or tensors do not qualify; EGC_GEMM_3XTF32 / EGC_GEMM_TF32 return EGC_ERR_UNSUPPORTED for the forward and d_x
+ * instead, while the parameter gradients fall back to the FFMA kernels under every algorithm. */
 
 /* bases[n, bd] = x[n, f_in] . w_bases[f_in, bd]
  * weightings[n, hab] = act(x . w_comb[hab, f_in]^T + b_comb[hab]),  act = sigmoid if `sigmoid`. */

@@ -330,13 +330,16 @@ def _src_ids(col, pos):
     return torch.where((pos >= 0) & (pos < nnz), col[pos.clamp(0, nnz - 1)], torch.full_like(pos, -1))
 
 
-def _traced(fn):
-    """fn()'s result and the demangled names of the CUDA kernels it launched (torch.profiler)."""
+def _traced(fn, trace=None):
+    """fn()'s result and the demangled names of the CUDA kernels it launched (torch.profiler).  With `trace` (a path) the
+    profile is also exported there as a chrome trace, whose kernel events carry the launch's grid and shared memory."""
     from torch.profiler import ProfilerActivity, profile
     torch.cuda.synchronize()
     with profile(activities=[ProfilerActivity.CUDA]) as prof:
         res = fn()
         torch.cuda.synchronize()
+    if trace is not None:
+        prof.export_chrome_trace(str(trace))
     return res, [e.name for e in prof.events() if e.device_type == torch.autograd.DeviceType.CUDA]
 
 
